@@ -11,9 +11,11 @@ Audio::convert_to_PV followed by PV::convert_to_audio, inputs resident in HBM. W
 as long and frame-range sharded (weak scaling): each rank transforms its contiguous frame range; resynthesis
 exchanges the per-bin phase state (all_gather) and the window-hop overlap-add halo (send/recv) over NCCL.
 
-One JSON line on stdout (rank 0). `value` = frames of all ranks / max-over-ranks device time (CUDA events); the K timed
-steps are repeated for `rounds` rounds (each bracketed by its own events) until about a second of device time has been
-measured, and `ms_per_step` is the mean over all of them.
+One JSON line on stdout (rank 0). `value` = frames of all ranks / max-over-ranks device time (CUDA events). With
+--steps K exactly K steps are timed; without it, rounds of 20 steps (each bracketed by its own events) are repeated until
+about --min-seconds of device time has been measured. `ms_per_step` is the mean over all timed steps.
+--dump-outputs DIR writes what the last timed step computed (a seeded sample of the PV rows and of the resynthesised
+audio, with their indices) as DIR/*.npy, so that two builds can be compared output for output on identical inputs.
 `e2e` = the same step through the reference-facing C++ API (tools/cpp/e2e_bench.cpp: flan::Audio holding a host
 std::vector -> convert_to_PV -> convert_to_audio -> get_buffer()), host vectors in and out every step, beside the
 copy-only ceiling of the same bytes over PCIe.
@@ -60,11 +62,18 @@ def parse():
     ap.add_argument("--no-summary-hint", action="store_true",
                     help="N = 1: analysis without flan_b200_hint_resynthesis (resynthesis then reads the rows twice, as in round 1)")
     ap.add_argument("--no-cfg3", action="store_true", help="skip the BASELINE config 3 leg (1 h mono 96 kHz through the multi-device handle)")
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="device time to cover with rounds of K steps")
+    ap.add_argument("--min-seconds", type=float, default=1.0, help="without --steps: device time to cover with rounds of 20 steps")
     ap.add_argument("--chain", action="store_true",
                     help="instead of the headline line: BASELINE config 4's chain (analysis -> repitch -> stretch -> resynthesis) "
                          "on one channel per GPU, with the reference's own PVModify.cpp timed beside it")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of what the last timed step computed (PV rows, audio) to DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.chain or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the headline round trip only")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -253,6 +262,24 @@ def copy_only_ceiling(torch, dev, nbytes_up, nbytes_down, steps):
     return (time.perf_counter() - t0) / steps
 
 
+DUMP_FRAMES, DUMP_SAMPLES, DUMP_SEED = 1024, 1 << 20, 20240601
+
+
+def dump_outputs(torch, outdir, pv, audio):
+    """The last timed step's outputs, as a caller receives them: PV rows (C, frames, bins, 2) and audio (C, n). A fixed,
+    seeded sample of at most DUMP_FRAMES rows and DUMP_SAMPLES audio samples per channel is written, with the indices it
+    was taken at (with the default workload: 3.69 GB of PV, about 50 MB written)."""
+    os.makedirs(outdir, exist_ok=True)
+    rng = np.random.default_rng(DUMP_SEED)
+    frames = np.sort(rng.choice(pv.shape[1], min(DUMP_FRAMES, pv.shape[1]), replace=False))
+    samples = np.sort(rng.choice(audio.shape[1], min(DUMP_SAMPLES, audio.shape[1]), replace=False))
+    pick = lambda t, idx: t.index_select(1, torch.from_numpy(idx).to(t.device)).cpu().numpy()  # noqa: E731
+    out = {"pv_frames": frames.astype(np.float64), "pv": pick(pv, frames).astype(np.float32),
+           "audio_samples": samples.astype(np.float64), "audio": pick(audio, samples).astype(np.float32)}
+    for name, a in out.items():
+        np.save(os.path.join(outdir, name + ".npy"), a)
+
+
 def cfg3_leg(world, steps, peak):
     """BASELINE config 3 (mono 96 kHz 1 h, window 8192 hop 512, round trip) through the multi-device handle of the C ABI
     (flan_b200_multi_*: one process, frame-range shards, P2P phase-state + halo exchange): on one device and, when the run
@@ -314,7 +341,9 @@ def e2e_cpp(args, local_rank, world, rank, steps, dist, dev):
     from flan_b200 import build
     from flan_b200.signals import noise_chirp
     os.environ["FLAN_B200_DEVICE"] = str(local_rank)      # the C++ layer's process-wide context
-    build.build_host()
+    # built by build(); the benchmark compiles nothing, so it can run from a read-only tree
+    if not os.path.exists(build.e2e_bench_path()):
+        raise RuntimeError("%s is missing: run `python -m flan_b200.build`" % build.e2e_bench_path())
     L = ctypes.CDLL(build.e2e_bench_path())
     L.e2e_round_trips.restype = ctypes.c_double
     L.e2e_round_trips.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_longlong, ctypes.c_float, ctypes.c_int, ctypes.c_int,
@@ -335,7 +364,7 @@ def e2e_cpp(args, local_rank, world, rank, steps, dist, dev):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return world * threads * k * CH * F / float(t.item())
 
-    k = max(steps, 10)
+    k = steps
     many = run(E2E_THREADS, k, 6)     # 6 untimed passes: by then the host vectors are recycled and page-locked
     two = run(2, k, 6)
     one = run(1, k, 6)
@@ -442,22 +471,23 @@ def run_ours(args):
     barrier()
 
     # ---- timed region: device-resident inputs, CUDA events on the launching stream -----------------------
-    # K steps per round; rounds are repeated until ~1 s of device time is covered so that the clock sampler sees the
-    # kernels under load (VERDICT r1: 20 x 3.9 ms gave it one sample).
+    # --steps K: one round of exactly K steps. Otherwise K = 20 steps per round, and rounds are repeated until ~1 s of
+    # device time is covered so that the clock sampler sees the kernels under load (20 x 3.9 ms gave it one sample).
     eng.set_timing(True)
-    for k in eng.KERNEL_KINDS:
-        eng.kernel_time(k)
-    launches0 = eng.launch_count()
-    probe0, probe1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    barrier()
-    probe0.record()
-    step(x)
-    probe1.record()
-    barrier()
-    est = torch.tensor([probe0.elapsed_time(probe1)], dtype=torch.float64, device=dev)
-    if world > 1:
-        dist.all_reduce(est, op=dist.ReduceOp.MAX)
-    rounds = int(max(1, min(200, np.ceil(args.min_seconds * 1e3 / max(float(est.item()) * steps, 1e-3)))))
+    rounds = 1
+    if args.steps is None:
+        for k in eng.KERNEL_KINDS:
+            eng.kernel_time(k)
+        probe0, probe1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        barrier()
+        probe0.record()
+        step(x)
+        probe1.record()
+        barrier()
+        est = torch.tensor([probe0.elapsed_time(probe1)], dtype=torch.float64, device=dev)
+        if world > 1:
+            dist.all_reduce(est, op=dist.ReduceOp.MAX)
+        rounds = int(max(1, min(200, np.ceil(args.min_seconds * 1e3 / max(float(est.item()) * steps, 1e-3)))))
     for k in eng.KERNEL_KINDS:
         eng.kernel_time(k)
     launches0 = eng.launch_count()
@@ -468,13 +498,16 @@ def run_ours(args):
             barrier()
             e0.record()
             for _ in range(steps):
-                step(x)
+                last = step(x)
             e1.record()
             barrier()
             round_ms.append(e0.elapsed_time(e1))
     launches = (eng.launch_count() - launches0) // rounds
     ktimes = {k: eng.kernel_time(k) for k in eng.KERNEL_KINDS}
     eng.set_timing(False)
+    if args.dump_outputs is not None and rank == 0:      # N > 1: rank 0's frame range and audio span
+        dump_outputs(torch, args.dump_outputs, pv, last)
+    del last
     # for comparison (N = 1): the same round trip without the hint -- analysis as a caller who keeps the PV for something
     # else runs it, resynthesis with its own pass over the rows for the phase summaries (round 1's form)
     plain_ms, plain_kernels = None, None
@@ -530,7 +563,7 @@ def run_ours(args):
         dist.barrier(group=cpu_group)        # every rank's GPU is idle from here on
     if rank == 0 and not args.no_cfg3:
         try:
-            cfg3 = cfg3_leg(world, max(5, steps // 2), measured_peak()[0])
+            cfg3 = cfg3_leg(world, steps, measured_peak()[0])
         except Exception as e:  # noqa: BLE001 - a leg must not take the headline line down with it
             cfg3 = {"error": repr(e)}
     if rank == 0:

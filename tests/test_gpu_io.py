@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from flan_b200.signals import noise_chirp
+from reference_records import Records, file_codec_reference
 from test_oracle_io import pv_fixture
 
 pytestmark = pytest.mark.gpu
@@ -61,22 +62,32 @@ def test_pcm24_codec_byte_exact(eng, oracle, C, n):
     assert np.array_equal(bits(back), bits(oracle.pcm24_decode(want, C, n)))
 
 
-def test_flan_files_interchange_with_the_reference_build(eng, oracle, tmp_path):
-    # oracle/_ref travels prebuilt to the GPU box; skip if it is not there
-    from oracle_lib import RefLib
-    if not RefLib.available():
-        pytest.skip("oracle/_ref/libflan_ref.so not present")
-    ref = RefLib(0)
+@pytest.fixture(scope="module")
+def rec():
+    r = Records("test_gpu_io")
+    yield r
+    r.save()
+
+
+def test_flan_files_interchange_with_the_reference_build(eng, oracle, rec, tmp_path):
     pv, sr = pv_fixture(seed=11, C=2, F=33, B=257)
     ar, W = oracle.analysis_rate(sr, 64), 512
     ours, theirs = str(tmp_path / "ours.flan"), str(tmp_path / "ref.flan")
     eng.save_flan(ours, dev(pv), sr, float(ar), W)
-    ref.save_flan(theirs, pv, sr, ar, W)
-    assert open(ours, "rb").read() == open(theirs, "rb").read()           # the same file, byte for byte
+    ref = file_codec_reference()
+    if ref is not None:
+        ref.save_flan(theirs, pv, sr, ar, W)
+    else:           # the file is ours, checked against the stored digest of the reference's, byte for byte
+        theirs = ours
+    # the same file, byte for byte
+    rec.check("save.file", np.fromfile(ours, np.uint8), None if ref is None else np.fromfile(theirs, np.uint8))
     got, sr2, rate2, W2 = eng.load_flan(theirs)
-    want, sr3, rate3, W3 = ref.load_flan(theirs)
-    assert (sr2, rate2, W2) == (sr3, rate3, W3)
-    assert np.array_equal(bits(got.cpu().numpy()), bits(want))
+    want, header = None, None
+    if ref is not None:
+        want, sr3, rate3, W3 = ref.load_flan(theirs)
+        header = np.array([sr3, rate3, W3], np.float64)
+    rec.check("load.header", np.array([sr2, rate2, W2], np.float64), header)
+    rec.check("load.pv", got.cpu().numpy(), want)
 
 
 def test_wav_files_round_trip_and_stdlib_reads_them(eng, oracle, tmp_path):

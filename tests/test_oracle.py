@@ -1,5 +1,6 @@
 """CPU tests of the checker itself: the C restatement (oracle/pv_oracle.c) against
- (1) the reference's own sources compiled verbatim (oracle/_ref), bit for bit;
+ (1) the reference's own sources compiled verbatim (oracle/_ref), bit for bit, or where that build is absent its
+     results as stored under tests/golden/reference/ (tests/reference_records.py);
  (2) the committed golden fixtures generated from that build (tests/golden/make_golden.py);
  (3) first-principles known answers that need no FFT library (SURVEY.md 8c pins 1-6).
 """
@@ -10,6 +11,7 @@ import numpy as np
 import pytest
 
 from flan_b200.signals import make_config, noise_chirp
+from reference_records import Records, live_reference
 
 GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "*.npz")))
 
@@ -18,46 +20,54 @@ def bits(a):
     return np.ascontiguousarray(a).view(np.uint32)
 
 
-@pytest.mark.parametrize("name,sec", [("cfg1", 1.0), ("cfg2", 0.5), ("cfg3", 0.5), ("cfg5", 0.5)])
-def test_oracle_bit_identical_to_reference_build(oracle, reflib, name, sec):
-    x, sr, W, h, N = make_config(name, sec)
+@pytest.fixture(scope="module")
+def rec():
+    r = Records("test_oracle")
+    yield r
+    r.save()
+
+
+def round_trip_matches_reference(oracle, ref, rec, key, x, sr, W, h, N, audio=True):
+    """The checker's analysis, and its resynthesis of the reference's PV, equal the reference build's bit for bit."""
     pv_o = oracle.convert_to_pv(x, sr, W, h, N)
-    pv_r, ar = reflib.convert_to_pv(x, sr, W, h, N)
-    assert ar == oracle.analysis_rate(sr, h)
-    assert np.array_equal(bits(pv_o), bits(pv_r))
-    a_o = oracle.convert_to_audio(pv_r, sr, ar, W)
-    a_r = reflib.convert_to_audio(pv_r, sr, ar, W)
-    assert np.array_equal(bits(a_o), bits(a_r))
+    ar = oracle.analysis_rate(sr, h)
+    pv_r, ar_r = ref.convert_to_pv(x, sr, W, h, N) if ref is not None else (None, None)
+    rec.check(key + ".analysis_rate", np.float32(ar), None if ref is None else np.float32(ar_r))
+    rec.check(key + ".pv", pv_o, pv_r)
+    if audio:       # pv_o equals the reference's PV here, so it stands in for it where the build is absent
+        pv_in = pv_r if pv_r is not None else pv_o
+        rec.check(key + ".audio", oracle.convert_to_audio(pv_in, sr, ar, W),
+                  None if ref is None else ref.convert_to_audio(pv_in, sr, ar, W))
 
 
-def test_oracle_bit_identical_zero_padded_and_odd_sizes(oracle, reflib):
+@pytest.mark.parametrize("name,sec", [("cfg1", 1.0), ("cfg2", 0.5), ("cfg3", 0.5), ("cfg5", 0.5)])
+def test_oracle_bit_identical_to_reference_build(oracle, rec, name, sec):
+    x, sr, W, h, N = make_config(name, sec)
+    round_trip_matches_reference(oracle, live_reference(), rec, name, x, sr, W, h, N)
+
+
+def test_oracle_bit_identical_zero_padded_and_odd_sizes(oracle, rec):
     x = np.stack([noise_chirp(5003, 32000, 9)])
     for W, h, N in [(256, 32, 1024), (512, 128, 512), (128, 8, 256), (1000, 100, 1024)]:
-        pv_o = oracle.convert_to_pv(x, 32000, W, h, N)
-        pv_r, ar = reflib.convert_to_pv(x, 32000, W, h, N)
-        assert np.array_equal(bits(pv_o), bits(pv_r)), (W, h, N)
-        assert np.array_equal(bits(oracle.convert_to_audio(pv_r, 32000, ar, W)),
-                              bits(reflib.convert_to_audio(pv_r, 32000, ar, W))), (W, h, N)
+        round_trip_matches_reference(oracle, live_reference(), rec, "odd_%d_%d_%d" % (W, h, N), x, 32000, W, h, N)
 
 
-def test_oracle_bit_identical_at_any_dft_size(oracle, reflib):
+def test_oracle_bit_identical_at_any_dft_size(oracle, rec):
     """FFTW plans any size (FFTHelper.cpp:16-26): the restatement follows the reference build's stand-in (radix-2 for
     powers of two, the O(n^2) definition in long double otherwise) at small, non-power-of-two and odd sizes. For an odd
     dft size the reference derives bin frequencies -- and, in convert_to_audio, the inverse transform's size -- from
     get_dft_size() = (num_bins - 1) * 2 (PVBuffer.cpp:356-359,443-446), i.e. from dft_size - 1."""
     x = np.stack([noise_chirp(2100, 32000, 11)])
     for W, h, N in [(64, 8, 64), (100, 10, 128), (300, 30, 300), (96, 12, 192), (250, 25, 375), (201, 20, 201), (120, 15, 255)]:
-        pv_o = oracle.convert_to_pv(x, 32000, W, h, N)
-        pv_r, ar = reflib.convert_to_pv(x, 32000, W, h, N)
-        assert np.array_equal(bits(pv_o), bits(pv_r)), (W, h, N)
-        if W <= (N // 2) * 2:       # the inverse runs at (num_bins - 1) * 2 points: the window must still fit
-            assert np.array_equal(bits(oracle.convert_to_audio(pv_r, 32000, ar, W)),
-                                  bits(reflib.convert_to_audio(pv_r, 32000, ar, W))), (W, h, N)
+        # the inverse runs at (num_bins - 1) * 2 points: the window must still fit
+        round_trip_matches_reference(oracle, live_reference(), rec, "dft_%d_%d_%d" % (W, h, N), x, 32000, W, h, N,
+                                     audio=W <= (N // 2) * 2)
 
 
-def test_oracle_hann_matches_reference_build(oracle, reflib):
+def test_oracle_hann_matches_reference_build(oracle, rec):
+    ref = live_reference()
     for W in (64, 1000, 2048, 8192):
-        assert np.array_equal(bits(oracle.hann(W)), bits(reflib.hann(W)))
+        rec.check("hann_%d" % W, oracle.hann(W), None if ref is None else ref.hann(W))
 
 
 @pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p) for p in GOLDEN])
@@ -148,13 +158,27 @@ def test_round_trip_gain_of_steady_sine(oracle):
     assert 0.999 < g < 1.003
 
 
-def test_ms_wrappers_null_unless_stereo(reflib):
-    mono = np.zeros((1, 4096), np.float32)
-    pv, _ = reflib.convert_to_pv(mono, 48000, 256, 32, 256, ms=True)
-    assert pv is None
-    tri = np.zeros((3, 4096), np.float32)
-    pv, _ = reflib.convert_to_pv(tri, 48000, 256, 32, 256, ms=True)
-    assert pv is None
+def test_ms_wrappers_null_unless_stereo(rec):
+    """convert_to_ms_PV returns a null PV unless the audio is stereo (AudioPV.cpp:82): the reference build does, and so
+    does this project's C++ API, which follows it (frames returned, -1 for a null PV)."""
+    import ctypes
+    from flan_b200 import build
+    build.build_host()
+    api = ctypes.CDLL(build.api_test_path())
+    fp = ctypes.POINTER(ctypes.c_float)
+    api.api_convert_to_pv.argtypes = [fp, ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_int, ctypes.c_int,
+                                      ctypes.c_int, ctypes.c_int, fp, fp]
+    ref = live_reference()
+    for C in (1, 3):
+        x = np.zeros((C, 4096), np.float32)
+        pv, ar = np.zeros((C, 129, 129, 2), np.float32), np.zeros(1, np.float32)
+        frames = api.api_convert_to_pv(x.ctypes.data_as(fp), C, 4096, 48000.0, 256, 32, 256, 1, pv.ctypes.data_as(fp),
+                                       ar.ctypes.data_as(fp))
+        theirs = None
+        if ref is not None:
+            pv_r, _ = ref.convert_to_pv(x, 48000, 256, 32, 256, ms=True)
+            theirs = np.array([-1 if pv_r is None else pv_r.shape[1]], np.int64)
+        rec.check("ms_pv_frames_%dch" % C, np.array([frames], np.int64), theirs)
 
 
 def test_chunked_oracle_equals_full(oracle):

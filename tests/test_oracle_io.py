@@ -7,6 +7,8 @@ import struct
 import numpy as np
 import pytest
 
+from reference_records import Records, file_codec_reference
+
 
 def bits(a):
     return np.ascontiguousarray(a).view(np.uint32)
@@ -23,21 +25,39 @@ def pv_fixture(seed=3, C=2, F=9, B=65, sr=44100.0):
     return pv, sr
 
 
-def test_flan_codec_matches_reference_file_bytes(oracle, reflib, tmp_path):
+@pytest.fixture(scope="module")
+def rec():
+    r = Records("test_oracle_io")
+    yield r
+    r.save()
+
+
+def test_flan_codec_matches_reference_file_bytes(oracle, rec, tmp_path):
     pv, sr = pv_fixture()
     ar, W = oracle.analysis_rate(sr, 32), 128
-    path = str(tmp_path / "ref.flan")
-    reflib.save_flan(path, pv, sr, ar, W)
-    raw = np.fromfile(path, np.uint8)
+    ref = file_codec_reference()
+    if ref is not None:
+        path = str(tmp_path / "ref.flan")
+        ref.save_flan(path, pv, sr, ar, W)
+        raw = np.fromfile(path, np.uint8)
+        got, sr2, ar2, W2 = ref.load_flan(path)
+        header = np.array([sr2, ar2, W2], np.float64)
+        rec.check("save.file", raw, raw, whole=True)
+        rec.check("load.header", header, header)
+    else:           # what the reference's save wrote and its load returned, as stored
+        raw = rec.stored_array("save.file")
+        sr2, ar2, W2 = rec.stored_array("load.header").tolist()
+        got = None
     assert raw[:4].tobytes() == b"RIFF" and raw[8:12].tobytes() == b"PV\0\0" and raw[12:16].tobytes() == b"fmt "
     fmt = struct.unpack("<IHHIIIIIIH", raw[16:50].tobytes())
     assert fmt == (30, 1, 2, 9, 65, 44100, 32, 128, 24, 1)
     assert raw[50:54].tobytes() == b"data" and struct.unpack("<I", raw[54:58].tobytes())[0] == pv.size * 3
     assert np.array_equal(raw[58:], oracle.flan_encode(pv, sr))
     # ... and back: the reference's load against the restated decode, bit for bit; load keeps the hop as analysis rate
-    got, sr2, ar2, W2 = reflib.load_flan(path)
     assert (sr2, ar2, W2) == (44100.0, 32.0, 128)
-    assert np.array_equal(bits(got), bits(oracle.flan_decode(raw[58:], pv.shape[:3], sr)))
+    decoded = oracle.flan_decode(raw[58:], pv.shape[:3], sr)
+    rec.check("load.pv", decoded, got)
+    got = decoded
     # quantisation error bound away from the clamp: 2^-23 of full scale
     inside = (np.abs(pv[..., 0]) < 128) & (np.abs(pv[..., 1]) < sr)
     assert np.max(np.abs(got[..., 0] - pv[..., 0])[inside]) <= 128 * 2.0 ** -23 * 1.0001

@@ -1,6 +1,6 @@
 """CPU tests of the checker for the PV-domain chain (SURVEY 8f-1): the C restatement of PV::repitch / PV::stretch /
 PV::modify_time (oracle/pv_oracle.c) against the reference's own PV/PVModify.cpp compiled verbatim
-(oracle/_ref/libflan_ref_modify.so), bit for bit, and against the committed fixtures generated from that build."""
+(oracle/_ref/libflan_ref_modify.so, or its results stored under tests/golden/reference/), bit for bit, and against the committed fixtures generated from that build."""
 import glob
 import os
 
@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from flan_b200.signals import make_config
+from reference_records import Records, live_reference_modify
 
 GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "modify", "modify_*.npz")))
 
@@ -17,11 +18,10 @@ def bits(a):
 
 
 @pytest.fixture(scope="module")
-def refmod(oracle):
-    from oracle_lib import RefModifyLib
-    if not RefModifyLib.available():
-        pytest.skip("oracle/_ref/libflan_ref_modify.so not built (needs /root/reference)")
-    return RefModifyLib()
+def rec():
+    r = Records("test_oracle_modify")
+    yield r
+    r.save()
 
 
 @pytest.fixture(scope="module")
@@ -40,16 +40,17 @@ def tables(F, B):
 
 
 @pytest.mark.parametrize("interp", range(10))
-def test_modify_oracle_bit_identical_to_reference_build(oracle, refmod, pv_case, interp):
+def test_modify_oracle_bit_identical_to_reference_build(oracle, rec, pv_case, interp):
     pv, sr, ar, W = pv_case
     _, F, B, _ = pv.shape
+    ref = live_reference_modify()
     for kind, fac in tables(F, B).items():
-        assert np.array_equal(bits(oracle.repitch(pv, sr, fac, interp)), bits(refmod.repitch(pv, sr, ar, W, fac, interp))), kind
-        a, b = oracle.stretch(pv, sr, ar, fac, interp), refmod.stretch(pv, sr, ar, W, fac, interp)
-        assert a.shape == b.shape and np.array_equal(bits(a), bits(b)), kind
+        key = "interp%d.%s." % (interp, kind)
+        rec.check(key + "repitch", oracle.repitch(pv, sr, fac, interp), None if ref is None else ref.repitch(pv, sr, ar, W, fac, interp))
+        rec.check(key + "stretch", oracle.stretch(pv, sr, ar, fac, interp), None if ref is None else ref.stretch(pv, sr, ar, W, fac, interp))
         sec = np.cumsum(fac, axis=0, dtype=np.float32) / np.float32(ar)
-        a, b = oracle.modify_time(pv, sr, ar, sec, interp), refmod.modify_time(pv, sr, ar, W, sec, interp)
-        assert a.shape == b.shape and np.array_equal(bits(a), bits(b)), kind
+        rec.check(key + "modify_time", oracle.modify_time(pv, sr, ar, sec, interp),
+                  None if ref is None else ref.modify_time(pv, sr, ar, W, sec, interp))
 
 
 @pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p) for p in GOLDEN])
