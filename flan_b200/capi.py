@@ -108,6 +108,8 @@ SYMBOLS = [
     ("flan_b200_multi_scatter_audio", _int, [_vp, _vp, _int, _i64, _int, _int, _int, _pa]),
     ("flan_b200_multi_convert_to_pv", _int, [_vp, _pa, _f, _int, _int, _int, _pp]),
     ("flan_b200_multi_convert_to_audio", _int, [_vp, _pp, _pa]),
+    ("flan_b200_multi_hint_resynthesis", _int, [_vp]),
+    ("flan_b200_multi_promise_unchanged", _int, [_vp, _pp]),
     ("flan_b200_multi_gather_audio", _int, [_vp, _pa, _vp]),
     ("flan_b200_multi_gather_pv", _int, [_vp, _pp, _vp, _int, _vp]),
     ("flan_b200_multi_free_audio", _int, [_vp, _pa]),

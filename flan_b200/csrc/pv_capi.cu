@@ -160,8 +160,10 @@ int get_plan( flan_b200_ctx * ctx, int N, int W, int hop, float sr, float ar, De
 	return FLAN_B200_OK;
 	}
 
-int get_workspace( flan_b200_ctx * ctx, size_t bytes, void ** out )
+int get_workspace( flan_b200_ctx * ctx, size_t bytes, void ** out, bool * kept )
 	{
+	ctx->summaries.drop();          // the caller overwrites them (a producer publishes again after its launch)
+	if( kept ) *kept = bytes <= ctx->workspace_bytes;
 	if( bytes > ctx->workspace_bytes )
 		{
 		if( ctx->workspace )
@@ -173,7 +175,6 @@ int get_workspace( flan_b200_ctx * ctx, size_t bytes, void ** out )
 		bytes = align_up( bytes + bytes / 4, size_t( 1 ) << 20 );       // grow with headroom: sizes creep call by call
 		CK( cudaMalloc( &ctx->workspace, bytes ), "workspace alloc" );
 		ctx->workspace_bytes = bytes;
-		ctx->seg_key.valid = false;
 		}
 	// one scratch area for every stream: a call on another stream than the last user's waits for that user
 	if( ctx->ws_recorded && ctx->ws_stream != ctx->compute ) CK( cudaStreamWaitEvent( ctx->compute, ctx->ws_event, 0 ), "workspace wait" );
@@ -406,7 +407,6 @@ int analysis_range( flan_b200_ctx * ctx, const AnalysisCall & c )
 		void * ws = nullptr;
 		rc = get_workspace( ctx, (size_t)( geo.blocks * geo.scratch_stride ), &ws );
 		if( rc ) return rc;
-		ctx->seg_key.valid = false;
 		ga.scratch = (unsigned char *) ws; ga.scratch_stride = geo.scratch_stride; ga.fft_in_smem = geo.fft_in_smem;
 		{ LaunchTimer lt( ctx, 0 ); CK( launch_generic_analysis( ga, geo, ctx->compute ), "analysis launch" ); }
 		return FLAN_B200_OK;
@@ -436,7 +436,6 @@ int analysis_range( flan_b200_ctx * ctx, const AnalysisCall & c )
 		*c.wave_out = ctx->sms * std::max( 1, last_occupancy() );
 		return FLAN_B200_OK;
 		}
-	ctx->seg_key.valid = false;
 	// Summaries for a resynthesis of these rows as they are (flan_b200_hint_resynthesis): the 16-point full-window kernel
 	// leaves them in the workspace, in the segments resynthesis will use; anything else ignores the hint.
 	// (a frame range without emit_seg_len is a shard of a per-GPU process: its resynthesis chooses the segments from the
@@ -454,13 +453,10 @@ int analysis_range( flan_b200_ctx * ctx, const AnalysisCall & c )
 			seg_len = lay.seg_len; segs = lay.segs;
 			a.seg_len = seg_len; a.segs_per_channel = segs;
 			a.seg_out = (PhaseSeg *) ws; a.P = plan->host.P; a.rcpP = plan->host.rcpP;
-			CK( cudaMemsetAsync( ctx->d_flags + flan_b200_ctx::FLAG_SLOTS + 1, 0, sizeof( int ), ctx->compute ), "flag clear" );
+			CK( cudaMemsetAsync( ctx->summaries.nan_flag, 0, sizeof( int ), ctx->compute ), "flag clear" );
 			{ LaunchTimer lt( ctx, 0 ); CK( launch_analysis( N, a, (int64_t) C * segs, ctx->compute, tps_a, pt ), "analysis launch" ); }
-			flan_b200_ctx::SegKey key;
-			key.pv = c.d_pv_rows; key.stride = c.pv_channel_stride; key.fb = c.frame_begin; key.fe = c.frame_end;
-			key.C = C; key.B = B; key.W = W; key.seg_len = seg_len; key.sr = fbits( c.sr ); key.ar = fbits( flan_b200_analysis_rate( c.sr, hop ) );
-			key.valid = true; key.nan_known = true; key.needs_fix = true;
-			ctx->seg_key = key;
+			ctx->summaries.publish( { c.d_pv_rows, c.pv_channel_stride, c.frame_begin, c.frame_end, C, B, W, seg_len, c.sr, flan_b200_analysis_rate( c.sr, hop ) },
+			                        { /* needs_fix */ true, /* nan_known */ true } );
 			return FLAN_B200_OK;
 			}
 		}
@@ -480,6 +476,7 @@ int analysis_range( flan_b200_ctx * ctx, const AnalysisCall & c )
 			a.seg_len = seg_len; a.segs_per_channel = segs;
 			}
 		}
+	ctx->summaries.drop();          // new rows, no summaries of them
 	{ LaunchTimer lt( ctx, 0 ); CK( launch_analysis( N, a, (int64_t) C * segs, ctx->compute, tps_a, pt ), "analysis launch" ); }
 	return FLAN_B200_OK;
 	}
@@ -493,11 +490,15 @@ int64_t ctas_per_slice( int64_t ctas, int64_t wave, size_t copy_bytes )
 	return ( ( waves + n - 1 ) / n ) * wave;
 	}
 
+int resynthesis_seg_len( const flan_b200_ctx * ctx, int C, int64_t frames, int N, int W, int hop )
+	{
+	return choose_seg_len( frames, C, ctx->sms, W, hop, seg_len_cap( ctx, N ), false, synth_ctas_per_sm( N ) );
+	}
+
 PhaseLayout phase_layout( const flan_b200_ctx * ctx, int C, int64_t frames, int B, int W, int hop, int seg_len_given )
 	{
 	PhaseLayout l{};
-	const int N = ( B - 1 ) * 2;
-	int seg_len = seg_len_given ? seg_len_given : choose_seg_len( frames, C, ctx->sms, W, hop, seg_len_cap( ctx, N ), false, synth_ctas_per_sm( N ) );
+	int seg_len = seg_len_given ? seg_len_given : resynthesis_seg_len( ctx, C, frames, ( B - 1 ) * 2, W, hop );
 	if( seg_len > frames ) seg_len = (int) frames;
 	if( seg_len < 1 ) seg_len = 1;
 	l.seg_len = seg_len;
@@ -510,6 +511,20 @@ PhaseLayout phase_layout( const flan_b200_ctx * ctx, int C, int64_t frames, int 
 	l.grp_bytes = align_up( sizeof( PhaseSeg ) * (size_t) C * l.groups * B, 256 );
 	return l;
 	}
+
+bool PhaseSummaries::Key::operator==( const Key & o ) const
+	{
+	return pv == o.pv && channel_stride == o.channel_stride && frame_begin == o.frame_begin && frame_end == o.frame_end
+	    && C == o.C && B == o.B && W == o.W && seg_len == o.seg_len && fbits( sr ) == fbits( o.sr ) && fbits( ar ) == fbits( o.ar );
+	}
+void PhaseSummaries::publish( const Key & key, const Source & source ) { key_ = key; source_ = source; valid_ = true; }
+std::optional<PhaseSummaries::Source> PhaseSummaries::match( const Key & key, bool need_nan_flag ) const
+	{
+	if( !valid_ || !( key_ == key ) || ( need_nan_flag && !source_.nan_known ) ) return std::nullopt;
+	return source_;
+	}
+void PhaseSummaries::drop() { valid_ = false; }
+void PhaseSummaries::drop_if_within( const Block & b ) { if( (uintptr_t) key_.pv >= (uintptr_t) b.ptr && (uintptr_t) key_.pv < (uintptr_t) b.ptr + b.bytes ) drop(); }
 
 // The promise of flan_b200_promise_unchanged, per calling thread: the next whole-signal resynthesis of exactly this
 // buffer may use the phase summaries its producer left in the workspace.
@@ -545,6 +560,10 @@ int synth_range( flan_b200_ctx * ctx, const SynthCall & s )
 	const PhaseLayout lay = phase_layout( ctx, C, frames, B, W, hop, s.seg_len );
 	const int seg_len = lay.seg_len, segs = lay.segs, group_len = lay.group_len, groups = lay.groups;
 	const size_t seg_bytes = lay.seg_bytes, acc_bytes = lay.acc_bytes, grp_bytes = lay.grp_bytes;
+	// summaries a producer left of exactly these rows, taken before get_workspace drops the record (summaries whose
+	// NaN / Inf flag is gone cannot serve a caller that asks for the flag), and forgotten if the workspace had to grow
+	const PhaseSummaries::Key key{ s.d_pv_rows, s.pv_channel_stride, s.frame_begin, s.frame_end, C, B, W, seg_len, s.sr, s.ar };
+	std::optional<PhaseSummaries::Source> held = s.reuse_summary ? ctx->summaries.match( key, s.d_nan_flag != nullptr ) : std::nullopt;
 	GenericSynthArgs ga{};
 	GenericGeometry geo{};
 	if( plan->generic )       // the per-CTA slabs of the run-time-sized transform go behind the phase scratch
@@ -554,31 +573,22 @@ int synth_range( flan_b200_ctx * ctx, const SynthCall & s )
 		}
 	const size_t phase_bytes = seg_bytes + acc_bytes + grp_bytes;
 	void * ws = nullptr;
-	rc = get_workspace( ctx, phase_bytes + (size_t)( geo.blocks * geo.scratch_stride ), &ws );
+	bool kept = false;
+	rc = get_workspace( ctx, phase_bytes + (size_t)( geo.blocks * geo.scratch_stride ), &ws, &kept );
 	if( rc ) return rc;
+	if( !kept ) held.reset();       // a new allocation: what the producer left is gone
 	ga.scratch = (unsigned char *) ws + phase_bytes; ga.scratch_stride = geo.scratch_stride; ga.fft_in_smem = geo.fft_in_smem;
 	PhaseSeg * d_seg = (PhaseSeg *) ws;
 	double * d_acc = (double *)( (char *) ws + seg_bytes );
 	PhaseSeg * d_grp = (PhaseSeg *)( (char *) ws + seg_bytes + acc_bytes );
 
-	flan_b200_ctx::SegKey key;
-	key.pv = s.d_pv_rows; key.stride = s.pv_channel_stride; key.fb = s.frame_begin; key.fe = s.frame_end;
-	key.C = C; key.B = B; key.W = W; key.seg_len = seg_len; key.sr = fbits( s.sr ); key.ar = fbits( s.ar ); key.valid = true;
-	const flan_b200_ctx::SegKey & old = ctx->seg_key;
-	// summaries whose NaN / Inf flag is gone cannot serve a caller that asks for the flag
-	const bool have_summaries = s.reuse_summary && ( !s.d_nan_flag || old.nan_known ) && old.valid && old.pv == key.pv && old.stride == key.stride && old.fb == key.fb
-	                         && old.fe == key.fe && old.C == key.C && old.B == key.B && old.W == key.W && old.seg_len == key.seg_len && old.sr == key.sr && old.ar == key.ar;
-	const bool old_group_prefix = old.group_prefix, old_nan_known = old.nan_known, old_needs_fix = old.needs_fix;
-	ctx->seg_key = key;
-
 	PhaseSegArgs sa{};
 	sa.pv = (const float2 *) s.d_pv_rows; sa.pv_channel_stride = s.pv_channel_stride;
 	sa.frame_begin = s.frame_begin; sa.frame_end = s.frame_end;
 	sa.seg_len = seg_len; sa.segs_per_channel = segs; sa.B = B;
-	sa.seg_out = d_seg; sa.nan_flag = s.d_nan_flag ? s.d_nan_flag : ctx->d_flags + flan_b200_ctx::FLAG_SLOTS;   // last slot + 1: write-only scratch
+	sa.seg_out = d_seg; sa.nan_flag = s.d_nan_flag ? s.d_nan_flag : ctx->summaries.sink;
 	sa.k = plan->host.k; sa.P = plan->host.P; sa.rcpP = plan->host.rcpP;
-	if( !have_summaries ) { LaunchTimer lt( ctx, 1 ); CK( launch_phase_seg( sa, C, ctx->compute ), "phase summary launch" ); }
-	else ctx->seg_key.nan_known = old_nan_known;
+	if( !held ) { LaunchTimer lt( ctx, 1 ); CK( launch_phase_seg( sa, C, ctx->compute ), "phase summary launch" ); }
 
 	PhaseScanArgs sc{};
 	sc.seg = d_seg; sc.segs_per_channel = segs; sc.B = B;
@@ -590,21 +600,23 @@ int synth_range( flan_b200_ctx * ctx, const SynthCall & s )
 	// earlier shards are known) leaves the carry-free group prefixes behind; the range call that follows on the same
 	// data then only re-walks the groups, entering each through carry (+) prefix.
 	const bool three_launches = segs > 256 || C > 65535;
-	sc.expand_only = ( have_summaries && old_group_prefix && three_launches && !s.summary_only && !s.d_carry_out ) ? 1 : 0;
+	sc.expand_only = ( held && held->group_prefix && three_launches && !s.summary_only && !s.d_carry_out ) ? 1 : 0;
 	sc.expand_carry = sc.expand_only ? s.d_carry_in : nullptr;
-	ctx->seg_key.group_prefix = s.summary_only && !s.d_carry_in && three_launches;
-	if( have_summaries && old_needs_fix )
+	if( held && held->needs_fix )
 		{
 		// summaries of the analysis kernel: the group reduction recomputes the entries it marked (the lowest bins, NaN / Inf)
 		if( !three_launches || sc.expand_only ) return fail( ctx, FLAN_B200_INVALID, "internal: marked summaries need the three-launch scan" );
 		sc.fix_pv = (const float2 *) s.d_pv_rows; sc.fix_channel_stride = s.pv_channel_stride;
 		sc.fix_frame_begin = s.frame_begin; sc.fix_frame_end = s.frame_end; sc.fix_seg_len = seg_len;
-		sc.fix_k = plan->host.k; sc.fix_nan_flag = ctx->d_flags + flan_b200_ctx::FLAG_SLOTS + 1;
+		sc.fix_k = plan->host.k; sc.fix_nan_flag = ctx->summaries.nan_flag;
 		}
 	{ LaunchTimer lt( ctx, 2 ); CK( launch_phase_scan( sc, C, ctx->compute ), "phase scan launch" );
 	  ctx->launches += three_launches ? ( sc.expand_only ? 0 : ( s.summary_only ? 1 : 2 ) ) : 0; }     // launch_phase_scan: one launch for short signals, else 1 to 3
-	if( have_summaries && s.d_nan_flag )
-		CK( cudaMemcpyAsync( s.d_nan_flag, ctx->d_flags + flan_b200_ctx::FLAG_SLOTS + 1, sizeof( int ), cudaMemcpyDeviceToDevice, ctx->compute ), "flag copy" );
+	if( held && s.d_nan_flag )
+		CK( cudaMemcpyAsync( s.d_nan_flag, ctx->summaries.nan_flag, sizeof( int ), cudaMemcpyDeviceToDevice, ctx->compute ), "flag copy" );
+	// the summaries stay for the next call on these rows, marked entries repaired by the scan
+	ctx->summaries.publish( key, { /* needs_fix */ false, /* nan_known */ held && held->nan_known,
+	                               /* group_prefix */ s.summary_only && !s.d_carry_in && three_launches } );
 	if( s.summary_only ) return FLAN_B200_OK;
 	if( cancelled( s.cancel ) ) return fail( ctx, FLAN_B200_CANCELLED, "cancelled" );
 
@@ -791,6 +803,8 @@ int flan_b200_create( int device, flan_b200_ctx ** out )
 	if( e == cudaSuccess ) e = cudaEventCreateWithFlags( &ctx->head_fork, cudaEventDisableTiming );
 	if( e == cudaSuccess ) e = cudaEventCreateWithFlags( &ctx->head_join, cudaEventDisableTiming );
 	if( e != cudaSuccess ) { g_create_error = cudaGetErrorString( e ); flan_b200_destroy( ctx ); return FLAN_B200_CUDA; }
+	ctx->summaries.sink = ctx->d_flags + flan_b200_ctx::FLAG_SLOTS;
+	ctx->summaries.nan_flag = ctx->d_flags + flan_b200_ctx::FLAG_SLOTS + 1;
 	*out = ctx;
 	return FLAN_B200_OK;
 	}
@@ -960,7 +974,7 @@ int flan_b200_free( flan_b200_ctx * ctx, void * d_ptr )
 	if( !b.main_pending ) { cudaEventRecord( b.main_event, ctx->stream ); b.main_pending = true; b.main_stream = ctx->stream; }
 	ctx->cached.emplace( b.bytes, b );
 	ctx->cached_bytes += b.bytes;
-	if( ctx->seg_key.valid && ctx->seg_key.pv >= b.ptr && (uintptr_t) ctx->seg_key.pv < (uintptr_t) b.ptr + b.bytes ) ctx->seg_key.valid = false;
+	ctx->summaries.drop_if_within( b );
 	return FLAN_B200_OK;
 	}
 
@@ -1144,20 +1158,13 @@ int flan_b200_convert_to_audio_range( flan_b200_ctx * ctx, const float * d_pv_ro
                                       const flan_b200_phase_state * d_carry_in, int reuse_summary,
                                       float * d_out_local, int64_t out_stride, int64_t out_offset, int64_t out_len )
 	{
-	if( !ctx ) return FLAN_B200_INVALID;
-	if( !( ar > 0.0f ) || !( sr > 0.0f ) || flan_b200_hop_from_rates( sr, ar ) < 1 )
-		return fail( ctx, FLAN_B200_INVALID, "bad rates" );
-	CallLock lock( ctx );
-	BlockUse use( ctx, { d_pv_rows, d_carry_in, d_out_local } );
-	SynthCall s{ d_pv_rows, pv_channel_stride, C, frame_begin, frame_end, frames_total, B, sr, ar, W };
-	s.d_carry_in = (const PhaseSeg *) d_carry_in; s.reuse_summary = reuse_summary != 0;
-	s.d_out = d_out_local; s.out_stride = out_stride; s.out_offset = out_offset; s.out_len = out_len;
-	return synth_range( ctx, s );
+	return flan_b200_convert_to_audio_range_head( ctx, d_pv_rows, pv_channel_stride, C, frame_begin, frame_end, frames_total, B, sr, ar, W,
+	                                              d_carry_in, reuse_summary, d_out_local, out_stride, out_offset, out_len, nullptr );
 	}
 
-// The same, with the frames whose windows reach into the previous shard launched FIRST: `head_event` (a cudaEvent_t of the
-// caller) is recorded on the stream right after them, so the caller can send the window - hop partial sums at the head of
-// d_out_local to the previous rank on another stream while the rest of the frames compute.
+// The same, with the frames whose windows reach into the previous shard launched FIRST when `head_event` (a cudaEvent_t of
+// the caller) is given: it is recorded on the stream right after them, so the caller can send the window - hop partial sums
+// at the head of d_out_local to the previous rank on another stream while the rest of the frames compute.
 int flan_b200_convert_to_audio_range_head( flan_b200_ctx * ctx, const float * d_pv_rows, int64_t pv_channel_stride,
                                            int C, int64_t frame_begin, int64_t frame_end, int64_t frames_total,
                                            int B, float sr, float ar, int W,

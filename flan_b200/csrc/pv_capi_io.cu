@@ -31,7 +31,6 @@ template<class Launch> int stream_file( flan_b200_ctx * ctx, FILE * f, bool writ
 	void * ws = nullptr;
 	int rc = get_workspace( ctx, (size_t) chunk * 3 + 16, &ws );
 	if( rc ) return rc;
-	ctx->seg_key.valid = false;
 	PinnedBuf host;
 	CK( cudaMallocHost( &host.p, (size_t) chunk * 3 ), "pinned staging buffer" );
 	for( int64_t v0 = 0; v0 < values; v0 += chunk )
@@ -145,6 +144,7 @@ int flan_b200_flan_decode( flan_b200_ctx * ctx, const uint8_t * d_bytes, int64_t
 	CallLock lock( ctx );
 	BlockUse use( ctx, { d_bytes, d_pv } );
 	if( count == 0 ) return FLAN_B200_OK;
+	ctx->summaries.drop();          // new rows, written without the workspace
 	{ LaunchTimer lt( ctx, 8 ); CK( pvio::launch_flan_decode( d_bytes, count, dft_size, sr, d_pv, ctx->sms, ctx->compute ), "flan decode launch" ); }
 	return FLAN_B200_OK;
 	}

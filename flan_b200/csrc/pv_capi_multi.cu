@@ -55,8 +55,7 @@ Plan make_plan( const flan_b200_multi * m, int C, int64_t n, int W, int hop, int
 	{
 	Plan p;
 	p.F = flan_b200_num_frames( n, hop );
-	const int cap = ( N >= 2048 ? 128 : 64 );
-	p.seg_len = choose_seg_len( p.F, C, m->ctx[0]->sms, W, hop, cap, false, synth_ctas_per_sm( N ) );
+	p.seg_len = resynthesis_seg_len( m->ctx[0], C, p.F, N, W, hop );
 	const int64_t reach = 2 * (int64_t)( ( W + hop - 1 ) / hop );
 	const int64_t min_frames = std::max<int64_t>( p.seg_len, ( reach + p.seg_len - 1 ) / p.seg_len * p.seg_len );
 	const int64_t segs = ( p.F + p.seg_len - 1 ) / p.seg_len;
@@ -324,11 +323,9 @@ int flan_b200_multi_convert_to_audio( flan_b200_multi * m, const flan_b200_shard
 	const int C = pv->channels, B = pv->bins, W = pv->window_size, R = pv->shards;
 	const float sr = pv->sample_rate, ar = pv->analysis_rate;
 	const int hop = flan_b200_hop_from_rates( sr, ar );
-	const int N = ( B - 1 ) * 2;
 	if( hop < 1 || C < 1 || B < 2 ) return mfail( FLAN_B200_INVALID, "bad PV format" );
 	const int64_t F = pv->frames;
-	const int cap = ( N >= 2048 ? 128 : 64 );
-	const int seg_len = choose_seg_len( F, C, m->ctx[0]->sms, W, hop, cap, false, synth_ctas_per_sm( N ) );
+	const int seg_len = resynthesis_seg_len( m->ctx[0], C, F, ( B - 1 ) * 2, W, hop );
 	for( int i = 1; i < R; ++i )
 		if( pv->frame_begin[i] % seg_len != 0 ) return mfail( FLAN_B200_INVALID, "shards must begin at multiples of the signal's segment length" );
 	*out = flan_b200_sharded_audio{};
@@ -529,6 +526,7 @@ int flan_b200_multi_gather_pv( flan_b200_multi * m, const flan_b200_sharded_pv *
 			{
 			flan_b200_ctx * dst = m->ctx[to];
 			CallLock cd( dst );
+			dst->summaries.drop();      // new rows in d_pv, written without the workspace
 			MCK( cudaStreamWaitEvent( dst->stream, m->ev_done[i], 0 ), "stream wait" );
 			for( int c = 0; c < C; ++c )
 				MCK( cudaMemcpyPeerAsync( d_pv + 2 * ( (int64_t) c * F + pv->frame_begin[i] ) * B, dst->device,

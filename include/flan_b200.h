@@ -237,9 +237,11 @@ int flan_b200_modify_time( flan_b200_ctx * ctx, const float * d_pv, int channels
                            int interp, int64_t out_frames, float * d_pv_out, int summary_window );
 /* summary_window > 0 (the PV's window size): when the time map is shared by all bins and never descends (PV::stretch with
  * a constant or time-only factor) the kernel walks its output frames in order and ALSO leaves behind the per-segment
- * phase summaries that flan_b200_convert_to_audio would otherwise compute with a second read of the rows. They stay
- * valid until the next call on this context that uses its scratch space or writes the buffer. A caller that knows d_pv is
- * unchanged since the call that produced it says so right before resynthesis (same host thread): */
+ * phase summaries that flan_b200_convert_to_audio would otherwise compute with a second read of the rows. The context
+ * holds the summaries of one set of rows at a time. They are dropped by the next call on this context that uses its
+ * scratch space or writes PV rows, and by flan_b200_free of their buffer. A write by other means (a copy, a kernel of the
+ * caller) is not seen. A caller that knows d_pv is unchanged since the call that produced it says so right before
+ * resynthesis (same host thread): */
 int flan_b200_promise_unchanged( flan_b200_ctx * ctx, const float * d_pv );
 /* The producer can also be the analysis itself: after this hint (same host thread) the next flan_b200_convert_to_pv also
  * leaves the phase summaries of the rows it writes, for a caller that will resynthesise them as they are -- the round trip
@@ -350,6 +352,11 @@ int  flan_b200_multi_convert_to_pv( flan_b200_multi * m, const flan_b200_sharded
                                     int window_size, int hop, int dft_size, flan_b200_sharded_pv * pv_out );
 /* PV::convert_to_audio (AudioPV.cpp:86-139) over the shards, with the phase-state and halo exchange. */
 int  flan_b200_multi_convert_to_audio( flan_b200_multi * m, const flan_b200_sharded_pv * pv, flan_b200_sharded_audio * audio_out );
+/* flan_b200_hint_resynthesis and flan_b200_promise_unchanged for the sharded forms (same host thread): after the hint the
+ * next flan_b200_multi_convert_to_pv also leaves every shard's phase summaries, in the segments of the whole signal; the
+ * promise that pv is unchanged since then lets the next flan_b200_multi_convert_to_audio use them. */
+int  flan_b200_multi_hint_resynthesis( flan_b200_multi * m );
+int  flan_b200_multi_promise_unchanged( flan_b200_multi * m, const flan_b200_sharded_pv * pv );
 /* Final samples of every shard -> host float[channels][n] (returns when the bytes have arrived). */
 int  flan_b200_multi_gather_audio( flan_b200_multi * m, const flan_b200_sharded_audio * audio, float * h_audio );
 /* PV rows of every shard -> host MF[channels][frames][bins] (h_pv, synchronous) and / or one device buffer of that layout

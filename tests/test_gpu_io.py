@@ -132,3 +132,32 @@ def test_cpp_api_files_either_side_of_the_path(oracle, tmp_path):
     assert np.max(np.abs(lpv[..., 0] - q[..., 0])[loud]) <= 1e-4 * ref_pv[..., 0].max()
     ref_out = oracle.convert_to_audio(lpv, sr, oracle.analysis_rate(sr, h), W)
     assert np.max(np.abs(out - ref_out)) <= 1e-5
+
+
+def test_flan_decode_drops_the_summaries_of_the_rows_it_overwrites(eng):
+    """flan_decode writes rows without the scratch space. Summaries an analysis left for the same buffer must not survive
+    it: a promise that the rows are unchanged since the last call that wrote them is then true, and resynthesis must read
+    the decoded rows."""
+    import torch
+    sr, N, hop = 48000.0, 4096, 256
+    n = int(sr * 200)
+    xd = torch.from_numpy(np.stack([noise_chirp(n, sr, 3), noise_chirp(n, sr, 5)])).cuda()
+    ar = eng.analysis_rate(sr, hop)
+    F, B = eng.num_frames(n, hop), N // 2 + 1
+    other = eng.flan_encode(eng.convert_to_pv(xd.flip(1).contiguous(), sr, N, hop, N), sr)
+    pv = torch.empty((2, F, B, 2), dtype=torch.float32, device="cuda")
+    eng.convert_to_pv(xd, sr, N, hop, N, out=pv, for_resynthesis=True)
+    # the summaries are recorded: a promised resynthesis saves the phase summary launch (and publishes them again)
+    n0 = eng.launch_count()
+    eng.convert_to_audio(pv, sr, ar, N, unchanged=True)
+    n_promised = eng.launch_count() - n0
+    n0 = eng.launch_count()
+    eng.convert_to_audio(pv, sr, ar, N)
+    n_plain = eng.launch_count() - n0
+    assert n_promised == n_plain - 1
+    eng._bind_stream()
+    eng.ctx.call("flan_b200_flan_decode", eng._chk(other, torch.uint8), 2 * F * B, float(N), sr, eng._chk(pv))
+    n0 = eng.launch_count()
+    after = eng.convert_to_audio(pv, sr, ar, N, unchanged=True)
+    assert eng.launch_count() - n0 == n_plain, "the rows were overwritten: nothing to reuse"
+    assert torch.equal(after, eng.convert_to_audio(pv, sr, ar, N))

@@ -224,3 +224,69 @@ def test_stretch_leaves_the_phase_summaries_resynthesis_needs(eng, factor, frame
     st3 = eng.stretch(pv, sr, ar, factor, 0, summary_window=W)
     assert torch.equal(eng.convert_to_audio(plain_st, sr, ar, W, unchanged=True), plain)
     del st3
+
+
+def test_modify_time_per_bin_drops_the_summaries_of_the_rows_it_overwrites(eng):
+    """The per-bin walk of modify_time writes rows without the scratch space. Summaries a stretch left for the same buffer
+    must not survive it: a promise that the rows are unchanged since the last call that wrote them is then true, and
+    resynthesis must read the new rows."""
+    import ctypes
+    import torch
+    sr, W, hop, B, F = 48000.0, 2048, 128, 1025, 3000
+    ar = eng.analysis_rate(sr, hop)
+    g = torch.Generator(device="cuda").manual_seed(9)
+    pv = torch.rand((2, F, B, 2), generator=g, device="cuda", dtype=torch.float32)
+    pv[..., 1] *= 20000.0
+    # a per-bin (B, 1) map that never descends and has the same maximum, hence the same output frame count (made first:
+    # stretch_map uses the scratch space)
+    seconds = eng.stretch_map(F, B, sr, ar, 2.0)
+    scale = torch.linspace(0.9, 1.0, B, device="cuda")
+    scale[-1] = 1.0
+    per_bin = (seconds * scale[None, :]).contiguous()
+    frames = ctypes.c_int64(0)
+    eng.ctx.call("flan_b200_modify_time_frames", eng._chk(per_bin), B, 1, F, B, sr, ar, ctypes.byref(frames))
+    Y = eng.stretch(pv, sr, ar, 2.0, 0, summary_window=W)
+    before = Y.clone()
+    assert frames.value == Y.shape[1]
+    # the summaries are recorded: a promised resynthesis saves the phase summary launch (and publishes them again)
+    n0 = eng.launch_count()
+    eng.convert_to_audio(Y, sr, ar, W, unchanged=True)
+    n_promised = eng.launch_count() - n0
+    n0 = eng.launch_count()
+    eng.convert_to_audio(Y, sr, ar, W)
+    n_plain = eng.launch_count() - n0
+    assert n_promised == n_plain - 1
+    eng.ctx.call("flan_b200_modify_time", eng._chk(pv), 2, F, B, sr, ar, eng._chk(per_bin), B, 1, 0, frames.value,
+                 eng._chk(Y), 0)
+    assert not torch.equal(Y, before)
+    n0 = eng.launch_count()
+    after = eng.convert_to_audio(Y, sr, ar, W, unchanged=True)
+    assert eng.launch_count() - n0 == n_plain, "the rows were overwritten: nothing to reuse"
+    assert torch.equal(after, eng.convert_to_audio(Y, sr, ar, W))
+
+
+def test_stretch_summaries_are_not_used_after_the_workspace_grows():
+    """At a dft size of the run-time-sized transform (16384) resynthesis needs per-CTA slabs of scratch beside the phase
+    summaries, more than the stretch asked for. On a fresh context the workspace then grows and loses what the stretch
+    left: the promised resynthesis computes the summaries again (as many launches as the plain one) and gives the same
+    bits. Once the workspace is large enough, the same promise saves the phase summary launch."""
+    import torch
+    from flan_b200.engine import Engine
+    e = Engine(0)           # a context of its own: its workspace is sized by the calls below only
+    sr, W, hop, B, F = 48000.0, 16384, 1024, 8193, 400
+    ar = e.analysis_rate(sr, hop)
+    g = torch.Generator(device="cuda").manual_seed(13)
+    pv = torch.rand((1, F, B, 2), generator=g, device="cuda", dtype=torch.float32)
+    pv[..., 1] *= 20000.0
+    st = e.stretch(pv, sr, ar, 2.0, 0, summary_window=W)
+    n0 = e.launch_count()
+    promised = e.convert_to_audio(st, sr, ar, W, unchanged=True)
+    n_promised = e.launch_count() - n0
+    n0 = e.launch_count()
+    plain = e.convert_to_audio(st, sr, ar, W)
+    assert e.launch_count() - n0 == n_promised, "the workspace grew: the summaries must be computed again"
+    assert torch.equal(promised, plain)
+    st2 = e.stretch(pv, sr, ar, 2.0, 0, summary_window=W)
+    n0 = e.launch_count()
+    assert torch.equal(e.convert_to_audio(st2, sr, ar, W, unchanged=True), plain)
+    assert e.launch_count() - n0 == n_promised - 1, "the workspace kept the summaries: one launch fewer"
