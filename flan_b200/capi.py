@@ -112,6 +112,9 @@ SYMBOLS = [
     ("flan_b200_multi_promise_unchanged", _int, [_vp, _pp]),
     ("flan_b200_multi_gather_audio", _int, [_vp, _pa, _vp]),
     ("flan_b200_multi_gather_pv", _int, [_vp, _pp, _vp, _int, _vp]),
+    ("flan_b200_multi_repitch", _int, [_vp, _pp, _vp, _i64, _int, _int, _pp]),
+    ("flan_b200_multi_stretch", _int, [_vp, _pp, _vp, _i64, _int, _int, _pp]),
+    ("flan_b200_multi_modify_time", _int, [_vp, _pp, _vp, _i64, _int, _int, _pp]),
     ("flan_b200_multi_free_audio", _int, [_vp, _pa]),
     ("flan_b200_multi_free_pv", _int, [_vp, _pp]),
     ("flan_b200_multi_convert_to_pv_host", _int, [_vp, _vp, _int, _i64, _f, _int, _int, _int, _pp]),

@@ -97,9 +97,11 @@ int pv_emu_repitch( const float * pv, int C, int64_t F, int B, float sr, const f
 
 // factor != null: PV::stretch (the map is built first); else map_seconds is the time map of PV::modify_time.
 // out == null: returns the output frame count only. force_sequential exercises the reference-order walk.
-int64_t pv_emu_stretch( const float * pv, int C, int64_t F, int B, float sr, float ar, const float * factor,
-                        const float * map_seconds, int64_t fs, int bs, int interp, int chunk, int force_sequential,
-                        int * used_sequential, float * out )
+// n_cuts > 0 (planned form only): the output is computed shard by shard, cut at cuts[0 .. n_cuts] (0, ..., out_frames);
+// used_rows (may be null) receives each shard's input row window.
+int64_t pv_emu_stretch_sharded( const float * pv, int C, int64_t F, int B, float sr, float ar, const float * factor,
+                                const float * map_seconds, int64_t fs, int bs, int interp, int chunk, int force_sequential,
+                                int * used_sequential, float * out, const int64_t * cuts, int n_cuts, int64_t * used_rows )
 	{
 	if( !strides_ok( fs, bs, B ) ) return -1;
 	const int hop = (int)( sr / ar );
@@ -134,7 +136,45 @@ int64_t pv_emu_stretch( const float * pv, int C, int64_t F, int B, float sr, flo
 	a.F = F; a.out_frames = out_frames; a.B = B; a.sample_rate = sr; a.hop = float( hop ); a.interp = interp;
 	a.chunk = chunk; a.chunks = ( F - 1 + chunk - 1 ) / chunk;
 	if( a.chunks < 1 ) a.chunks = 1;
-	if( !descends && !force_sequential && bs == 0 )
+	a.pv_channel_stride = F * B; a.out_channel_stride = out_frames * B;
+	if( !descends && !force_sequential && bs == 0 && n_cuts > 0 )
+		{
+		// as flan_b200_multi_stretch / _modify_time: the plan of the whole signal, then per output shard
+		// [cuts[i], cuts[i+1]) (multiples of seg_len) its row window (stretch_window) staged into a buffer of its own and
+		// the shard's segments written into another. Rows outside the window and cells outside the shard are NaN, so a read
+		// or write past them changes the result.
+		const int seg_len = chunk;
+		if( cuts[0] != 0 || cuts[n_cuts] != out_frames ) return -3;
+		std::vector<int> xpos( F ); std::vector<float> mix( out_frames ); std::vector<int> src( out_frames, -1 );
+		StretchPlan plan{ xpos.data(), mix.data(), src.data() };
+		for( int64_t f = F - 1; f >= 0; --f ) stretch_plan_frame( a, plan, f );
+		pvk::PvConsts k{};
+		const float nan = std::nanf( "" );
+		constexpr int64_t GUARD = 2;
+		for( int s = n_cuts - 1; s >= 0; --s )
+			{
+			const int64_t x0 = cuts[s], x1 = cuts[s + 1];
+			if( x1 < x0 || x0 % seg_len != 0 ) return -3;
+			int64_t r0 = 0, r1 = 0;
+			stretch_window( plan, F, x0, x1, &r0, &r1 );
+			if( used_rows ) { used_rows[2 * s] = r0; used_rows[2 * s + 1] = r1; }
+			const int64_t rows = r1 - r0, in_stride = ( rows + 2 * GUARD ) * B, out_stride = ( x1 - x0 ) * B;
+			std::vector<float2> win( (size_t)( C * in_stride ), make_float2( nan, nan ) ), part( (size_t)( C * out_stride ), make_float2( nan, nan ) );
+			for( int c = 0; c < C; ++c )
+				std::memcpy( win.data() + c * in_stride + GUARD * B, (const float2 *) pv + ( c * F + r0 ) * B, sizeof( float2 ) * rows * B );
+			StretchArgs sa = a;
+			sa.pv = win.data() + GUARD * B; sa.row0 = r0; sa.pv_channel_stride = in_stride;
+			sa.out = part.data(); sa.out_row0 = x0; sa.out_channel_stride = out_stride;
+			sa.seg0 = x0 / seg_len;
+			const int64_t segs = ( x1 - x0 + seg_len - 1 ) / seg_len;
+			for( int c = C - 1; c >= 0; --c )
+				for( int64_t sgm = segs - 1; sgm >= 0; --sgm )
+					for( int b = B - 1; b >= 0; --b ) stretch_segment_planned<false>( sa, plan, c, sgm, seg_len, b, nullptr, k );
+			for( int c = 0; c < C; ++c )
+				std::memcpy( (float2 *) out + ( c * out_frames + x0 ) * B, part.data() + c * out_stride, sizeof( float2 ) * out_stride );
+			}
+		}
+	else if( !descends && !force_sequential && bs == 0 )
 		{
 		// as on the device: plan, then the gather by segments of output frames (`chunk` doubles as the segment length here,
 		// so the tests cut segments inside pairs, at pair boundaries and beyond the covered range)
@@ -161,6 +201,14 @@ int64_t pv_emu_stretch( const float * pv, int C, int64_t F, int B, float sr, flo
 			for( int b = 0; b < B; ++b ) stretch_column( a, c, b );
 		}
 	return out_frames;
+	}
+
+int64_t pv_emu_stretch( const float * pv, int C, int64_t F, int B, float sr, float ar, const float * factor,
+                        const float * map_seconds, int64_t fs, int bs, int interp, int chunk, int force_sequential,
+                        int * used_sequential, float * out )
+	{
+	return pv_emu_stretch_sharded( pv, C, F, B, sr, ar, factor, map_seconds, fs, bs, interp, chunk, force_sequential,
+	                               used_sequential, out, nullptr, 0, nullptr );
 	}
 
 }

@@ -50,6 +50,10 @@ int repitch_common( flan_b200_ctx * ctx, const float * d_pv, int C, int64_t F, i
 
 size_t repitch_plan_bytes( int B ) { return align_up( sizeof( float ) * 2 * (size_t) B + sizeof( int ), 256 ); }
 
+} // namespace
+
+namespace pvrt {
+
 // Reads the reduction back (synchronises the stream).
 int read_map_check( flan_b200_ctx * ctx, float sr, int hop, int64_t * out_frames, bool * descends )
 	{
@@ -63,7 +67,7 @@ int read_map_check( flan_b200_ctx * ctx, float sr, int hop, int64_t * out_frames
 	return FLAN_B200_OK;
 	}
 
-} // namespace
+} // namespace pvrt
 
 extern "C" {
 
@@ -179,6 +183,7 @@ int flan_b200_modify_time( flan_b200_ctx * ctx, const float * d_pv, int C, int64
 	a.pv = (const float2 *) d_pv; a.out = (float2 *) d_pv_out; a.mod = mod;
 	a.F = F; a.out_frames = out_frames; a.B = B;
 	a.sample_rate = sr; a.hop = float( hop ); a.interp = interp;
+	a.pv_channel_stride = F * B; a.out_channel_stride = out_frames * B;
 	a.chunk = 32;
 	a.chunks = ( F - 1 + a.chunk - 1 ) / a.chunk;
 	if( a.chunks < 1 ) a.chunks = 1;

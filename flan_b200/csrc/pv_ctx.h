@@ -316,4 +316,8 @@ struct AnalysisCall
 	};
 int analysis_range( flan_b200_ctx * ctx, const AnalysisCall & a );
 
+// The time-map reduction of pvm::launch_map_check, read back (synchronises the calling stream): the output frame count
+// of PV::modify_time (PVModify.cpp:312) and whether some column of the map descends.
+int read_map_check( flan_b200_ctx * ctx, float sr, int hop, int64_t * out_frames, bool * descends );
+
 } // namespace pvrt

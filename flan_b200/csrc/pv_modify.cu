@@ -248,17 +248,45 @@ cudaError_t launch_repitch_shared( const RepitchArgs & a, const RepitchPlan & pl
 	return launch_repitch_shared_t<1024>( a, plan, hz, rows, sms, st );
 	}
 
-cudaError_t launch_stretch_planned( const StretchArgs & a, const StretchPlan & plan, const StretchSummary & summ, int C, cudaStream_t st )
+__global__ void pv_stretch_window_kernel( const StretchPlan plan, int64_t F, const StretchWindows w, int64_t * rows )
+	{
+	const int i = threadIdx.x;
+	if( i < w.n ) stretch_window( plan, F, w.xb[i], w.xb[i + 1], rows + 2 * i, rows + 2 * i + 1 );
+	}
+
+cudaError_t launch_stretch_plan( const StretchArgs & a, const StretchPlan & plan, cudaStream_t st )
+	{
+	cudaError_t e = cudaMemsetAsync( plan.src, 0xff, sizeof( int ) * (size_t) a.out_frames, st );      // -1: no pair covers the frame
+	if( e != cudaSuccess ) return e;
+	pv_stretch_plan_kernel<<<(unsigned)( ( a.F + 127 ) / 128 ), 128, 0, st>>>( a, plan );
+	return cudaGetLastError();
+	}
+
+cudaError_t launch_stretch_windows( const StretchPlan & plan, int64_t F, const StretchWindows & w, int64_t * rows, cudaStream_t st )
+	{
+	if( w.n < 1 || w.n > StretchWindows::MAX ) return cudaErrorInvalidValue;
+	pv_stretch_window_kernel<<<1, 32, 0, st>>>( plan, F, w, rows );
+	return cudaGetLastError();
+	}
+
+cudaError_t launch_stretch_segments( const StretchArgs & a, const StretchPlan & plan, const StretchSummary & summ, int C, cudaStream_t st )
 	{
 	const int bin_tiles = ( a.B + 127 ) / 128;
 	const int64_t blocks = (int64_t) summ.segs_per_channel * bin_tiles;
 	if( blocks > 0x7fffffff || summ.seg_len < 1 ) return cudaErrorInvalidValue;
-	cudaError_t e = cudaMemsetAsync( plan.src, 0xff, sizeof( int ) * (size_t) a.out_frames, st );      // -1: no pair covers the frame
-	if( e != cudaSuccess ) return e;
-	pv_stretch_plan_kernel<<<(unsigned)( ( a.F + 127 ) / 128 ), 128, 0, st>>>( a, plan );
+	if( blocks == 0 ) return cudaSuccess;
 	if( summ.seg_out ) pv_stretch_planned_kernel<true><<<dim3( (unsigned) blocks, C ), 128, 0, st>>>( a, plan, summ, bin_tiles );
 	else pv_stretch_planned_kernel<false><<<dim3( (unsigned) blocks, C ), 128, 0, st>>>( a, plan, summ, bin_tiles );
 	return cudaGetLastError();
+	}
+
+cudaError_t launch_stretch_planned( const StretchArgs & a, const StretchPlan & plan, const StretchSummary & summ, int C, cudaStream_t st )
+	{
+	const int bin_tiles = ( a.B + 127 ) / 128;
+	if( (int64_t) summ.segs_per_channel * bin_tiles > 0x7fffffff || summ.seg_len < 1 ) return cudaErrorInvalidValue;
+	const cudaError_t e = launch_stretch_plan( a, plan, st );
+	if( e != cudaSuccess ) return e;
+	return launch_stretch_segments( a, plan, summ, C, st );
 	}
 
 cudaError_t launch_bin_prefix( const Table & factor, int64_t rows, int B, float sample_rate, float dft, float * out, cudaStream_t st )

@@ -31,6 +31,13 @@ struct StretchSummary
 	pvk::PvConsts k; double P, rcpP;
 	};
 cudaError_t launch_stretch_planned( const StretchArgs & a, const StretchPlan & plan, const StretchSummary & summ, int C, cudaStream_t st );
+// ... and its two halves, for output shards (pv_capi_multi.cu): the plan of the whole signal, then the segments
+// a.seg0 .. a.seg0 + summ.segs_per_channel - 1 from the row windows that StretchArgs describes.
+cudaError_t launch_stretch_plan( const StretchArgs & a, const StretchPlan & plan, cudaStream_t st );
+cudaError_t launch_stretch_segments( const StretchArgs & a, const StretchPlan & plan, const StretchSummary & summ, int C, cudaStream_t st );
+// Output shards [xb[i], xb[i+1]) -> rows[2i], rows[2i+1]: the input rows each one reads (stretch_window), device memory.
+struct StretchWindows { static constexpr int MAX = 16; int n; int64_t xb[MAX + 1]; };
+cudaError_t launch_stretch_windows( const StretchPlan & plan, int64_t F, const StretchWindows & w, int64_t * rows, cudaStream_t st );
 cudaError_t launch_stretch_parallel( const StretchArgs & a, int C, cudaStream_t st );
 cudaError_t launch_stretch_sequential( const StretchArgs & a, int C, cudaStream_t st );
 

@@ -429,6 +429,13 @@ struct StretchArgs
 	int interp;
 	int chunk;                  // frame pairs per thread in the parallel form
 	int64_t chunks;
+	// Planned form only: a window of the rows, so that one launch writes the segments of one output shard (pv_capi_multi.cu).
+	// pv holds input frames [row0, ...) with pv_channel_stride MF between channels, out holds output frames
+	// [out_row0, ...) with out_channel_stride; the launch's segments are seg0, seg0 + 1, ... Whole signal: 0, F * B, 0,
+	// out_frames * B, 0.
+	int64_t row0, pv_channel_stride;
+	int64_t out_row0, out_channel_stride;
+	int64_t seg0;
 	};
 
 PVM_HD float time_to_frame( const StretchArgs & a, float t ) { return t * a.sample_rate / a.hop; }
@@ -555,6 +562,19 @@ PVM_HD void stretch_plan_frame( const StretchArgs & a, const StretchPlan & plan,
 	for( ; xs < x; ++xs ) { plan.mix[xs] = interp_eval( a.interp, ( (float) xs - lFrame ) / den ); plan.src[xs] = (int) f; }
 	}
 
+// Input rows [*r0, *r1) that stretch_segment_planned reads for the output frames [x0, x1): the frames of the pairs that
+// cover them, and the left frame of the first -- the pair a segment that begins inside it looks back into. Empty when no
+// pair covers any of them (zeros below xpos[0] and above xpos[F-1]).
+PVM_HD void stretch_window( const StretchPlan & plan, int64_t F, int64_t x0, int64_t x1, int64_t * r0, int64_t * r1 )
+	{
+	int64_t c0 = plan.xpos[0], c1 = plan.xpos[F - 1];
+	if( c0 < x0 ) c0 = x0;
+	if( c1 > x1 ) c1 = x1;
+	if( c0 >= c1 ) { *r0 = 0; *r1 = 0; return; }
+	*r0 = plan.src[c0] - 1;
+	*r1 = plan.src[c1 - 1] + 1;
+	}
+
 // The same arithmetic by OUTPUT segments: thread = (channel, run of seg_len output frames, bin) gathers its frames in
 // increasing order -- the order in which PV::convert_to_audio accumulates the phase of a bin (phase_vocoder.cpp:57-59)
 // -- so it can leave the segment's phase summary behind (summary != null) and resynthesis need not read the rows again.
@@ -564,12 +584,12 @@ template<bool SUMM>
 PVM_HD void stretch_segment_planned( const StretchArgs & a, const StretchPlan & plan, int c, int64_t seg, int seg_len, int bin,
                                      pvk::PhaseSegAcc * summary, const pvk::PvConsts & k )
 	{
-	const float2 * in = a.pv + (int64_t) c * a.F * a.B + bin;
+	const float2 * in = a.pv + (int64_t) c * a.pv_channel_stride + bin;
 	const int64_t B = a.B;
-	int x = (int)( seg * seg_len );                                     // the planned form runs below 2^31 frames
+	int x = (int)( ( a.seg0 + seg ) * seg_len );                        // the planned form runs below 2^31 frames
 	int x1 = x + seg_len;
 	if( (int64_t) x1 > a.out_frames ) x1 = (int) a.out_frames;
-	float2 * o = a.out + ( (int64_t) c * a.out_frames + x ) * B + bin;  // the output cell of frame x
+	float2 * o = a.out + (int64_t) c * a.out_channel_stride + ( x - a.out_row0 ) * B + bin;     // the output cell of frame x
 	const float2 zero = make_float2( 0.0f, 0.0f );
 	// The pairs cover [xpos[0], xpos[F-1]) without gaps (the map never descends): zeros below, pairs f_lo .. f_hi, zeros above.
 	int c0 = plan.xpos[0], c1 = plan.xpos[a.F - 1];
@@ -580,7 +600,7 @@ PVM_HD void stretch_segment_planned( const StretchArgs & a, const StretchPlan & 
 	if( x < c1 )
 		{
 		const int f_lo = plan.src[x], f_hi = plan.src[c1 - 1];
-		const float2 * row = in + (int64_t) f_lo * B;                   // right frame of the current pair
+		const float2 * row = in + ( f_lo - a.row0 ) * B;                // right frame of the current pair
 		float2 l = *( row - B );
 		bool live = true;
 		// a segment that begins inside a pair: did an earlier frame of the pair end it (PVModify.cpp:351-352)?

@@ -36,7 +36,8 @@ flan_b200_ctx * context();
 // Every visible GPU behind one handle (include/flan_b200.h: flan_b200_multi_*), or nullptr when the process uses a
 // single device: $FLAN_B200_DEVICE names one, or only one is visible. $FLAN_B200_DEVICES="0,1,..." picks a subset.
 // When it exists, context() is its device 0. Long signals are then cut into frame-range shards, one per GPU, by
-// Audio::convert_to_PV, and PV::convert_to_audio resynthesises them with the phase-state and halo exchange between
+// Audio::convert_to_PV, PV::repitch / stretch / modify_time keep them sharded (a per-bin or descending time map
+// gathers onto device 0), and PV::convert_to_audio resynthesises them with the phase-state and halo exchange between
 // the devices; the result is the single-device result bit for bit.
 flan_b200_multi * multi();
 
@@ -44,6 +45,11 @@ flan_b200_multi * multi();
 struct ShardedStore;
 std::shared_ptr<ShardedStore> new_sharded_store();
 void * sharded_descriptor( ShardedStore & );      // flan_b200_sharded_pv * (include/flan_b200.h)
+// The call that wrote the shards also left their phase summaries on every device (flan_b200_multi_stretch /
+// _modify_time): a resynthesis of the shards as they are may say so (flan_b200_multi_promise_unchanged). A mutable host
+// access drops the shards, so a store that still exists still holds the rows that call wrote.
+void set_sharded_summaries( ShardedStore & );
+bool sharded_summaries( const ShardedStore & );
 
 // Recycled host vectors (see the header comment). `pinned` reports whether the vector's storage is page-locked.
 template<typename T> std::vector<T> pool_take( size_t count, bool zeroed, bool * pinned, bool only_if_pooled = false );

@@ -168,8 +168,10 @@ Audio PV::convert_to_audio( flan_CANCEL_ARG_CPP ) const
 			bool pinned = false;
 			std::vector<Sample> host = b200::pool_take<Sample>( size_t( af.num_channels ) * size_t( af.num_frames ), false, &pinned );
 			int nan_or_inf = 0;
-			const int rc = flan_b200_multi_convert_to_audio_host( m, static_cast<const flan_b200_sharded_pv *>( b200::sharded_descriptor( *store ) ),
-				host.data(), &nan_or_inf );
+			const auto * desc = static_cast<const flan_b200_sharded_pv *>( b200::sharded_descriptor( *store ) );
+			// shards still exactly as PV::stretch / modify_time wrote them: the phase summaries it left are used
+			if( b200::sharded_summaries( *store ) ) flan_b200_multi_promise_unchanged( m, desc );
+			const int rc = flan_b200_multi_convert_to_audio_host( m, desc, host.data(), &nan_or_inf );
 			if( rc != FLAN_B200_OK )
 				{
 				std::cout << "flan::PV::convert_to_audio failed on the GPU engine: " << flan_b200_multi_last_error( m ) << std::endl;

@@ -6,6 +6,7 @@
 
 #include <algorithm>
 #include <iostream>
+#include <optional>
 #include <thread>
 #include <vector>
 
@@ -51,11 +52,13 @@ template<class Body> void for_rows( ExecutionPolicy policy, Frame rows, Body bod
 	}
 
 // sample_function_over_domain (PV.h:31-35): value( frame, bin ) = f( { frame * ( 1 / analysis_rate ), bin * bin_to_frequency( 1 ) } ).
-bool sample_over_domain( const PV & pv, const Function<TF, float> & f, DeviceTable & t )
+// Host memory; *frame_stride, *bin_stride: (0, 0) for a constant, (B, 1) otherwise.
+std::vector<float> sample_on_host( const PV & pv, const Function<TF, float> & f, int64_t * frame_stride, int * bin_stride )
 	{
 	const Frame F = pv.get_num_frames();
 	const Bin B = pv.get_num_bins();
 	std::vector<float> host;
+	*frame_stride = 0; *bin_stride = 0;
 	if( f.is_constant() )
 		host.assign( 1, f( TF{ 0, 0 } ) );
 	else
@@ -66,9 +69,14 @@ bool sample_over_domain( const PV & pv, const Function<TF, float> & f, DeviceTab
 			{
 			for( Bin y = 0; y < B; ++y ) host[size_t( x ) * B + y] = f( TF{ x * x_scale, y * y_scale } );
 			} );
-		t.frame_stride = B; t.bin_stride = 1;
+		*frame_stride = B; *bin_stride = 1;
 		}
-	t.data = b200::Mirror<float>( std::move( host ) );
+	return host;
+	}
+
+bool sample_over_domain( const PV & pv, const Function<TF, float> & f, DeviceTable & t )
+	{
+	t.data = b200::Mirror<float>( sample_on_host( pv, f, &t.frame_stride, &t.bin_stride ) );
 	t.d = t.data.device();
 	return t.d != nullptr;
 	}
@@ -87,6 +95,30 @@ int device_interp( const char * what, const Interpolator & interp )
 	}
 
 const float * as_floats( const MF * p ) { return reinterpret_cast<const float *>( p ); }
+
+// A PV sharded over several GPUs (Audio::convert_to_PV of a long signal): the multi-device form of repitch, stretch or
+// modify_time (include/flan_b200.h) with the host table, and the result stays sharded -- null when the PV is not sharded.
+using MultiCall = int ( * )( flan_b200_multi *, const flan_b200_sharded_pv *, const float *, int64_t, int, int, flan_b200_sharded_pv * );
+std::optional<PV> on_shards( const PV & me, const char * what, MultiCall call, const Function<TF, float> & f, int interp, bool summaries )
+	{
+	const auto & store = me.storage().shards();
+	flan_b200_multi * m = b200::multi();
+	if( !store || !m ) return std::nullopt;
+	int64_t fs = 0; int bs = 0;
+	const std::vector<float> table = sample_on_host( me, f, &fs, &bs );
+	auto out = b200::new_sharded_store();
+	auto * desc = static_cast<flan_b200_sharded_pv *>( b200::sharded_descriptor( *out ) );
+	if( call( m, static_cast<const flan_b200_sharded_pv *>( b200::sharded_descriptor( *store ) ), table.data(), fs, bs, interp, desc ) != FLAN_B200_OK )
+		{
+		std::cout << "flan::" << what << " failed on the GPU engine: " << flan_b200_multi_last_error( m ) << std::endl;
+		return PV();
+		}
+	if( summaries ) b200::set_sharded_summaries( *out );
+	PVBuffer::Format format = me.get_format();
+	format.num_frames = Frame( desc->frames );
+	const size_t count = size_t( format.num_channels ) * size_t( format.num_frames ) * size_t( format.num_bins );
+	return PV( PVBuffer::from_device_result( format, b200::Mirror<MF>::from_shards( count, std::move( out ) ) ) );
+	}
 
 // modify_time_base (PVModify.cpp:307-362) on a device time map in seconds.
 PV modify_time_on_device( const PV & me, const char * what, const float * d_map, int64_t fs, int bs, int interp )
@@ -114,6 +146,8 @@ PV PV::repitch( const Function<TF, float> & factor, const Interpolator & interp 
 	{
 	if( is_null() ) return PV();                                         // PVModify.cpp:202
 	const int id = device_interp( "PV::repitch", interp );
+	if( id < 0 ) return PV();
+	if( auto sharded = on_shards( *this, "PV::repitch", flan_b200_multi_repitch, factor, id, false ) ) return std::move( *sharded );
 	flan_b200_ctx * ctx = b200::context();
 	DeviceTable t;
 	if( id < 0 || !ctx || !sample_over_domain( *this, factor, t ) ) return PV();
@@ -160,6 +194,8 @@ PV PV::modify_time( const Function<TF, Second> & mod, const Interpolator & inter
 	{
 	if( is_null() ) return PV();                                         // PVModify.cpp:309
 	const int id = device_interp( "PV::modify_time", interp );
+	if( id < 0 ) return PV();
+	if( auto sharded = on_shards( *this, "PV::modify_time", flan_b200_multi_modify_time, mod, id, true ) ) return std::move( *sharded );
 	DeviceTable t;
 	if( id < 0 || !b200::context() || !sample_over_domain( *this, mod, t ) ) return PV();
 	return modify_time_on_device( *this, "PV::modify_time", t.d, t.frame_stride, t.bin_stride, id );
@@ -169,6 +205,8 @@ PV PV::stretch( const Function<TF, float> & factor, const Interpolator & interp 
 	{
 	if( is_null() ) return PV();
 	const int id = device_interp( "PV::stretch", interp );
+	if( id < 0 ) return PV();
+	if( auto sharded = on_shards( *this, "PV::stretch", flan_b200_multi_stretch, factor, id, true ) ) return std::move( *sharded );
 	flan_b200_ctx * ctx = b200::context();
 	DeviceTable t;
 	if( id < 0 || !ctx || !sample_over_domain( *this, factor, t ) ) return PV();

@@ -73,11 +73,14 @@ flan_b200_multi * multi()
 struct ShardedStore
 	{
 	flan_b200_sharded_pv desc{};
+	bool summaries = false;
 	~ShardedStore() { if( flan_b200_multi * m = engine().multi ) flan_b200_multi_free_pv( m, &desc ); }
 	};
 
 std::shared_ptr<ShardedStore> new_sharded_store() { return std::make_shared<ShardedStore>(); }
 void * sharded_descriptor( ShardedStore & s ) { return &s.desc; }
+void set_sharded_summaries( ShardedStore & s ) { s.summaries = true; }
+bool sharded_summaries( const ShardedStore & s ) { return s.summaries; }
 
 namespace {
 

@@ -310,6 +310,8 @@ int flan_b200_convert_to_audio_host( flan_b200_ctx * ctx, const float * h_pv, in
  * moves the per-bin phase state (32 * channels * bins bytes per shard) and the window - hop overlap-add halo of every
  * shard boundary device to device (cudaMemcpyPeerAsync over NVLink), the halo behind the interior frames' compute.
  * Short signals use fewer shards than devices (a shard is at least one segment and 2 * ceil(window / hop) frames).
+ * Between the two, repitch, and stretch / modify_time with a bin-shared map that never descends, keep the PV sharded
+ * (flan_b200_multi_repitch / _stretch / _modify_time); other maps gather it onto device 0 and give a one-shard PV.
  * The structs are plain data owned by the caller; their device blocks come from the per-device contexts. */
 #define FLAN_B200_MAX_DEVICES 16
 typedef struct flan_b200_multi flan_b200_multi;
@@ -362,6 +364,21 @@ int  flan_b200_multi_gather_audio( flan_b200_multi * m, const flan_b200_sharded_
 /* PV rows of every shard -> host MF[channels][frames][bins] (h_pv, synchronous) and / or one device buffer of that layout
  * on device `to` of the handle (d_pv, asynchronous on that device's stream). Either pointer may be NULL. */
 int  flan_b200_multi_gather_pv( flan_b200_multi * m, const flan_b200_sharded_pv * pv, float * h_pv, int to, float * d_pv );
+/* The PV-domain chain over the shards (PV::repitch, PV::stretch, PV::modify_time): each reads pv, leaves it unchanged and
+ * writes a new sharded PV into pv_out. Tables are HOST memory with the strides of the single-device forms: (bins,1),
+ * (0,1), (1,0) or (0,0). Repitch: every device repitches its own rows with its rows of the table; pv_out has pv's frame
+ * ranges. Stretch / modify_time with a map shared by all bins that never descends (a constant or time-only factor):
+ * pv_out is cut like an analysed PV of its own frame count, each output shard is computed on its device from the input
+ * rows it needs (read in place when the input shard on that device holds them, else peer-copied there), and leaves its
+ * phase summaries, so that flan_b200_multi_promise_unchanged then lets flan_b200_multi_convert_to_audio skip the second
+ * read of the rows. Any other map (per bin, or descending) gathers the PV onto device 0 and runs the single-device path
+ * there: pv_out then has one shard. Either way the rows are the single-device result bit for bit. */
+int  flan_b200_multi_repitch( flan_b200_multi * m, const flan_b200_sharded_pv * pv, const float * h_factor,
+                              int64_t factor_frame_stride, int factor_bin_stride, int interp, flan_b200_sharded_pv * pv_out );
+int  flan_b200_multi_stretch( flan_b200_multi * m, const flan_b200_sharded_pv * pv, const float * h_factor,
+                              int64_t factor_frame_stride, int factor_bin_stride, int interp, flan_b200_sharded_pv * pv_out );
+int  flan_b200_multi_modify_time( flan_b200_multi * m, const flan_b200_sharded_pv * pv, const float * h_map_seconds,
+                                  int64_t map_frame_stride, int map_bin_stride, int interp, flan_b200_sharded_pv * pv_out );
 int  flan_b200_multi_free_audio( flan_b200_multi * m, flan_b200_sharded_audio * audio );
 int  flan_b200_multi_free_pv( flan_b200_multi * m, flan_b200_sharded_pv * pv );
 /* What flan::Audio::convert_to_PV / flan::PV::convert_to_audio call for long signals when several GPUs are visible. */
