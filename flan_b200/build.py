@@ -102,6 +102,11 @@ def api_test_path():
     return os.path.join(LIB, "libflan_api_test.so")
 
 
+def wav_test_path():
+    """tests/cpp/wav_formats_driver.cpp: WAV files of every sample type through flan::Audio::load / save."""
+    return os.path.join(LIB, "libflan_wav_test.so")
+
+
 def e2e_bench_path():
     return os.path.join(LIB, "libflan_e2e_bench.so")
 
@@ -123,6 +128,9 @@ def build_host(force=False):
     drv = os.path.join(root, "tests", "cpp", "flan_api_driver.cpp")
     if force or _newer(api_test_path(), [drv, host_path()] + hdrs):
         subprocess.run(common + ["-o", api_test_path(), drv] + link + ["-lflan_b200_host", "-lflan_b200"], check=True)
+    wav_drv = os.path.join(root, "tests", "cpp", "wav_formats_driver.cpp")
+    if os.path.exists(wav_drv) and (force or _newer(wav_test_path(), [wav_drv, host_path()] + hdrs)):
+        subprocess.run(common + ["-o", wav_test_path(), wav_drv] + link + ["-lflan_b200_host", "-lflan_b200"], check=True)
     e2e = os.path.join(root, "tools", "cpp", "e2e_bench.cpp")
     if os.path.exists(e2e) and (force or _newer(e2e_bench_path(), [e2e, host_path()] + hdrs)):
         subprocess.run(common + ["-o", e2e_bench_path(), e2e] + link + ["-lflan_b200_host", "-lflan_b200", "-lpthread"], check=True)

@@ -14,6 +14,10 @@ _f = ctypes.c_float
 
 OK, INVALID, UNSUPPORTED, CUDA, CANCELLED, NOMEM = range(6)
 
+# WAV sample types (FLAN_B200_WAV_*): libsndfile's sub-type codes, and the bytes a value takes
+WAV_PCM_16, WAV_PCM_24, WAV_PCM_32, WAV_PCM_U8, WAV_FLOAT, WAV_DOUBLE = 0x2, 0x3, 0x4, 0x5, 0x6, 0x7
+WAV_WIDTH = {WAV_PCM_U8: 1, WAV_PCM_16: 2, WAV_PCM_24: 3, WAV_PCM_32: 4, WAV_FLOAT: 4, WAV_DOUBLE: 8}
+
 MAX_DEVICES = 16
 
 
@@ -91,10 +95,14 @@ SYMBOLS = [
     ("flan_b200_flan_info", _int, [_vp, ctypes.c_char_p, ctypes.POINTER(_int), ctypes.POINTER(_i64), ctypes.POINTER(_int),
                                    ctypes.POINTER(_f), ctypes.POINTER(_f), ctypes.POINTER(_int)]),
     ("flan_b200_load_flan", _int, [_vp, ctypes.c_char_p, _vp, _i64]),
+    ("flan_b200_pcm_encode", _int, [_vp, _vp, _int, _i64, _int, _vp]),
+    ("flan_b200_pcm_decode", _int, [_vp, _vp, _int, _i64, _int, _vp]),
     ("flan_b200_pcm24_encode", _int, [_vp, _vp, _int, _i64, _vp]),
     ("flan_b200_pcm24_decode", _int, [_vp, _vp, _int, _i64, _vp]),
+    ("flan_b200_save_wav_as", _int, [_vp, ctypes.c_char_p, _vp, _int, _i64, _f, _int]),
     ("flan_b200_save_wav", _int, [_vp, ctypes.c_char_p, _vp, _int, _i64, _f]),
     ("flan_b200_wav_info", _int, [_vp, ctypes.c_char_p, ctypes.POINTER(_int), ctypes.POINTER(_i64), ctypes.POINTER(_f)]),
+    ("flan_b200_wav_format", _int, [_vp, ctypes.c_char_p, ctypes.POINTER(_int)]),
     ("flan_b200_load_wav", _int, [_vp, ctypes.c_char_p, _vp, _i64]),
     ("flan_b200_multi_create", _int, [ctypes.POINTER(_int), _int, ctypes.POINTER(_vp)]),
     ("flan_b200_multi_destroy", None, [_vp]),

@@ -274,10 +274,30 @@ class Engine:
         self.ctx.call("flan_b200_pcm24_decode", self._chk(data, torch.uint8), C, n, self._chk(out))
         return out
 
-    def save_wav(self, path, audio, sr):
+    def pcm_encode(self, audio, subtype):
+        """audio: cuda float32 [C, n] -> interleaved sample bytes of a WAV sample type (capi.WAV_*)."""
+        C, n = audio.shape
+        out = torch.empty((C * n * capi.WAV_WIDTH[subtype],), dtype=torch.uint8, device=self.device)
+        self._bind_stream()
+        self.ctx.call("flan_b200_pcm_encode", self._chk(audio), C, n, subtype, self._chk(out, torch.uint8))
+        return out
+
+    def pcm_decode(self, data, C, n, subtype):
+        out = torch.empty((C, n), dtype=torch.float32, device=self.device)
+        self._bind_stream()
+        self.ctx.call("flan_b200_pcm_decode", self._chk(data, torch.uint8), C, n, subtype, self._chk(out))
+        return out
+
+    def save_wav(self, path, audio, sr, subtype=capi.WAV_PCM_24):
         C, n = audio.shape
         self._bind_stream()
-        self.ctx.call("flan_b200_save_wav", path.encode(), self._chk(audio), C, n, sr)
+        self.ctx.call("flan_b200_save_wav_as", path.encode(), self._chk(audio), C, n, sr, subtype)
+
+    def wav_format(self, path):
+        """The sample type (capi.WAV_*) of a WAV file's data."""
+        t = ctypes.c_int()
+        self.ctx.call("flan_b200_wav_format", path.encode(), ctypes.byref(t))
+        return t.value
 
     def load_wav(self, path):
         C, n, sr = ctypes.c_int(), ctypes.c_int64(), ctypes.c_float()

@@ -1,8 +1,9 @@
 // flan::AudioBuffer of the B200 build: the reference's public surface (src/flan/Audio/AudioBuffer.h:20-228) for
 // everything on the phase-vocoder path, over device-resident storage (flan/b200_storage.h). Layout contract:
 // planar, channel-major, pos = channel * num_frames + frame (AudioBuffer.cpp:479-482) -- computed in 64 bits here.
-// File I/O: 24-bit PCM WAV, the reference's default save format (AudioBuffer.cpp:136), with the sample conversion and the
-// (de)interleave on the GPU; libsndfile's other formats and its metadata strings are outside the scope of this build.
+// File I/O: WAV with libsndfile's sample types for it (8-bit unsigned, 16-, 24- and 32-bit PCM, 32- and 64-bit float;
+// 24-bit PCM is the reference's default save format, AudioBuffer.cpp:136), with the sample conversion and the
+// (de)interleave on the GPU; libsndfile's other major formats and its metadata strings are outside the scope of this build.
 #pragma once
 
 #include <iosfwd>
@@ -11,6 +12,7 @@
 
 #include "flan/defines.h"
 #include "flan/b200_storage.h"
+#include "flan/Audio/SndfileFormats.h"
 
 namespace flan {
 
@@ -61,10 +63,12 @@ public:
 	size_t get_buffer_pos( Channel, Frame ) const;
 
 	// B200 build: device-side view for the conversion entry points (not part of the reference's surface)
-	/** Load a 24-bit PCM WAV file (reference AudioBuffer::load, AudioBuffer.cpp:80-128). false + message on failure. */
+	/** Load a WAV file of PCM (8, 16, 24, 32 bits) or float (32, 64 bits) samples (reference AudioBuffer::load,
+	 *  AudioBuffer.cpp:80-128). false + message on failure. */
 	bool load( const std::string & filename );
-	/** Save as 24-bit PCM WAV, samples clamped to [-1,1] (reference AudioBuffer::save with its default format,
-	 *  AudioBuffer.cpp:130-170). Any other \param format prints a message and returns false. */
+	/** Save as WAV, samples clamped to [-1,1] (reference AudioBuffer::save, AudioBuffer.cpp:130-170). \param format is
+	 *  libsndfile's: -1 (the default, 24-bit PCM) or SF_FORMAT_WAV | SF_FORMAT_PCM_U8 / _PCM_16 / _PCM_24 / _PCM_32 /
+	 *  _FLOAT / _DOUBLE, with SF_ENDIAN_FILE or SF_ENDIAN_LITTLE. Any other format prints a message and returns false. */
 	bool save( const std::string & filename, int format = -1 ) const;
 
 	const b200::Mirror<Sample> & storage() const { return buffer; }

@@ -109,20 +109,44 @@ std::ostream & operator<<( std::ostream & os, const AudioBuffer & a )
 	}
 
 
-// ---- WAV files (reference AudioBuffer.cpp:80-192 through libsndfile): 24-bit PCM through the GPU codec -------------
+// ---- WAV files (reference AudioBuffer.cpp:80-192 through libsndfile): the sample codecs run on the GPU ---------------
+
+static_assert( SF_FORMAT_PCM_U8 == FLAN_B200_WAV_PCM_U8 && SF_FORMAT_PCM_16 == FLAN_B200_WAV_PCM_16 &&
+               SF_FORMAT_PCM_24 == FLAN_B200_WAV_PCM_24 && SF_FORMAT_PCM_32 == FLAN_B200_WAV_PCM_32 &&
+               SF_FORMAT_FLOAT == FLAN_B200_WAV_FLOAT && SF_FORMAT_DOUBLE == FLAN_B200_WAV_DOUBLE, "libsndfile's sub-type codes" );
+
+// The FLAN_B200_WAV_* sample type a libsndfile format asks for, or 0 where this build does not write it: another major
+// format, big-endian, or a sub-type libsndfile does not accept for WAV (PCM_S8) or this build does not know.
+static int wav_subtype_of( int file_format )
+	{
+	if( file_format == -1 ) return FLAN_B200_WAV_PCM_24;                  // AudioBuffer.cpp:136
+	if( ( file_format & SF_FORMAT_TYPEMASK ) != SF_FORMAT_WAV ) return 0;
+	const int endian = file_format & SF_FORMAT_ENDMASK;
+	if( endian != SF_ENDIAN_FILE && endian != SF_ENDIAN_LITTLE ) return 0;
+	if( file_format & ~( SF_FORMAT_TYPEMASK | SF_FORMAT_SUBMASK | SF_FORMAT_ENDMASK ) ) return 0;
+	switch( file_format & SF_FORMAT_SUBMASK )          // libsndfile's sub-type codes are the FLAN_B200_WAV_* codes
+		{
+		case SF_FORMAT_PCM_U8: case SF_FORMAT_PCM_16: case SF_FORMAT_PCM_24: case SF_FORMAT_PCM_32:
+		case SF_FORMAT_FLOAT: case SF_FORMAT_DOUBLE:
+			return file_format & SF_FORMAT_SUBMASK;
+		default: return 0;
+		}
+	}
+
 bool AudioBuffer::save( const std::string & filename, int file_format ) const
 	{
-	if( file_format != -1 )
+	const int subtype = wav_subtype_of( file_format );
+	if( !subtype )
 		{
 		std::cout << "Sound file formatting invalid while attempting to save to " << filename << ",\n"
-		          << "(the B200 build writes the reference's default, 24-bit PCM WAV, only)" << std::endl;
+		          << "(the B200 build writes WAV, little-endian, with PCM_U8, PCM_16, PCM_24, PCM_32, FLOAT or DOUBLE samples)" << std::endl;
 		return false;
 		}
 	flan_b200_ctx * ctx = b200::context();
 	if( !ctx ) return false;
 	const Sample * d = buffer.empty() ? nullptr : buffer.device();
 	if( !buffer.empty() && !d ) return false;
-	const int rc = flan_b200_save_wav( ctx, filename.c_str(), d, get_num_channels(), get_num_frames(), get_sample_rate() );
+	const int rc = flan_b200_save_wav_as( ctx, filename.c_str(), d, get_num_channels(), get_num_frames(), get_sample_rate(), subtype );
 	if( rc != FLAN_B200_OK ) std::cout << flan_b200_last_error( ctx ) << std::endl;
 	return rc == FLAN_B200_OK;
 	}

@@ -268,14 +268,41 @@ int flan_b200_flan_info( flan_b200_ctx * ctx, const char * path, int * channels,
                          float * sample_rate, float * rate_field, int * window_size );
 int flan_b200_load_flan( flan_b200_ctx * ctx, const char * path, float * d_pv, int64_t capacity_mf );
 
-/* WAV PCM-24, the format AudioBuffer::save defaults to (src/flan/Audio/AudioBuffer.cpp:136; load :80-128). The reference
- * goes through libsndfile (external, not vendored, version unpinned): its published 24-bit conversions are restated --
- * write: clamp to [-1,1] (AudioBuffer.cpp:158-161), lrintf( x * 0x7FFFFF ); read: value / 2^23 -- with the
- * planar <-> interleaved reshuffle of AudioBuffer.cpp:122-125,152-155 fused in. Metadata strings are not carried. */
+/* WAV (RIFF, little-endian), as AudioBuffer::save / load handle it through libsndfile (src/flan/Audio/AudioBuffer.cpp:
+ * 80-192; save defaults to PCM-24, :136). The sample types are libsndfile's for SF_FORMAT_WAV, and the codes below are
+ * its sub-type values (SF_FORMAT_PCM_16 ...). libsndfile is external, not vendored, version unpinned: its default
+ * conversions (normalisation on, clipping off) are restated. Write: clamp to [-1,1] (AudioBuffer.cpp:158-161; NaN passes
+ * through), then
+ *   PCM_U8  lrintf( x * 127 ) + 128        PCM_16  lrintf( x * 32767 )        PCM_24  lrintf( x * 8388607 )
+ *   PCM_32  lrintf( x * 2^31 ), where +1.0 and NaN give 0x80000000 as on x86     FLOAT  the bits     DOUBLE  (double) x
+ * (lrintf rounds half to even). Read: ( v - 128 ) / 128, v / 32768, v / 2^23, v / 2^31 (int -> float rounds to nearest
+ * even), the bits, ( float ) d. The planar <-> interleaved reshuffle of AudioBuffer.cpp:122-125,152-155 is fused in.
+ * Files read: format tag 1 (PCM, 1-4 byte containers), 3 (IEEE float, 32 or 64 bits) and WAVE_FORMAT_EXTENSIBLE with
+ * the PCM or IEEE-float sub-format; the container width block_align / channels must be ceil( bits / 8 ) (20 valid bits in
+ * 3 bytes read as PCM_24); anything else is FLAN_B200_UNSUPPORTED. Files written: PCM with the canonical 44-byte header,
+ * FLOAT / DOUBLE with tag 3, an 18-byte fmt chunk and a fact chunk. Metadata strings are not carried, and a file over the
+ * 4 GiB RIFF limit is refused before it is created. */
+#define FLAN_B200_WAV_PCM_16  0x0002
+#define FLAN_B200_WAV_PCM_24  0x0003
+#define FLAN_B200_WAV_PCM_32  0x0004
+#define FLAN_B200_WAV_PCM_U8  0x0005
+#define FLAN_B200_WAV_FLOAT   0x0006
+#define FLAN_B200_WAV_DOUBLE  0x0007
+/* Sample codec on device buffers: planar float[channels][n] <-> interleaved frames, width( subtype ) * channels * n bytes
+ * (16-byte aligned). */
+int flan_b200_pcm_encode( flan_b200_ctx * ctx, const float * d_audio, int channels, int64_t n, int subtype, uint8_t * d_bytes );
+int flan_b200_pcm_decode( flan_b200_ctx * ctx, const uint8_t * d_bytes, int channels, int64_t n, int subtype, float * d_audio );
+/* The PCM_24 forms of the two above. */
 int flan_b200_pcm24_encode( flan_b200_ctx * ctx, const float * d_audio, int channels, int64_t n, uint8_t * d_bytes );
 int flan_b200_pcm24_decode( flan_b200_ctx * ctx, const uint8_t * d_bytes, int channels, int64_t n, float * d_audio );
+/* Whole files: header + samples streamed between the file and the device in chunks (synchronous). save_wav writes
+ * PCM_24, AudioBuffer::save's default. */
+int flan_b200_save_wav_as( flan_b200_ctx * ctx, const char * path, const float * d_audio, int channels, int64_t n, float sample_rate,
+                           int subtype );
 int flan_b200_save_wav( flan_b200_ctx * ctx, const char * path, const float * d_audio, int channels, int64_t n, float sample_rate );
 int flan_b200_wav_info( flan_b200_ctx * ctx, const char * path, int * channels, int64_t * n, float * sample_rate );
+/* *subtype: the FLAN_B200_WAV_* code of the samples the file holds. */
+int flan_b200_wav_format( flan_b200_ctx * ctx, const char * path, int * subtype );
 int flan_b200_load_wav( flan_b200_ctx * ctx, const char * path, float * d_audio, int64_t capacity_samples );
 
 /* ---- pipelined host-buffer forms: what flan::Audio::convert_to_PV / flan::PV::convert_to_audio call when the newest
