@@ -12,6 +12,8 @@
 #include <atomic>
 #include <cmath>
 #include <barrier>
+#include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <memory>
 #include <thread>
@@ -56,6 +58,42 @@ struct HostEnv
 		while( std::atomic_ref<BulkBarrier>( *bar ).load( std::memory_order_acquire ) <= bulk_waits ) std::this_thread::yield();
 		++bulk_waits;
 		}
+	// tensor memory: the CTA's 128 lanes x TMEM_COLS words, lane = thread; a column read before this thread wrote it aborts
+	static constexpr int TMEM_COLS = 128;
+	float * tmem_words;
+	unsigned char * tmem_written;
+	template<int K> void tmem_st( int col, const float * r )
+		{
+		for( int i = 0; i < K; ++i )
+			{
+			tmem_check( col + i );
+			tmem_words[tid * TMEM_COLS + col + i] = r[i];
+			tmem_written[tid * TMEM_COLS + col + i] = 1;
+			}
+		}
+	void tmem_wait_st() {}
+	template<int K> void tmem_ld( int col, float * r )
+		{
+		for( int i = 0; i < K; ++i )
+			{
+			tmem_check( col + i );
+			if( !tmem_written[tid * TMEM_COLS + col + i] )
+				{
+				std::fprintf( stderr, "pv_emu: thread %d reads tensor-memory column %d before writing it\n", tid, col + i );
+				std::abort();
+				}
+			r[i] = tmem_words[tid * TMEM_COLS + col + i];
+			}
+		}
+	template<int K> void tmem_wait( float * ) {}
+	void tmem_check( int col )
+		{
+		if( tid >= 128 || col < 0 || col >= TMEM_COLS )
+			{
+			std::fprintf( stderr, "pv_emu: tensor-memory access of thread %d, column %d, outside the 128 lanes x %d columns\n", tid, col, TMEM_COLS );
+			std::abort();
+			}
+		}
 	};
 
 template<int N, int PT, class Body> void run_cta( Body && body )
@@ -63,6 +101,8 @@ template<int N, int PT, class Body> void run_cta( Body && body )
 	constexpr int T = N / ( 2 * PT );
 	std::vector<float> ring( N );
 	std::vector<float2> x0( XBuf<N / 2>::size ), x1( XBuf<N / 2>::size ), rowbuf( N / 2 + 16 );
+	std::vector<float> tmem( 128 * HostEnv::TMEM_COLS );
+	std::vector<unsigned char> tmem_written( 128 * HostEnv::TMEM_COLS, 0 );
 	std::barrier<> bar( T );
 	std::vector<std::unique_ptr<std::barrier<>>> warpbars;
 	for( int w = 0; w < ( T + 31 ) / 32; ++w ) warpbars.emplace_back( new std::barrier<>( T - 32 * w < 32 ? T - 32 * w : 32 ) );
@@ -70,7 +110,7 @@ template<int N, int PT, class Body> void run_cta( Body && body )
 	for( int t = 0; t < T; ++t )
 		th.emplace_back( [&, t]
 			{
-			HostEnv env{ t, &bar, 0, warpbars[t / 32].get() };
+			HostEnv env{ t, &bar, 0, warpbars[t / 32].get(), tmem.data(), tmem_written.data() };
 			body( env, ring.data(), x0.data(), x1.data(), rowbuf.data() );
 			} );
 	for( auto & x : th ) x.join();

@@ -114,6 +114,16 @@ struct AnalysisArgs
 	double P, rcpP;
 	};
 
+// Tensor memory of the 16-point analysis at dft 4096 (128 threads: thread t owns TMEM lane t; 128 columns per CTA, so the
+// four CTAs an SM holds at 128 registers use all 512 columns). What a thread reads every frame and never changes during
+// the walk is stored there once, instead of living in registers (the window) or being re-read through L1 (the tables):
+//   columns  0..31  window coefficients w[0..31]
+//           32..59  the 14 twiddles of the last pass (radix 8, two butterflies)
+//           64..127 per slot u, 8 columns: binc4[k] (4), post_rot[k] (2), two unused, k = t + u*T
+// The first pass's twiddles stay in L1: their index is t mod 16, 240 entries in all.
+template<int N, int PT> constexpr bool analysis_tmem() { return PT == 16 && N == 4096; }
+constexpr int AN_TM_COLS = 128, AN_TM_WIN = 0, AN_TM_TW = 32, AN_TM_BIN = 64;
+
 // PAD: a zero-padded window that fills whole slots of the thread layout (window a multiple of 2T samples, < dft: the
 // API default window 2048 / dft 4096, Audio.h:158-163) loads its samples as vectors like the full window does; a
 // separate instantiation so that the full-window kernels keep their register budget.
@@ -125,10 +135,14 @@ struct AnalysisArgs
 // frames * c + 2^-22 * sum is exact in double and equals the plain double running sum of pv_phase_seg_kernel bit for
 // bit (that sum is exact too: multiples of 2^-22 below 2^18); increments are positive, so the running maximum is the
 // total. A bin that ever leaves those conditions (the lowest bins, NaN / Inf) is marked and gets the NaN entry.
-template<int N, int PT, bool ONE, bool PAD, bool EMIT = false, class Env>
+// TM: the tensor-memory form (analysis_tmem); the Env then addresses the CTA's AN_TM_COLS columns.
+template<int N, int PT, bool ONE, bool PAD, bool EMIT = false, bool TM = analysis_tmem<N, PT>(), class Env>
 PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float2 * x0, float2 * x1, int * ssum = nullptr )
 	{
 	constexpr int M = N / 2, T = M / PT, H = PT / 2;      // H pairs of bins (k, M-k) per thread
+	using P = FftPlan<M, PT>;
+	static_assert( !TM || ( T == 128 && P::num_passes == 3 && 2 * PT == 32 && ( P::radix( 2 ) - 1 ) * ( PT / P::radix( 2 ) ) == 14 && H * 8 == 64 ),
+	               "tensor-memory layout of the dft-4096 analysis" );
 	const int t = env.tid;
 	const int c = (int)( block / a.segs_per_channel );
 	const int seg = (int)( block % a.segs_per_channel );
@@ -149,6 +163,31 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 		const int i0 = 2 * ( t + s * T );
 		w[2 * s]     = ( i0 < W )     ? 0.5f * env.ldg( a.win + i0 ) : 0.0f;
 		w[2 * s + 1] = ( i0 + 1 < W ) ? 0.5f * env.ldg( a.win + i0 + 1 ) : 0.0f;
+		}
+	if constexpr( TM )
+		{
+		env.template tmem_st<32>( AN_TM_WIN, w );
+		float2 tw2[16];
+		fft_load_twiddles<M, PT, P::radix( 2 ), P::ns( 2 )>( t, tw2, a.pass_tw + P::tw_offset( 2 ), [&]( const float2 * q ) { return env.ldg2( q ); } );
+		tw2[14].x = tw2[14].y = tw2[15].x = tw2[15].y = 0.0f;
+		env.template tmem_st<32>( AN_TM_TW, reinterpret_cast<const float *>( tw2 ) );
+#pragma unroll
+		for( int h = 0; h < 2; ++h )
+			{
+			float tb[32];
+#pragma unroll
+			for( int j = 0; j < 4; ++j )
+				{
+				const int k = t + ( 4 * h + j ) * T;
+				const float4 cc = env.ldg4( a.binc4 + k );
+				const float2 pr = env.ldg2( a.post_rot + k );
+				tb[8 * j] = cc.x; tb[8 * j + 1] = cc.y; tb[8 * j + 2] = cc.z; tb[8 * j + 3] = cc.w;
+				tb[8 * j + 4] = pr.x; tb[8 * j + 5] = pr.y; tb[8 * j + 6] = 0.0f; tb[8 * j + 7] = 0.0f;
+				}
+			env.template tmem_st<32>( AN_TM_BIN + 32 * h, tb );
+			}
+		env.tmem_wait_st();
+		env.template tmem_ld<32>( AN_TM_WIN, w );           // the first frame's window; every later one is requested a frame ahead
 		}
 	// Bins of this thread: slot u holds k = t + u*T and its mirror M-k (k = 0: DC and Nyquist), whose previous phases
 	// travel as one packed pair; bin M/2 is the extra bin of thread T/2.
@@ -190,6 +229,7 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 		const int64_t start = (int64_t) hop * f - half;                 // AudioPV.cpp:52
 		const float * src = xch + ( start - a.audio_offset ) + 2 * t;   // this thread's first sample pair
 		float2 v[PT];
+		if constexpr( TM ) env.template tmem_wait<2 * PT>( w );
 		// pass 0: windowed load (AudioPV.cpp:54-62; zero padding :65) + radix-PT. Windows overlap by W-hop samples:
 		// all but the newest hop are L1 hits.
 		if( !PAD && full_window && start >= 0 && start + W <= a.n_total )
@@ -238,9 +278,36 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 			if( t * 32 < hop && p >= 0 && p < a.n_total ) env.prefetch( xch + ( p - a.audio_offset ) );
 			}
 
+		float tab[2][8];            // TM: binc4[k] and post_rot[k] of slot u in tab[u & 1]
+		if constexpr( TM )
+			{
+			// the fft_pass_chain of passes 1 and 2 with the last pass's twiddles from tensor memory, requested before the
+			// barrier that publishes the pass's inputs (as are the first slot's bin constants before the unpack's barrier)
+			float2 * x = ONE ? x0 : x1;
+			fft_load<M, PT, 1>( t, v, x0 );
+			if constexpr( ONE ) env.sync();
+			fft_butterflies<M, PT, PT, P::ns( 1 )>( t, v, a.pass_tw + P::tw_offset( 1 ), [&]( const float2 * q ) { return env.ldg2( q ); } );
+			fft_store<M, PT, PT, P::ns( 1 )>( t, v, x );
+			float2 tw2[14];
+			env.template tmem_ld<16>( AN_TM_TW, reinterpret_cast<float *>( tw2 ) );
+			env.template tmem_ld<8>( AN_TM_TW + 16, reinterpret_cast<float *>( tw2 ) + 16 );
+			env.template tmem_ld<4>( AN_TM_TW + 24, reinterpret_cast<float *>( tw2 ) + 24 );
+			env.sync();
+			fft_load<M, PT, P::ns( 1 )>( t, v, x );
+			if constexpr( ONE ) env.sync();
+			env.template tmem_wait<28>( reinterpret_cast<float *>( tw2 ) );
+			fft_butterflies_w<M, PT, P::radix( 2 ), P::ns( 2 )>( v, tw2 );
+			env.template tmem_ld<8>( AN_TM_BIN, tab[0] );
+#pragma unroll
+			for( int s = PT / 2; s < PT; ++s ) x0[t + s * T] = v[s];
+			env.sync();
+			}
+		else
+			{
 #ifndef PV_ABL_NOFFT
-		fft_pass_chain<M, PT, 1, true, ONE, false>( t, v, x0, x1, a.pass_tw, env, (float2 *) nullptr );
+			fft_pass_chain<M, PT, 1, true, ONE, false>( t, v, x0, x1, a.pass_tw, env, (float2 *) nullptr );
 #endif
+			}
 		const float2 * z = fft_result_buffer<M, PT, ONE>( x0, x1 );     // upper half of Z/2 in natural order
 
 		// real-FFT unpack + phase vocoder (AudioPV.cpp:69-73). The warm-up frame runs the same code with its stores
@@ -258,9 +325,23 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 			const float2 A = add2( zk, pn2( zm ) );
 			const float2 D = add2( zk, np2( zm ) );
 #ifndef PV_ABL_NOTAB
-			const float2 Pq = cmul2( D, env.ldg2( a.post_rot + k ) );
+			float2 rot;
+			float4 cc;
+			if constexpr( TM )
+				{
+				// slot u's constants were requested one slot ahead (slot 0's before the barrier)
+				float * tu = tab[u & 1];
+				env.template tmem_wait<6>( tu );
+				cc.x = tu[0]; cc.y = tu[1]; cc.z = tu[2]; cc.w = tu[3]; rot.x = tu[4]; rot.y = tu[5];
+				if( u + 1 < H ) env.template tmem_ld<8>( AN_TM_BIN + 8 * ( u + 1 ), tab[( u + 1 ) & 1] );
+				}
+			else
+				{
+				rot = env.ldg2( a.post_rot + k );
+				cc = env.ldg4( a.binc4 + k );
+				}
+			const float2 Pq = cmul2( D, rot );
 			const float2 xk = add2( A, Pq ), xmc = sub2( A, Pq );
-			const float4 cc = env.ldg4( a.binc4 + k );
 #else
 			float2 wq; wq.x = 0.5f + k; wq.y = 0.25f;                        // ablation build only: no table traffic
 			const float2 Pq = cmul2( D, wq );
@@ -298,6 +379,7 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 					}
 				}
 			}
+		if constexpr( TM ) { if( f + 1 < fb ) env.template tmem_ld<2 * PT>( AN_TM_WIN, w ); }     // the next frame's window
 		if( t == T / 2 )
 			{
 			const float2 zh = z[M / 2];                           // X[M/2] = conj(Z[M/2])
@@ -892,7 +974,17 @@ template<int R> PV_HD int mpad( int i )
 // two exchange barriers of the next frame order one frame's accumulation before the next one's; no barrier is added),
 // and whether a thread's last used slot starts a ring entry and whether its slot 0 is final depends on the thread (two
 // predicates, fixed over the walk). !GEN is the standard shape (window == dft, hop == dft/16) with everything resolved at compile time.
-template<int N, bool ONE, bool GEN, class Env>
+// Tensor memory of the mirrored resynthesis at dft 4096, standard shape (128 threads, thread t owns lane t, 128 columns per
+// CTA: four CTAs per SM at 128 registers use all 512):
+//   columns  0..31  window coefficients w[0..31]
+//           32..47  post_tw[k] of the thread's 8 bins (slot r at 32 + 2r)
+//           48..77  the 15 twiddles of the second radix-16 pass (78..79 unused)
+// The window is read once per frame, for the overlap-add; the first pass's twiddles stay in L1 (index t mod 8).
+template<int N, bool GEN> constexpr bool synthesis_tmem() { return N == 4096 && !GEN; }
+constexpr int SY_TM_COLS = 128, SY_TM_WIN = 0, SY_TM_POST = 32, SY_TM_TW = 48;
+
+// TM: the tensor-memory form (synthesis_tmem); the Env then addresses the CTA's SY_TM_COLS columns.
+template<int N, bool ONE, bool GEN, bool TM = synthesis_tmem<N, GEN>(), class Env>
 PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, float2 * ring, float2 * x0, float2 * x1, float2 * rowbuf,
                                  typename Env::BulkBarrier * bar )
 	{
@@ -900,6 +992,7 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 	constexpr int PT = 16, M = MP::M, T = MP::T, R = MP::R, NS = MP::NS, Q = MP::Q, B = M + 1;
 	using RP = RevPlan<M, R>;
 	static_assert( T % ( 16 * R ) == 0, "threads per frame" );
+	static_assert( !TM || ( T == 128 && Q == 1 && R == 8 && RP::R3 == 1 && !GEN ), "tensor-memory layout of the dft-4096 resynthesis" );
 	const int t = env.tid;
 	const int per_launch = a.seg_count > 0 ? a.seg_count : a.segs_per_channel;
 	const int c = (int)( block / per_launch );
@@ -947,6 +1040,19 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 			acc[q][r][1] = acc0[M - k];
 			}
 	if( irregular ) acc_mid = acc0[M / 2];
+	if constexpr( TM )
+		{
+		env.template tmem_st<32>( SY_TM_WIN, w );
+		float2 tb[32];              // columns 32..95: post_tw, the pass twiddles, zeros
+#pragma unroll
+		for( int r = 0; r < R; ++r ) tb[r] = env.ldg2( a.post_tw + ( t + ( ( r >= R / 2 ) ? khi : 0 ) + r * NS ) );
+		fft_load_twiddles<M, PT, PT, RP::NS2>( t, tb + 8, a.pass_tw_rev + RP::tw2, [&]( const float2 * q ) { return env.ldg2( q ); } );
+#pragma unroll
+		for( int i = 23; i < 32; ++i ) { tb[i].x = 0.0f; tb[i].y = 0.0f; }
+		env.template tmem_st<32>( SY_TM_POST, reinterpret_cast<const float *>( tb ) );
+		env.template tmem_st<32>( SY_TM_POST + 32, reinterpret_cast<const float *>( tb + 16 ) );
+		env.tmem_wait_st();
+		}
 
 	// thread-private overlap-add ring: 16 pairs at ring[t + T*j]; absolute pair index t + T*A lives in slot A & 15
 #pragma unroll
@@ -1011,8 +1117,11 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 		{
 		const int64_t start = (int64_t) hop * f - half;                          // AudioPV.cpp:125
 		const float2 * row = rowbuf;
+		float2 ptw[R];              // TM: post_tw of the thread's bins
+		if constexpr( TM ) env.template tmem_ld<2 * R>( SY_TM_POST, reinterpret_cast<float *>( ptw ) );
 		if( cur_bulk ) { env.bulk_wait( bar, bulk_phase & 1 ); ++bulk_phase; row = rowbuf + ( row_elem( f ) & 1 ); }
 		else env.cp_async_wait_all();                                            // this thread's bins of row f have landed
+		if constexpr( TM ) env.template tmem_wait<2 * R>( reinterpret_cast<float *>( ptw ) );
 		float2 v[PT];
 #pragma unroll
 		for( int q = 0; q < Q; ++q )
@@ -1028,7 +1137,7 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 				inverse_pv_pair( row[k], row[M - k], acc[q][r][0], acc[q][r][1], a.k, a.P, a.rcpP, xk, xm );
 				// a c2r transform ignores the imaginary parts of bins 0 and N/2 (slot 0 of the irregular pair)
 				if( r == 0 && irr ) { xk.y = 0.0f; xm.y = 0.0f; }
-				const float2 tw = env.ldg2( a.post_tw + k );
+				const float2 tw = TM ? ptw[r] : env.ldg2( a.post_tw + k );
 				const float2 A = add2( xk, pn2( xm ) );
 				const float2 Bv = add2( xk, np2( xm ) );
 				const float2 Qv = cmulc2( Bv, tw );
@@ -1095,7 +1204,15 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 #pragma unroll
 			for( int r = 0; r < PT; ++r ) x1[base + r * R] = v[r];
 			}
-		fft_load_twiddles<M, PT, PT, RP::NS2>( t, tw, a.pass_tw_rev + RP::tw2, ldtw );
+		if constexpr( TM )
+			{
+			float * twf = reinterpret_cast<float *>( tw );
+			env.template tmem_ld<16>( SY_TM_TW, twf );
+			env.template tmem_ld<8>( SY_TM_TW + 16, twf + 16 );
+			env.template tmem_ld<4>( SY_TM_TW + 24, twf + 24 );
+			env.template tmem_ld<2>( SY_TM_TW + 28, twf + 28 );
+			}
+		else fft_load_twiddles<M, PT, PT, RP::NS2>( t, tw, a.pass_tw_rev + RP::tw2, ldtw );
 		env.sync();
 		// pass 2: radix 16, Ns = 16R. Without a fourth pass (T == 16R) its outputs are t + r*T, i.e. v[s] = swapped z[t + s*T]:
 		// y[2n] = v.y, y[2n+1] = v.x
@@ -1105,6 +1222,11 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 			for( int s = 0; s < PT; ++s ) v[s] = base[s * ( T + R * ( T / ( 16 * R ) ) )];
 			}
 		if constexpr( ONE && RP::R3 > 1 ) env.sync();       // everyone has read before anyone writes
+		if constexpr( TM )
+			{
+			env.template tmem_wait<2 * ( PT - 1 )>( reinterpret_cast<float *>( tw ) );
+			env.template tmem_ld<2 * PT>( SY_TM_WIN, w );      // this frame's window, for the overlap-add
+			}
 		fft_butterflies_w<M, PT, PT, RP::NS2>( v, tw );
 		if constexpr( RP::R3 > 1 )
 			{
@@ -1129,6 +1251,7 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 		const unsigned xb = GEN ? (unsigned)( ( (int64_t) hp * f - wp / 2 + t + (int64_t) PT * T * 4096 ) & (int64_t)( PT * T - 1 ) ) * 8u
 		                        : ( (unsigned) t + (unsigned) T * (unsigned)( ( f + 8 ) & 15 ) ) * 8u;
 		auto slot = [&]( int s ) { return reinterpret_cast<float2 *>( reinterpret_cast<char *>( ring ) + ( ( xb + (unsigned)( s * T * 8 ) ) & (unsigned)( 16 * T * 8 - 1 ) ) ); };
+		if constexpr( TM ) env.template tmem_wait<2 * PT>( w );
 		float2 sum[PT];
 #pragma unroll
 		for( int s = 0; s < PT; ++s )

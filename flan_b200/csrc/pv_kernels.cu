@@ -83,10 +83,100 @@ struct DeviceEnv
 #else
 	__device__ __forceinline__ void prefetch( const void * p ) { asm volatile( "prefetch.global.L2 [%0];" :: "l"( p ) ); }
 #endif
+	// Tensor memory as per-thread storage (no MMA): `tmem` is the CTA's allocation plus this warp's lane quarter, so
+	// column j of the calling thread is word j of its private row. tcgen05.ld / .st are .sync.aligned: every lane of the
+	// warp issues them together. A load's registers are defined only after tmem_wait, which also ties them to it so
+	// that no use can be scheduled above the wait.
+	uint32_t tmem;
+	template<int K> __device__ __forceinline__ void tmem_st( int col, const float * r )
+		{
+		static_assert( K == 32, "stores go in 32-column chunks" );
+		asm volatile( "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,"
+		              "%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,%32};"
+		              :: "r"( tmem + (uint32_t) col ),
+		                 "f"( r[0] ), "f"( r[1] ), "f"( r[2] ), "f"( r[3] ), "f"( r[4] ), "f"( r[5] ), "f"( r[6] ), "f"( r[7] ),
+		                 "f"( r[8] ), "f"( r[9] ), "f"( r[10] ), "f"( r[11] ), "f"( r[12] ), "f"( r[13] ), "f"( r[14] ), "f"( r[15] ),
+		                 "f"( r[16] ), "f"( r[17] ), "f"( r[18] ), "f"( r[19] ), "f"( r[20] ), "f"( r[21] ), "f"( r[22] ), "f"( r[23] ),
+		                 "f"( r[24] ), "f"( r[25] ), "f"( r[26] ), "f"( r[27] ), "f"( r[28] ), "f"( r[29] ), "f"( r[30] ), "f"( r[31] ) : "memory" );
+		}
+	__device__ __forceinline__ void tmem_wait_st() { asm volatile( "tcgen05.wait::st.sync.aligned;" ::: "memory" ); }
+	template<int K> __device__ __forceinline__ void tmem_ld( int col, float * r )
+		{
+		const uint32_t a = tmem + (uint32_t) col;
+		if constexpr( K == 2 )
+			asm volatile( "tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0,%1}, [%2];" : "=f"( r[0] ), "=f"( r[1] ) : "r"( a ) );
+		else if constexpr( K == 4 )
+			asm volatile( "tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0,%1,%2,%3}, [%4];" : "=f"( r[0] ), "=f"( r[1] ), "=f"( r[2] ), "=f"( r[3] ) : "r"( a ) );
+		else if constexpr( K == 8 )
+			asm volatile( "tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+			              : "=f"( r[0] ), "=f"( r[1] ), "=f"( r[2] ), "=f"( r[3] ), "=f"( r[4] ), "=f"( r[5] ), "=f"( r[6] ), "=f"( r[7] ) : "r"( a ) );
+		else if constexpr( K == 16 )
+			asm volatile( "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+			              : "=f"( r[0] ), "=f"( r[1] ), "=f"( r[2] ), "=f"( r[3] ), "=f"( r[4] ), "=f"( r[5] ), "=f"( r[6] ), "=f"( r[7] ),
+			                "=f"( r[8] ), "=f"( r[9] ), "=f"( r[10] ), "=f"( r[11] ), "=f"( r[12] ), "=f"( r[13] ), "=f"( r[14] ), "=f"( r[15] ) : "r"( a ) );
+		else if constexpr( K == 32 )
+			asm volatile( "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,"
+			              "%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+			              : "=f"( r[0] ), "=f"( r[1] ), "=f"( r[2] ), "=f"( r[3] ), "=f"( r[4] ), "=f"( r[5] ), "=f"( r[6] ), "=f"( r[7] ),
+			                "=f"( r[8] ), "=f"( r[9] ), "=f"( r[10] ), "=f"( r[11] ), "=f"( r[12] ), "=f"( r[13] ), "=f"( r[14] ), "=f"( r[15] ),
+			                "=f"( r[16] ), "=f"( r[17] ), "=f"( r[18] ), "=f"( r[19] ), "=f"( r[20] ), "=f"( r[21] ), "=f"( r[22] ), "=f"( r[23] ),
+			                "=f"( r[24] ), "=f"( r[25] ), "=f"( r[26] ), "=f"( r[27] ), "=f"( r[28] ), "=f"( r[29] ), "=f"( r[30] ), "=f"( r[31] ) : "r"( a ) );
+		else static_assert( K == 2, "tcgen05.ld widths 2, 4, 8, 16, 32" );
+		}
+	// waits for every outstanding tmem_ld of the thread; the K registers at r are the ones its callers go on to use.
+	// The loads and the wait carry no memory clobber: they touch no memory the compiler sees, so shared- and global-memory
+	// accesses may be scheduled across them.
+	template<int K> __device__ __forceinline__ void tmem_wait( float * r )
+		{
+		asm volatile( "tcgen05.wait::ld.sync.aligned;" );
+#pragma unroll
+		for( int i = 0; i < K; ++i ) asm volatile( "" : "+f"( r[i] ) );
+		}
+	};
+
+// Tensor-memory lifetime of one CTA (128-thread bodies, COLS columns per thread). Warp 0 allocates and gives up its
+// permit to allocate again, the fences order the allocation's shared-memory result around the barrier, and a final
+// barrier on every path precedes the deallocation: a CTA that exited holding columns would leave the SM unable to
+// allocate them. The bodies return to the kernel wrapper on every path (the early return of an empty segment too).
+template<int COLS> struct TmemScope
+	{
+	static_assert( COLS >= 32 && COLS <= 512 && ( COLS & ( COLS - 1 ) ) == 0, "tcgen05.alloc takes a power of two >= 32 columns" );
+	uint32_t * slot;
+	__device__ __forceinline__ explicit TmemScope( uint32_t * s ) : slot( s )
+		{
+		if( threadIdx.x < 32 )
+			{
+			asm volatile( "tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"( (unsigned) __cvta_generic_to_shared( slot ) ), "n"( COLS ) : "memory" );
+			asm volatile( "tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory" );
+			}
+		asm volatile( "tcgen05.fence::before_thread_sync;" ::: "memory" );
+		__syncthreads();
+		asm volatile( "tcgen05.fence::after_thread_sync;" ::: "memory" );
+		}
+	__device__ __forceinline__ uint32_t base() const { return *slot + ( ( threadIdx.x & 96u ) << 16 ); }   // this warp's 32 lanes
+	__device__ __forceinline__ ~TmemScope()
+		{
+		asm volatile( "tcgen05.fence::before_thread_sync;" ::: "memory" );
+		__syncthreads();
+		asm volatile( "tcgen05.fence::after_thread_sync;" ::: "memory" );
+		if( threadIdx.x < 32 ) asm volatile( "tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"( *slot ), "n"( COLS ) : "memory" );
+		}
 	};
 
 // TPS = resident threads per SM the register allocation is sized for (512 -> 128, 768 -> 85, 1024 -> 64 registers).
 constexpr int min_blocks( int threads, int TPS ) { return TPS / threads > 32 ? 32 : ( TPS / threads > 0 ? TPS / threads : 1 ); }
+
+// The analysis instantiations that keep their loop invariants in tensor memory: those whose register budget admits no
+// more CTAs per SM than 512 columns serve (development builds also carry 5- and 6-CTA variants, which keep the L1 form).
+template<int N, int PT, int TPS> constexpr bool analysis_uses_tmem()
+	{
+	return analysis_tmem<N, PT>() && min_blocks( N / ( 2 * PT ), TPS ) * AN_TM_COLS <= 512;
+	}
+
+template<int N, int TPS, bool GEN> constexpr bool synthesis_uses_tmem()
+	{
+	return synthesis_tmem<N, GEN>() && min_blocks( N / 32, TPS ) * SY_TM_COLS <= 512;
+	}
 
 // PT = complex points per thread: 8 (radix-8 passes, N/16 threads per frame) or 16 (radix-16 passes, N/32 threads).
 template<int N, int PT, int TPS, bool ONE, bool PAD = false, bool EMIT = false>
@@ -97,7 +187,14 @@ __global__ void __launch_bounds__( N / ( 2 * PT ), min_blocks( N / ( 2 * PT ), T
 	float2 * x1 = ONE ? x0 : x0 + XBuf<N / 2>::size;
 	int * ssum = EMIT ? reinterpret_cast<int *>( x1 + XBuf<N / 2>::size ) : nullptr;      // N/2 + 1 per-bin sums (EMIT only)
 	DeviceEnv env; env.tid = threadIdx.x;
-	analysis_cta<N, PT, ONE, PAD, EMIT>( a, (int64_t) blockIdx.x, env, x0, x1, ssum );
+	if constexpr( analysis_uses_tmem<N, PT, TPS>() )
+		{
+		__shared__ uint32_t tmem_slot;
+		TmemScope<AN_TM_COLS> scope( &tmem_slot );
+		env.tmem = scope.base();
+		analysis_cta<N, PT, ONE, PAD, EMIT, true>( a, (int64_t) blockIdx.x, env, x0, x1, ssum );
+		}
+	else analysis_cta<N, PT, ONE, PAD, EMIT, false>( a, (int64_t) blockIdx.x, env, x0, x1, ssum );
 	}
 
 // Mirrored last pass (pv_body.cuh: analysis_cta_mirror): 16 points per thread, unpack + phase vocoder on the thread's own registers.
@@ -136,7 +233,14 @@ __global__ void __launch_bounds__( N / 32, min_blocks( N / 32, TPS ) ) pv_synthe
 	float2 * rowbuf = x1 + XBuf<N / 2>::size;                               // N/2 + 2 pairs
 	__shared__ __align__( 8 ) DeviceEnv::BulkBarrier bar;
 	DeviceEnv env; env.tid = threadIdx.x;
-	synthesis_cta_mirror<N, ONE, GEN>( a, (int64_t) blockIdx.x, env, ring, x0, x1, rowbuf, &bar );
+	if constexpr( synthesis_uses_tmem<N, TPS, GEN>() )
+		{
+		__shared__ uint32_t tmem_slot;
+		TmemScope<SY_TM_COLS> scope( &tmem_slot );
+		env.tmem = scope.base();
+		synthesis_cta_mirror<N, ONE, GEN, true>( a, (int64_t) blockIdx.x, env, ring, x0, x1, rowbuf, &bar );
+		}
+	else synthesis_cta_mirror<N, ONE, GEN, false>( a, (int64_t) blockIdx.x, env, ring, x0, x1, rowbuf, &bar );
 	}
 
 // One thread per (channel, segment, bin): summary of the segment's phase increments.
@@ -386,43 +490,58 @@ template<class K> static cudaError_t report_occupancy( K kernel, int threads, si
 	}
 int last_occupancy() { return g_occupancy; }
 
+// CTAs per SM of a kernel that allocates COLS columns of tensor memory. The driver's occupancy query answers 1 for such
+// kernels (measured on a B200, tools/micro/tmem.cu: query 1, 4 resident), so the bound is taken from the register file
+// and the thread limit, and it must not exceed what the columns allow (512 / COLS): surplus CTAs would wait in
+// tcgen05.alloc for others of the same launch to finish. Evaluated once per kernel.
+template<auto KERNEL, int THREADS, int COLS> static cudaError_t tmem_kernel_ctas( int * ctas )
+	{
+	static int n = 0;
+	static const cudaError_t r = []
+		{
+		cudaFuncAttributes fa;
+		const cudaError_t e = cudaFuncGetAttributes( &fa, KERNEL );
+		if( e != cudaSuccess ) return e;
+		const int by_regs = 65536 / ( ( fa.numRegs > 0 ? fa.numRegs : 1 ) * THREADS ), by_threads = 2048 / THREADS;
+		n = by_regs < by_threads ? by_regs : by_threads;
+		return n * COLS <= 512 ? cudaSuccess : cudaErrorInvalidConfiguration;
+		}();
+	*ctas = n;
+	return r;
+	}
+template<int N, int PT, int TPS, bool ONE, bool PAD, bool EMIT> static cudaError_t launch_analysis_kernel( const AnalysisArgs & a, int64_t blocks, size_t smem, cudaStream_t st )
+	{
+	auto kernel = pv_analysis_kernel<N, PT, TPS, ONE, PAD, EMIT>;
+	cudaError_t e = cudaFuncSetAttribute( kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem );
+	if( e != cudaSuccess ) return e;
+	apply_carveout( kernel );
+	if constexpr( analysis_uses_tmem<N, PT, TPS>() )
+		{
+		int ctas = 0;
+		e = tmem_kernel_ctas<pv_analysis_kernel<N, PT, TPS, ONE, PAD, EMIT>, N / ( 2 * PT ), AN_TM_COLS>( &ctas );
+		if( e != cudaSuccess ) return e;
+		if( blocks < 0 ) { g_occupancy = ctas; return cudaSuccess; }
+		}
+	if( blocks < 0 ) return report_occupancy( kernel, N / ( 2 * PT ), smem );
+	kernel<<<(unsigned) blocks, N / ( 2 * PT ), smem, st>>>( a );
+	return cudaGetLastError();
+	}
 template<int N, int PT, int TPS, bool ONE> static cudaError_t launch_analysis_nto( const AnalysisArgs & a, int64_t blocks, cudaStream_t st )
 	{
 	const size_t smem = ( ONE ? 1 : 2 ) * sizeof( float2 ) * XBuf<N / 2>::size + smem_pad();
-	cudaError_t e = cudaFuncSetAttribute( pv_analysis_kernel<N, PT, TPS, ONE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem );
-	if( e != cudaSuccess ) return e;
-	apply_carveout( pv_analysis_kernel<N, PT, TPS, ONE> );
 	// zero-padded windows that fill whole slots (the API default shape): vector loads, 16 points per thread form only
 	if constexpr( PT == 16 && ONE )
 		{
-		if( a.W < N && a.W % ( N / PT ) == 0 && a.aligned2 )
-			{
-			e = cudaFuncSetAttribute( pv_analysis_kernel<N, PT, TPS, ONE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem );
-			if( e != cudaSuccess ) return e;
-			if( blocks < 0 ) return report_occupancy( pv_analysis_kernel<N, PT, TPS, ONE, true>, N / ( 2 * PT ), smem );
-			pv_analysis_kernel<N, PT, TPS, ONE, true><<<(unsigned) blocks, N / ( 2 * PT ), smem, st>>>( a );
-			return cudaGetLastError();
-			}
+		if( a.W < N && a.W % ( N / PT ) == 0 && a.aligned2 ) return launch_analysis_kernel<N, PT, TPS, ONE, true, false>( a, blocks, smem, st );
 		}
 	// the full-window launch that also leaves the phase summaries of its rows (16 points per thread, one buffer, TPS 512: the
 	// policy's variant from dft 2048 up)
 	if constexpr( PT == 16 && ONE && TPS == 512 && N >= 2048 )
 		{
-		if( a.seg_out )
-			{
-			const size_t smem_emit = smem + sizeof( int ) * ( N / 2 + 4 );
-			e = cudaFuncSetAttribute( pv_analysis_kernel<N, PT, TPS, ONE, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem_emit );
-			if( e != cudaSuccess ) return e;
-			apply_carveout( pv_analysis_kernel<N, PT, TPS, ONE, false, true> );
-			if( blocks < 0 ) return report_occupancy( pv_analysis_kernel<N, PT, TPS, ONE, false, true>, N / ( 2 * PT ), smem_emit );
-			pv_analysis_kernel<N, PT, TPS, ONE, false, true><<<(unsigned) blocks, N / ( 2 * PT ), smem_emit, st>>>( a );
-			return cudaGetLastError();
-			}
+		if( a.seg_out ) return launch_analysis_kernel<N, PT, TPS, ONE, false, true>( a, blocks, smem + sizeof( int ) * ( N / 2 + 4 ), st );
 		}
 	if( a.seg_out ) return cudaErrorInvalidValue;          // the caller asks for summaries only where this form exists
-	if( blocks < 0 ) return report_occupancy( pv_analysis_kernel<N, PT, TPS, ONE>, N / ( 2 * PT ), smem );
-	pv_analysis_kernel<N, PT, TPS, ONE><<<(unsigned) blocks, N / ( 2 * PT ), smem, st>>>( a );
-	return cudaGetLastError();
+	return launch_analysis_kernel<N, PT, TPS, ONE, false, false>( a, blocks, smem, st );
 	}
 // the one-buffer form is built for 16 points per thread only (the variant the large transforms use)
 template<int N, int PT, int TPS> static cudaError_t launch_analysis_nt( const AnalysisArgs & a, int64_t blocks, cudaStream_t st )
@@ -502,6 +621,13 @@ template<int N, int TPS, bool ONE, bool GEN> static cudaError_t launch_synthesis
 	cudaError_t e = cudaFuncSetAttribute( pv_synthesis_mirror_kernel<N, TPS, ONE, GEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem );
 	if( e != cudaSuccess ) return e;
 	apply_carveout( pv_synthesis_mirror_kernel<N, TPS, ONE, GEN> );
+	if constexpr( synthesis_uses_tmem<N, TPS, GEN>() )
+		{
+		int ctas = 0;
+		e = tmem_kernel_ctas<pv_synthesis_mirror_kernel<N, TPS, ONE, GEN>, N / 32, SY_TM_COLS>( &ctas );
+		if( e != cudaSuccess ) return e;
+		if( blocks < 0 ) { g_occupancy = ctas; return cudaSuccess; }
+		}
 	if( blocks < 0 ) return report_occupancy( pv_synthesis_mirror_kernel<N, TPS, ONE, GEN>, N / 32, smem );
 	pv_synthesis_mirror_kernel<N, TPS, ONE, GEN><<<(unsigned) blocks, N / 32, smem, st>>>( a );
 	return cudaGetLastError();
@@ -542,6 +668,8 @@ template<int N> static cudaError_t launch_synthesis_n( const SynthArgs & a, int6
 			if( tps >= 512 ) return a.one_buffer ? launch_synthesis_mirror_nt<N, 512, true>( a, blocks, st ) : launch_synthesis_mirror_nt<N, 512, false>( a, blocks, st );
 			if( a.one_buffer ) return launch_synthesis_mirror_nt<N, 384, true>( a, blocks, st );
 #endif
+			// dft 4096, standard shape: window and tables in tensor memory, 128 registers, one exchange buffer, 4 CTAs per SM
+			if constexpr( N == 4096 ) { if( a.W == N && a.hop == N / 16 ) return launch_synthesis_mirror_ntg<N, 512, true, false>( a, blocks, st ); }
 			return launch_synthesis_mirror_nt<N, 384, false>( a, blocks, st );
 			}
 		}
