@@ -46,10 +46,12 @@ def debug_lib_path():
 
 def build_library(force=False, verbose=False, debug=False):
     os.makedirs(LIB, exist_ok=True)
-    # (source, extra flags): the PV-domain kernels must reproduce the reference's float arithmetic bit for bit, so
-    # their translation unit is compiled without FMA contraction.
+    # (source, extra flags): the PV-domain kernels must reproduce the reference's float arithmetic bit for bit, and the
+    # expression kernels the host evaluation of flan_b200_fx_eval, so their translation units are compiled without FMA
+    # contraction.
     units = [("pv_kernels.cu", []), ("pv_capi.cu", []), ("pv_capi_modify.cu", []), ("pv_capi_io.cu", []),
-             ("pv_modify.cu", ["-fmad=false"]), ("pv_io.cu", ["-fmad=false"])]
+             ("pv_capi_fx.cu", []), ("pv_modify.cu", ["-fmad=false"]), ("pv_io.cu", ["-fmad=false"]),
+             ("pv_fx.cu", ["-fmad=false"])]
     units = [u for u in units if os.path.exists(os.path.join(CSRC, u[0]))]
     for extra_unit in ("pv_generic.cu", "pv_capi_multi.cu", "pv_capi_exchange.cu"):
         if os.path.exists(os.path.join(CSRC, extra_unit)):
@@ -107,6 +109,16 @@ def wav_test_path():
     return os.path.join(LIB, "libflan_wav_test.so")
 
 
+def fx_test_path():
+    """tests/cpp/fx_driver.cpp: expression Functions (flan/fx.h) and their lambdas through the PV-domain methods."""
+    return os.path.join(LIB, "libflan_fx_test.so")
+
+
+def fx_bench_path():
+    """tools/cpp/fx_bench.cpp: the PV-domain methods timed with lambdas and expressions (tools/fxbench.py)."""
+    return os.path.join(LIB, "libflan_fx_bench.so")
+
+
 def e2e_bench_path():
     return os.path.join(LIB, "libflan_e2e_bench.so")
 
@@ -116,7 +128,7 @@ def build_host(force=False):
     build_library(force)
     os.makedirs(LIB, exist_ok=True)
     root = os.path.dirname(HERE)
-    srcs = [os.path.join(HOST, "src", n) for n in ("b200_storage.cpp", "AudioBuffer.cpp", "PVBuffer.cpp", "AudioPV.cpp", "PVModify.cpp")]
+    srcs = [os.path.join(HOST, "src", n) for n in ("b200_storage.cpp", "AudioBuffer.cpp", "PVBuffer.cpp", "AudioPV.cpp", "PVModify.cpp", "fx.cpp")]
     hdrs = []
     for d, _, files in os.walk(os.path.join(HOST, "include")):
         hdrs += [os.path.join(d, f) for f in files]
@@ -131,9 +143,15 @@ def build_host(force=False):
     wav_drv = os.path.join(root, "tests", "cpp", "wav_formats_driver.cpp")
     if os.path.exists(wav_drv) and (force or _newer(wav_test_path(), [wav_drv, host_path()] + hdrs)):
         subprocess.run(common + ["-o", wav_test_path(), wav_drv] + link + ["-lflan_b200_host", "-lflan_b200"], check=True)
+    fx_drv = os.path.join(root, "tests", "cpp", "fx_driver.cpp")
+    if force or _newer(fx_test_path(), [fx_drv, host_path()] + hdrs):
+        subprocess.run(common + ["-o", fx_test_path(), fx_drv] + link + ["-lflan_b200_host", "-lflan_b200"], check=True)
     e2e = os.path.join(root, "tools", "cpp", "e2e_bench.cpp")
     if os.path.exists(e2e) and (force or _newer(e2e_bench_path(), [e2e, host_path()] + hdrs)):
         subprocess.run(common + ["-o", e2e_bench_path(), e2e] + link + ["-lflan_b200_host", "-lflan_b200", "-lpthread"], check=True)
+    fxb = os.path.join(root, "tools", "cpp", "fx_bench.cpp")
+    if os.path.exists(fxb) and (force or _newer(fx_bench_path(), [fxb, host_path()] + hdrs)):
+        subprocess.run(common + ["-o", fx_bench_path(), fxb] + link + ["-lflan_b200_host", "-lflan_b200"], check=True)
     ex = os.path.join(root, "examples", "pv_chain.cpp")
     exe = os.path.join(LIB, "pv_chain")
     if os.path.exists(ex) and (force or _newer(exe, [ex, host_path()] + hdrs)):

@@ -36,6 +36,48 @@ class ShardedPV(ctypes.Structure):
 
 _pa, _pp = ctypes.POINTER(ShardedAudio), ctypes.POINTER(ShardedPV)
 
+# expression programs (flan_b200_fx_program): op codes in the order of the header's enum
+FX_MAX_OPS, FX_MAX_STACK, FX_MAX_CURVES, FX_MAX_POINTS = 64, 16, 8, 64
+FX_OPS = ["t", "f", "const", "add", "sub", "mul", "div", "min", "max", "lt", "le", "gt", "ge", "eq", "ne", "pow",
+          "neg", "abs", "floor", "ceil", "round", "sqrt", "sin", "cos", "exp", "log", "curve", "where"]
+FX = {name: code for code, name in enumerate(FX_OPS)}
+
+
+class FxOp(ctypes.Structure):
+    _fields_ = [("code", ctypes.c_int32), ("index", ctypes.c_int32), ("value", _f)]
+
+
+class FxCurve(ctypes.Structure):
+    _fields_ = [("points", ctypes.c_int32), ("interp", ctypes.c_int32),
+                ("x", _f * FX_MAX_POINTS), ("y", _f * FX_MAX_POINTS)]
+
+
+class FxProgram(ctypes.Structure):
+    _fields_ = [("ops", ctypes.c_int32), ("curves", ctypes.c_int32),
+                ("op", FxOp * FX_MAX_OPS), ("curve", FxCurve * FX_MAX_CURVES)]
+
+
+def fx_program(ops, curves=()):
+    """ops: postfix list of op names, floats (constants) or ("curve", index); curves: (points [(x, y), ...], interp)."""
+    p = FxProgram()
+    p.ops = len(ops)
+    for i, o in enumerate(ops):
+        if isinstance(o, (int, float)) and not isinstance(o, bool):
+            p.op[i].code, p.op[i].value = FX["const"], float(o)
+        elif isinstance(o, tuple):
+            p.op[i].code, p.op[i].index = FX[o[0]], o[1]
+        else:
+            p.op[i].code = FX[o]
+    p.curves = len(curves)
+    for c, (pts, interp) in enumerate(curves):
+        p.curve[c].points, p.curve[c].interp = len(pts), interp
+        for j, (x, y) in enumerate(pts):
+            p.curve[c].x[j], p.curve[c].y[j] = x, y
+    return p
+
+
+_px = ctypes.POINTER(FxProgram)
+
 # every symbol include/flan_b200.h declares: (name, restype, argtypes)
 SYMBOLS = [
     ("flan_b200_device_count", _int, []),
@@ -89,6 +131,11 @@ SYMBOLS = [
     ("flan_b200_modify_time", _int, [_vp, _vp, _int, _i64, _int, _f, _f, _vp, _i64, _int, _int, _i64, _vp, _int]),
     ("flan_b200_promise_unchanged", _int, [_vp, _vp]),
     ("flan_b200_hint_resynthesis", _int, [_vp]),
+    ("flan_b200_fx_check", _int, [_px, ctypes.POINTER(_int), ctypes.POINTER(_int)]),
+    ("flan_b200_fx_last_error", ctypes.c_char_p, []),
+    ("flan_b200_fx_eval", _int, [_px, _f, _f, ctypes.POINTER(_f)]),
+    ("flan_b200_fx_sample", _int, [_vp, _px, _i64, _int, _f, _f, _vp, ctypes.POINTER(_i64), ctypes.POINTER(_int)]),
+    ("flan_b200_fx_at_pv", _int, [_vp, _px, _vp, _int, _i64, _int, _f, _vp]),
     ("flan_b200_flan_encode", _int, [_vp, _vp, _i64, _f, _f, _vp]),
     ("flan_b200_flan_decode", _int, [_vp, _vp, _i64, _f, _f, _vp]),
     ("flan_b200_save_flan", _int, [_vp, ctypes.c_char_p, _vp, _int, _i64, _int, _f, _f, _int]),

@@ -229,6 +229,28 @@ class Engine:
         C, F, B, _ = pv.shape
         return self.modify_time(pv, sr, ar, self.stretch_map(F, B, sr, ar, factor), interp, summary_window)
 
+    # -- expression Functions (flan_b200_fx_*): a capi.FxProgram sampled on the grid or evaluated at every MF -------
+    def fx_sample(self, prog, F, B, time_step, bin_width):
+        """The program over the F x B grid, in the view its dependence selects: [F, B], [F, 1], [B] or [1]."""
+        ut, uf = ctypes.c_int(), ctypes.c_int()
+        if self.lib.flan_b200_fx_check(ctypes.byref(prog), ctypes.byref(ut), ctypes.byref(uf)) != capi.OK:
+            raise capi.FlanB200Error(capi.INVALID, self.lib.flan_b200_fx_last_error().decode())
+        shape = {(1, 1): (F, B), (1, 0): (F, 1), (0, 1): (B,), (0, 0): (1,)}[(ut.value, uf.value)]
+        out = torch.empty(shape, dtype=torch.float32, device=self.device)
+        fs, bs = ctypes.c_int64(), ctypes.c_int()
+        self._bind_stream()
+        self.ctx.call("flan_b200_fx_sample", ctypes.byref(prog), F, B, time_step, bin_width, self._chk(out),
+                      ctypes.byref(fs), ctypes.byref(bs))
+        return out
+
+    def fx_at_pv(self, prog, pv, frame_rate):
+        """program( float(x) / frame_rate, pv[c, x, b].f ) for every MF: cuda float32 [C, F, B]."""
+        C, F, B, _ = pv.shape
+        out = torch.empty((C, F, B), dtype=torch.float32, device=self.device)
+        self._bind_stream()
+        self.ctx.call("flan_b200_fx_at_pv", ctypes.byref(prog), self._chk(pv), C, F, B, frame_rate, self._chk(out))
+        return out
+
     # -- file formats either side of the path (PVBuffer::save / load, AudioBuffer::save / load) -----------------
     def flan_encode(self, pv, sr):
         C, F, B, _ = pv.shape

@@ -27,8 +27,14 @@ public:
 	Audio convert_to_lr_audio( flan_CANCEL_ARG ) const;
 
 	// ---- PV-domain chain (reference PV/PVModify.cpp:196-385), on the GPU, data stays device-resident -------------
-	// The Function argument is sampled over the frame x bin grid on the host, as the reference does (PV.h:31-35); a
-	// constant Function is passed to the device as a single value. NOTE: in the reference a constant Function makes
+	// A lambda Function argument is sampled over the frame x bin grid on the host, as the reference does (PV.h:31-35); a
+	// constant Function is passed to the device as a single value. An expression of t and f (flan/fx.h, e.g.
+	// `1.0f + fx::t / 20.0f`) is sampled on the GPU into the table its dependence needs -- one value, one per frame, one
+	// per bin, or the grid -- so a time-only stretch / modify_time and a frequency-only repitch take the kernels a
+	// constant takes, modify_frequency evaluates it at every MF on the device without downloading the PV, and on a sharded
+	// PV a time-only stretch / modify_time keeps the shards. Same results as the lambda [&]( TF x ){ return e( x ); }.
+	// An invalid expression (past its limits, or a curve with a user-callable Interpolator) prints why and yields a null
+	// PV. NOTE: in the reference a constant Function makes
 	// repitch / stretch alias one scalar (FunctionSample.h:185-189: `at( f, b ) += at( f, b - 1 )` doubles it every
 	// step until it overflows), which is undefined further down (float -> int of inf, PVModify.cpp:222,312-315); here
 	// a constant behaves like the lambda that returns it -- the evident intent. Named interpolators only

@@ -1,7 +1,8 @@
 // PV-domain methods of the B200 build: PV::repitch, PV::stretch, PV::modify_time, PV::modify_frequency with the
 // reference's signatures (src/flan/PV/PV.h:276-310, bodies PV/PVModify.cpp:196-385). The host does what only the host
 // can do -- call the user's Function over the frame x bin grid (PV.h:31-35, Function.h:155-171) -- and the C ABI of
-// libflan_b200.so (include/flan_b200.h) does the arithmetic on the device-resident PV data.
+// libflan_b200.so (include/flan_b200.h) does the arithmetic on the device-resident PV data. An expression Function
+// (flan/fx.h) is sampled on the device instead, into the compact table its dependence allows.
 #include "flan/PV/PV.h"
 
 #include <algorithm>
@@ -51,8 +52,29 @@ template<class Body> void for_rows( ExecutionPolicy policy, Frame rows, Body bod
 	for( auto & t : pool ) t.join();
 	}
 
+// The program of an expression Function that is valid, else null after printing why it is not (also null for any other
+// Function, silently).
+const flan_b200_fx_program * expr_program( const char * what, const Function<TF, float> & f )
+	{
+	const fx::Expr * e = f.expr();
+	if( e && !e->valid() ) std::cout << "flan::" << what << ": " << e->error() << std::endl;
+	return e ? e->program() : nullptr;
+	}
+bool invalid_expr( const char * what, const Function<TF, float> & f ) { return f.expr() && !expr_program( what, f ); }
+
+// What an expression reads decides the view it is sampled into: (B, 1) for t and f, (1, 0) for t, (0, 1) for f, (0, 0)
+// for neither.
+void expr_view( const flan_b200_fx_program * p, Frame F, Bin B, Frame * rows, Bin * cols, int64_t * frame_stride, int * bin_stride )
+	{
+	int ut = 0, uf = 0;
+	flan_b200_fx_check( p, &ut, &uf );
+	*rows = ut ? F : 1; *cols = uf ? B : 1;
+	*frame_stride = ut ? *cols : 0; *bin_stride = uf ? 1 : 0;
+	}
+
 // sample_function_over_domain (PV.h:31-35): value( frame, bin ) = f( { frame * ( 1 / analysis_rate ), bin * bin_to_frequency( 1 ) } ).
-// Host memory; *frame_stride, *bin_stride: (0, 0) for a constant, (B, 1) otherwise.
+// Host memory; *frame_stride, *bin_stride: (0, 0) for a constant, the expression's view (expr_view) for a valid
+// expression, (B, 1) otherwise.
 std::vector<float> sample_on_host( const PV & pv, const Function<TF, float> & f, int64_t * frame_stride, int * bin_stride )
 	{
 	const Frame F = pv.get_num_frames();
@@ -61,6 +83,17 @@ std::vector<float> sample_on_host( const PV & pv, const Function<TF, float> & f,
 	*frame_stride = 0; *bin_stride = 0;
 	if( f.is_constant() )
 		host.assign( 1, f( TF{ 0, 0 } ) );
+	else if( const flan_b200_fx_program * p = expr_program( "PV", f ) )
+		{
+		Frame rows; Bin cols;
+		expr_view( p, F, B, &rows, &cols, frame_stride, bin_stride );
+		host.resize( size_t( rows ) * size_t( cols ) );
+		const float x_scale = 1.0f / pv.get_analysis_rate(), y_scale = pv.bin_to_frequency( 1 );
+		for_rows( f.get_execution_policy(), rows, [&]( Frame x )
+			{
+			for( Bin y = 0; y < cols; ++y ) flan_b200_fx_eval( p, x * x_scale, y * y_scale, &host[size_t( x ) * cols + y] );
+			} );
+		}
 	else
 		{
 		host.resize( size_t( F ) * size_t( B ) );
@@ -74,17 +107,30 @@ std::vector<float> sample_on_host( const PV & pv, const Function<TF, float> & f,
 	return host;
 	}
 
-bool sample_over_domain( const PV & pv, const Function<TF, float> & f, DeviceTable & t )
-	{
-	t.data = b200::Mirror<float>( sample_on_host( pv, f, &t.frame_stride, &t.bin_stride ) );
-	t.d = t.data.device();
-	return t.d != nullptr;
-	}
-
 int report( flan_b200_ctx * ctx, const char * what, int rc )
 	{
 	if( rc != FLAN_B200_OK ) std::cout << "flan::" << what << " failed on the GPU engine: " << flan_b200_last_error( ctx ) << std::endl;
 	return rc;
+	}
+
+// The same table on the device. An expression is sampled there (flan_b200_fx_sample), in its compact view.
+bool sample_over_domain( const char * what, const PV & pv, const Function<TF, float> & f, DeviceTable & t )
+	{
+	if( const flan_b200_fx_program * p = expr_program( what, f ) )
+		{
+		Frame rows; Bin cols;
+		expr_view( p, pv.get_num_frames(), pv.get_num_bins(), &rows, &cols, &t.frame_stride, &t.bin_stride );
+		float * d = nullptr;
+		t.data = b200::Mirror<float>::device_result( size_t( rows ) * size_t( cols ), &d );
+		flan_b200_ctx * ctx = b200::context();
+		if( !d || !ctx || report( ctx, what, flan_b200_fx_sample( ctx, p, pv.get_num_frames(), pv.get_num_bins(), 1.0f / pv.get_analysis_rate(),
+				pv.bin_to_frequency( 1 ), d, &t.frame_stride, &t.bin_stride ) ) ) return false;
+		t.d = d;
+		return true;
+		}
+	t.data = b200::Mirror<float>( sample_on_host( pv, f, &t.frame_stride, &t.bin_stride ) );
+	t.d = t.data.device();
+	return t.d != nullptr;
 	}
 
 int device_interp( const char * what, const Interpolator & interp )
@@ -146,11 +192,11 @@ PV PV::repitch( const Function<TF, float> & factor, const Interpolator & interp 
 	{
 	if( is_null() ) return PV();                                         // PVModify.cpp:202
 	const int id = device_interp( "PV::repitch", interp );
-	if( id < 0 ) return PV();
+	if( id < 0 || invalid_expr( "PV::repitch", factor ) ) return PV();
 	if( auto sharded = on_shards( *this, "PV::repitch", flan_b200_multi_repitch, factor, id, false ) ) return std::move( *sharded );
 	flan_b200_ctx * ctx = b200::context();
 	DeviceTable t;
-	if( id < 0 || !ctx || !sample_over_domain( *this, factor, t ) ) return PV();
+	if( id < 0 || !ctx || !sample_over_domain( "PV::repitch", *this, factor, t ) ) return PV();
 	const MF * d_pv = storage().device();
 	MF * d_out = nullptr;
 	b200::Mirror<MF> data = b200::Mirror<MF>::device_result( storage().size(), &d_out );
@@ -168,19 +214,35 @@ PV PV::modify_frequency( const Function<TF, Frequency> & mod, const Interpolator
 	const int id = device_interp( "PV::modify_frequency", interp );
 	flan_b200_ctx * ctx = b200::context();
 	DeviceTable t;
-	if( id < 0 || !ctx || !sample_over_domain( *this, mod, t ) ) return PV();
-	// mod evaluated at every MF's own frequency (PVModify.cpp:263-268): a user lambda of the data, so it runs here
-	const std::vector<MF> & host = get_buffer();
-	std::vector<float> in_modified( host.size() );
+	if( id < 0 || invalid_expr( "PV::modify_frequency", mod ) || !ctx || !sample_over_domain( "PV::modify_frequency", *this, mod, t ) ) return PV();
 	const Frame F = get_num_frames(); const Bin B = get_num_bins();
-	for_rows( mod.get_execution_policy(), Frame( get_num_channels() ) * F, [&]( Frame row )
+	// mod evaluated at every MF's own frequency (PVModify.cpp:263-268)
+	b200::Mirror<float> in_mod;
+	const float * d_in_mod = nullptr;
+	if( const flan_b200_fx_program * p = expr_program( "PV::modify_frequency", mod ) )
 		{
-		const Frame frame = row % F;
-		for( Bin bin = 0; bin < B; ++bin )
-			in_modified[size_t( row ) * B + bin] = mod( TF{ frame_to_time( frame ), host[size_t( row ) * B + bin].f } );
-		} );
-	b200::Mirror<float> in_mod( std::move( in_modified ) );
-	const float * d_in_mod = in_mod.device();
+		// an expression: on the device, from the device copy of the PV (frame_to_time( x ) = x / ( sr / hop ))
+		const MF * d_src = storage().device();
+		float * d = nullptr;
+		in_mod = b200::Mirror<float>::device_result( storage().size(), &d );
+		if( !d_src || !d || report( ctx, "PV::modify_frequency", flan_b200_fx_at_pv( ctx, p, as_floats( d_src ), get_num_channels(), F, B,
+				float( get_sample_rate() ) / float( get_hop_size() ), d ) ) ) return PV();
+		d_in_mod = d;
+		}
+	else
+		{
+		// a user lambda of the data, so it runs here
+		const std::vector<MF> & host = get_buffer();
+		std::vector<float> in_modified( host.size() );
+		for_rows( mod.get_execution_policy(), Frame( get_num_channels() ) * F, [&]( Frame row )
+			{
+			const Frame frame = row % F;
+			for( Bin bin = 0; bin < B; ++bin )
+				in_modified[size_t( row ) * B + bin] = mod( TF{ frame_to_time( frame ), host[size_t( row ) * B + bin].f } );
+			} );
+		in_mod = b200::Mirror<float>( std::move( in_modified ) );
+		d_in_mod = in_mod.device();
+		}
 	const MF * d_pv = storage().device();
 	MF * d_out = nullptr;
 	b200::Mirror<MF> data = b200::Mirror<MF>::device_result( storage().size(), &d_out );
@@ -194,10 +256,10 @@ PV PV::modify_time( const Function<TF, Second> & mod, const Interpolator & inter
 	{
 	if( is_null() ) return PV();                                         // PVModify.cpp:309
 	const int id = device_interp( "PV::modify_time", interp );
-	if( id < 0 ) return PV();
+	if( id < 0 || invalid_expr( "PV::modify_time", mod ) ) return PV();
 	if( auto sharded = on_shards( *this, "PV::modify_time", flan_b200_multi_modify_time, mod, id, true ) ) return std::move( *sharded );
 	DeviceTable t;
-	if( id < 0 || !b200::context() || !sample_over_domain( *this, mod, t ) ) return PV();
+	if( id < 0 || !b200::context() || !sample_over_domain( "PV::modify_time", *this, mod, t ) ) return PV();
 	return modify_time_on_device( *this, "PV::modify_time", t.d, t.frame_stride, t.bin_stride, id );
 	}
 
@@ -205,11 +267,11 @@ PV PV::stretch( const Function<TF, float> & factor, const Interpolator & interp 
 	{
 	if( is_null() ) return PV();
 	const int id = device_interp( "PV::stretch", interp );
-	if( id < 0 ) return PV();
+	if( id < 0 || invalid_expr( "PV::stretch", factor ) ) return PV();
 	if( auto sharded = on_shards( *this, "PV::stretch", flan_b200_multi_stretch, factor, id, true ) ) return std::move( *sharded );
 	flan_b200_ctx * ctx = b200::context();
 	DeviceTable t;
-	if( id < 0 || !ctx || !sample_over_domain( *this, factor, t ) ) return PV();
+	if( id < 0 || !ctx || !sample_over_domain( "PV::stretch", *this, factor, t ) ) return PV();
 	// running sum along frames, frames -> seconds (PVModify.cpp:373-382), on the device
 	const int cols = t.bin_stride ? get_num_bins() : 1;
 	float * d_map = nullptr;

@@ -199,7 +199,8 @@ int flan_b200_mid_side( flan_b200_ctx * ctx, const float * d_in, float * d_out, 
  * PV::repitch / PV::modify_frequency (src/flan/PV/PVModify.cpp:196-305, decl PV/PV.h:288-330) and PV::stretch /
  * PV::modify_time (PVModify.cpp:307-385, decl PV/PV.h:300-352) on device-resident PV data. Results are bit-identical
  * to the reference's float arithmetic for interpolators 0-6 and 9; 7 (sine) and 8 (sine2) evaluate cos / sin in
- * double and round, which differs from glibc's cosf in the last bit for a few inputs per thousand.
+ * double and round, which differs from glibc's cosf in the last bit for a few inputs per thousand. Expression
+ * Functions (flan_b200_fx_*, below) take the same approach for their transcendental ops, with the same caveat.
  *
  * The reference samples its Function<TF,float> argument over the frame x bin grid on the host (PV/PV.h:31-35);
  * here the sampled table arrives as a strided device view: element (frame, bin) = d_table[frame * frame_stride +
@@ -251,6 +252,63 @@ int flan_b200_promise_unchanged( flan_b200_ctx * ctx, const float * d_pv );
  * read of the rows (0.56 of 3.9 ms on cfg2). flan_b200_convert_to_pv_range consumes the hint too (a shard of a per-GPU
  * process: flan_b200_promise_unchanged before flan_b200_phase_summary then uses what it left). */
 int flan_b200_hint_resynthesis( flan_b200_ctx * ctx );
+
+/* ---- expression Functions: a Function<TF, float> as a program of t and f (flan/fx.h) ------------------------------
+ * Postfix ops over a value stack, float constants and breakpoint curves. What a program depends on is known from its ops,
+ * so it is sampled on the device into the compact view that dependence allows, and evaluated on the host by the same
+ * source (flan_b200/csrc/pv_fx.cuh). Every node is one IEEE float32 operation with round to nearest, without contraction,
+ * reassociation or folding, in the order of the ops. Operands: a binary op takes x (pushed first) and y (on top) and
+ * pushes x op y; WHERE takes c, a, b and pushes c != 0 ? a : b; comparisons push 1.0f or 0.0f; MIN / MAX have fminf /
+ * fmaxf semantics (a NaN operand yields the other one) with -0 < +0; ROUND is roundf (half away from zero). CURVE pops x
+ * and pushes the envelope curve[index]: x <= x_0 gives y_0, x >= x_last gives y_last, NaN gives NaN, otherwise
+ * y_i + interp( u ) * ( y_{i+1} - y_i ), u = ( x - x_i ) / ( x_{i+1} - x_i ), x_i <= x < x_{i+1}, interp one of the ids
+ * 0-9 above. SIN, COS, EXP, LOG and POW compute ( float ) fn( ( double ) x ) on both sides; like interpolators 7 and 8
+ * they are where host and device may differ: CUDA's and glibc's double results can round to different floats near a
+ * tie. A NaN result is always the quiet NaN 0x7fc00000, on both sides (their hardware makes different NaN bits). Every
+ * entry point validates the program (op codes, stack depth, a single result, curve indices, at least one
+ * point per curve, finite and strictly ascending x, finite y, interpolator ids) and returns FLAN_B200_INVALID with a
+ * message (flan_b200_fx_last_error) for a bad one. */
+#define FLAN_B200_FX_MAX_OPS     64
+#define FLAN_B200_FX_MAX_STACK   16
+#define FLAN_B200_FX_MAX_CURVES  8
+#define FLAN_B200_FX_MAX_POINTS  64
+enum
+	{
+	FLAN_B200_FX_T, FLAN_B200_FX_F, FLAN_B200_FX_CONST,                                                     /* push */
+	FLAN_B200_FX_ADD, FLAN_B200_FX_SUB, FLAN_B200_FX_MUL, FLAN_B200_FX_DIV, FLAN_B200_FX_MIN, FLAN_B200_FX_MAX,
+	FLAN_B200_FX_LT, FLAN_B200_FX_LE, FLAN_B200_FX_GT, FLAN_B200_FX_GE, FLAN_B200_FX_EQ, FLAN_B200_FX_NE,
+	FLAN_B200_FX_POW,                                                                                       /* x op y */
+	FLAN_B200_FX_NEG, FLAN_B200_FX_ABS, FLAN_B200_FX_FLOOR, FLAN_B200_FX_CEIL, FLAN_B200_FX_ROUND, FLAN_B200_FX_SQRT,
+	FLAN_B200_FX_SIN, FLAN_B200_FX_COS, FLAN_B200_FX_EXP, FLAN_B200_FX_LOG, FLAN_B200_FX_CURVE,              /* op x */
+	FLAN_B200_FX_WHERE,                                                                                     /* c a b */
+	FLAN_B200_FX_OP_COUNT
+	};
+typedef struct { int32_t code; int32_t index; float value; } flan_b200_fx_op;   /* value: CONST; index: CURVE */
+typedef struct { int32_t points; int32_t interp; float x[FLAN_B200_FX_MAX_POINTS], y[FLAN_B200_FX_MAX_POINTS]; } flan_b200_fx_curve;
+typedef struct flan_b200_fx_program
+	{
+	int32_t ops, curves;
+	flan_b200_fx_op op[FLAN_B200_FX_MAX_OPS];
+	flan_b200_fx_curve curve[FLAN_B200_FX_MAX_CURVES];
+	} flan_b200_fx_program;
+/* Validation and dependence: *uses_t / *uses_f (may be NULL) say whether the program reads t / f. */
+int flan_b200_fx_check( const flan_b200_fx_program * prog, int * uses_t, int * uses_f );
+/* Text of the calling thread's last failure of a flan_b200_fx_* call. */
+const char * flan_b200_fx_last_error( void );
+/* The host evaluation, the code the kernels run: *out = program( t, f ). */
+int flan_b200_fx_eval( const flan_b200_fx_program * prog, float t, float f, float * out );
+/* sample_function_over_domain (PV/PV.h:31-35) on the device: value( x, y ) = program( float( x ) * time_step,
+ * float( y ) * bin_width ), with time_step = 1.0f / analysis_rate and bin_width = bin_to_frequency( 1 ), as PV::repitch
+ * samples a lambda. Only what the program depends on is written: d_out receives frames * bins values (strides (bins, 1))
+ * when it reads t and f, frames values (1, 0) for t alone, bins values (0, 1) for f alone, one value (0, 0) for neither:
+ * the views of the PV-domain entry points above. flan_b200_fx_check tells the size in advance. Indices are 64-bit. */
+int flan_b200_fx_sample( flan_b200_ctx * ctx, const flan_b200_fx_program * prog, int64_t frames, int bins,
+                         float time_step, float bin_width, float * d_out, int64_t * frame_stride, int * bin_stride );
+/* The program at every MF, as PV::modify_frequency evaluates its mod (PVModify.cpp:263-268): d_out[c][x][b] =
+ * program( float( x ) / frame_rate, d_pv[c][x][b].f ) with frame_rate = float( sample_rate ) / float( hop )
+ * (PVBuffer::frame_to_time). d_out: float[C][F][B], the d_in_mod of flan_b200_modify_frequency. */
+int flan_b200_fx_at_pv( flan_b200_ctx * ctx, const flan_b200_fx_program * prog, const float * d_pv, int channels,
+                        int64_t frames, int bins, float frame_rate, float * d_out );
 
 /* ---- file formats either side of the path (SURVEY 8f-4) ---------------------------------------------------------
  * .flan RIFF-PV (PVBuffer::save / load, src/flan/PV/PVBuffer.cpp:99-140, 216-273; format described at
