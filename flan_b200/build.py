@@ -83,7 +83,8 @@ def build_emulator(force=False):
     os.makedirs(LIB, exist_ok=True)
     src = os.path.join(CSRC, "emu", "pv_emu.cpp")
     src_modify = os.path.join(CSRC, "emu", "pv_modify_emu.cpp")
-    deps = [src, src_modify] + _sources("pv_core.cuh", "pv_body.cuh", "pv_tables.h", "pv_modify_body.cuh")
+    deps = [src, src_modify] + _sources("pv_core.cuh", "pv_body.cuh", "pv_tables.h", "pv_modify_body.cuh", "pv_policy.h", "pv_kernel_list.h",
+                                        "pv_generic.h", "pv_generic_body.cuh")
     if not force and not _newer(emu_path(), deps):
         return emu_path()
     cuda_inc = os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "include")

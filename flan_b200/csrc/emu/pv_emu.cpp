@@ -8,6 +8,8 @@
 #include "../pv_body.cuh"
 #include "../pv_tables.h"
 #include "../pv_generic.h"
+#include "../pv_kernel_list.h"
+#include "../pv_policy.h"
 
 #include <atomic>
 #include <cmath>
@@ -16,6 +18,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <memory>
+#include <string>
 #include <thread>
 #include <vector>
 
@@ -116,16 +119,16 @@ template<int N, int PT, class Body> void run_cta( Body && body )
 	for( auto & x : th ) x.join();
 	}
 
-template<int N, int PT> void analysis_n( const AnalysisArgs & a, int64_t blocks )
+// The instantiation k names (PAD and EMIT as the launch policy, pv_policy.h, decides them).
+template<int N, int PT> void analysis_n( const TransformKernel & k, const AnalysisArgs & a, int64_t blocks )
 	{
 	for( int64_t b = 0; b < blocks; ++b )
 		{
-		if( a.one_buffer && PT == 16 )
+		if( k.ONE )
 			{
-			// the product's choice: zero-padded windows of whole slots take the vector-load instantiation
-			if( a.W < N && a.W % ( N / PT ) == 0 && a.aligned2 )
+			if( k.PAD )
 				run_cta<N, PT>( [&]( HostEnv & env, float *, float2 * x0, float2 * x1, float2 * ) { analysis_cta<N, PT, true, true>( a, b, env, x0, x0 ); } );
-			else if( a.seg_out )      // the instantiation that also leaves the phase summaries (ring: N floats = room for the N/2 + 1 ints)
+			else if( k.EMIT )      // the instantiation that also leaves the phase summaries (ring: N floats = room for the N/2 + 1 ints)
 				run_cta<N, PT>( [&]( HostEnv & env, float * ring, float2 * x0, float2 * x1, float2 * ) { analysis_cta<N, PT, true, false, true>( a, b, env, x0, x0, (int *) ring ); } );
 			else
 				run_cta<N, PT>( [&]( HostEnv & env, float *, float2 * x0, float2 * x1, float2 * ) { analysis_cta<N, PT, true, false>( a, b, env, x0, x0 ); } );
@@ -153,7 +156,7 @@ template<int N> void synthesis_mirror_n( const SynthArgs & a, int64_t blocks )
 	for( int64_t b = 0; b < blocks; ++b )
 		run_cta<N, 16>( [&]( HostEnv & env, float * ola, float2 * x0, float2 * x1, float2 * rowbuf )
 			{
-			const bool gen = !( a.W == N && a.hop == N / 16 );
+			const bool gen = !standard_shape( N, a.W, a.hop );
 			if( gen ) { if( a.one_buffer ) synthesis_cta_mirror<N, true, true>( a, b, env, (float2 *) ola, x0, x0, rowbuf, &bar_word ); else synthesis_cta_mirror<N, false, true>( a, b, env, (float2 *) ola, x0, x1, rowbuf, &bar_word ); }
 			else if( a.one_buffer ) synthesis_cta_mirror<N, true, false>( a, b, env, (float2 *) ola, x0, x0, rowbuf, &bar_word );
 			else synthesis_cta_mirror<N, false, false>( a, b, env, (float2 *) ola, x0, x1, rowbuf, &bar_word );
@@ -213,7 +216,11 @@ int pv_emu_analysis( const float * audio, int64_t audio_stride, int64_t audio_of
 	a.one_buffer = one_buffer;
 	a.k = tb.k;
 	a.seg_out = seg_out; a.P = tb.P; a.rcpP = tb.rcpP;
-	if( seg_out && !( pt16 && one_buffer && W == N && points_per_thread == 16 ) ) return 5;
+	TransformKernel k;
+	k.kind = KernelKind::analysis; k.N = N; k.PT = pt16 ? 16 : 8; k.TPS = pt16 ? 512 : 768; k.ONE = pt16 && one_buffer;
+	k.PAD = analysis_pad_fits( k, W, a.aligned2 );
+	k.EMIT = seg_out != nullptr;
+	if( k.EMIT && ( points_per_thread != 16 || !analysis_emit_fits( k, W ) ) ) return 5;
 	const int64_t blocks = (int64_t) C * segs;
 	if( !dft_size_is_templated( N ) )
 		{
@@ -229,9 +236,9 @@ int pv_emu_analysis( const float * audio, int64_t audio_stride, int64_t audio_of
 			} );
 		return 0;
 		}
-	if( points_per_thread == 17 )       // PV_PT_MIRROR
+	if( points_per_thread == 17 )       // the mirrored last pass
 		{
-		if( !( W == N && hop == N / 16 ) ) return 3;
+		if( !analysis_mirror_fits( N, W, hop ) ) return 3;
 		a.pass_tw = tb.pass_tw16.data();
 		switch( N )
 			{
@@ -243,12 +250,12 @@ int pv_emu_analysis( const float * audio, int64_t audio_stride, int64_t audio_of
 		}
 	switch( N )
 		{
-		case 256: analysis_n<256, 8>( a, blocks ); break;
-		case 512: if( pt16 ) analysis_n<512, 16>( a, blocks ); else analysis_n<512, 8>( a, blocks ); break;
-		case 1024: if( pt16 ) analysis_n<1024, 16>( a, blocks ); else analysis_n<1024, 8>( a, blocks ); break;
-		case 2048: if( pt16 ) analysis_n<2048, 16>( a, blocks ); else analysis_n<2048, 8>( a, blocks ); break;
-		case 4096: if( pt16 ) analysis_n<4096, 16>( a, blocks ); else analysis_n<4096, 8>( a, blocks ); break;
-		case 8192: if( pt16 ) analysis_n<8192, 16>( a, blocks ); else analysis_n<8192, 8>( a, blocks ); break;
+		case 256: analysis_n<256, 8>( k, a, blocks ); break;
+		case 512: if( pt16 ) analysis_n<512, 16>( k, a, blocks ); else analysis_n<512, 8>( k, a, blocks ); break;
+		case 1024: if( pt16 ) analysis_n<1024, 16>( k, a, blocks ); else analysis_n<1024, 8>( k, a, blocks ); break;
+		case 2048: if( pt16 ) analysis_n<2048, 16>( k, a, blocks ); else analysis_n<2048, 8>( k, a, blocks ); break;
+		case 4096: if( pt16 ) analysis_n<4096, 16>( k, a, blocks ); else analysis_n<4096, 8>( k, a, blocks ); break;
+		case 8192: if( pt16 ) analysis_n<8192, 16>( k, a, blocks ); else analysis_n<8192, 8>( k, a, blocks ); break;
 		default: return 2;
 		}
 	return 0;
@@ -325,9 +332,9 @@ int pv_emu_synthesis( const float * pv_rows, int64_t pv_channel_stride, int C, i
 			} );
 		return 0;
 		}
-	if( variant == 17 )     // PV_PT_MIRROR: the standard shape, or the general form for any aligned window and even hop
+	if( variant == 17 )     // mirrored: the standard shape, or the general form for any aligned window and even hop
 		{
-		if( !( W >= N / 16 && W % ( N / 16 ) == 0 && hop >= 2 && hop % 2 == 0 && hop <= W && hop <= N / 16 ) ) return 3;
+		if( !synthesis_mirror_fits( N, W, hop ) ) return 3;
 		switch( N )
 			{
 			case 1024: synthesis_mirror_n<1024>( a, blocks ); return 0;
@@ -368,6 +375,44 @@ int pv_emu_phase_segments( const float * pv_rows, int C, int64_t frames, int B, 
 				}
 	if( nan_flag ) *nan_flag = flag;
 	return 0;
+	}
+
+// The launch policy (pv_policy.h), for tests/test_launch_policy.py: the name of the kernel choose_analysis /
+// choose_synthesis return is written to out (cap bytes); returns its length, or -1 when it does not fit.
+static int put_name( const std::string & s, char * out, int cap )
+	{
+	if( (int) s.size() >= cap ) return -1;
+	std::memcpy( out, s.c_str(), s.size() + 1 );
+	return (int) s.size();
+	}
+int pv_emu_choose_analysis( int N, int W, int hop, int C, int64_t signal_frames, int sms, int aligned2, int emit, char * out, int cap )
+	{
+	return put_name( choose_analysis( N, W, hop, C, signal_frames, sms, aligned2 != 0, emit != 0 ).name(), out, cap );
+	}
+int pv_emu_choose_synthesis( int N, int W, int hop, char * out, int cap )
+	{
+	return put_name( choose_synthesis( N, W, hop ).name(), out, cap );
+	}
+// The release kernel list (pv_kernel_list.h), one name per line.
+int pv_emu_release_kernels( char * out, int cap )
+	{
+	std::string s;
+	auto add = [&]( KernelKind kind, int N, int PT, int TPS, bool ONE, bool PAD, bool EMIT, bool GEN )
+		{
+		TransformKernel k;
+		k.kind = kind; k.N = N; k.PT = PT; k.TPS = TPS; k.ONE = ONE; k.PAD = PAD; k.EMIT = EMIT; k.GEN = GEN;
+		s += k.name() + "\n";
+		};
+#define PV_A( N, PT, TPS, ONE, PAD, EMIT ) add( KernelKind::analysis, N, PT, TPS, ONE, PAD, EMIT, false );
+#define PV_AM( N, TPS ) add( KernelKind::analysis_mirror, N, 16, TPS, true, false, false, false );
+#define PV_S( N, TPS, ONE ) add( KernelKind::synthesis, N, 8, TPS, ONE, false, false, false );
+#define PV_SM( N, TPS, ONE, GEN ) add( KernelKind::synthesis_mirror, N, 16, TPS, ONE, false, false, GEN );
+	PV_RELEASE_KERNELS( PV_A, PV_AM, PV_S, PV_SM )
+#undef PV_A
+#undef PV_AM
+#undef PV_S
+#undef PV_SM
+	return put_name( s, out, cap );
 	}
 
 // Frames per CTA as the launch policy chooses them (pv_tables.h), for the whole-wave tests.

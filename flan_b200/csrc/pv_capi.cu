@@ -364,6 +364,64 @@ int copy_d2h_2d( flan_b200_ctx * ctx, void * h, size_t h_pitch, const void * d, 
 
 static int seg_len_cap( const flan_b200_ctx * ctx, int N ) { return ctx->max_seg_len ? ctx->max_seg_len : ( N >= 2048 ? 128 : 64 ); }
 
+// 8-byte loads of the input: hop, half window, stride, offset and address all even
+static bool audio_aligned2( int W, int hop, const float * audio, int64_t stride, int64_t offset )
+	{
+	return hop % 2 == 0 && ( W / 2 ) % 2 == 0 && stride % 2 == 0 && offset % 2 == 0 && (uintptr_t) audio % 8 == 0;
+	}
+
+// The analysis kernel of a call: the launch policy's choice (pv_policy.h), decided on the whole signal's frame count.
+// Development builds apply the overrides of FLAN_B200_PT_ANALYSIS (8, 16 or 17: the mirrored last pass where it fits),
+// FLAN_B200_TPS_ANALYSIS and FLAN_B200_ONEBUF here, snapped to the variants they carry.
+static TransformKernel analysis_kernel( const flan_b200_ctx * ctx, int N, int W, int hop, int C, int64_t n_total, bool aligned2, bool emit )
+	{
+	TransformKernel k = choose_analysis( N, W, hop, C, n_total / hop + 1, ctx->sms, aligned2, emit );
+#ifdef FLAN_B200_DEBUG
+	if( k.kind == KernelKind::generic_analysis ) return k;
+	int pt = ctx->pt_analysis ? ctx->pt_analysis : ( k.kind == KernelKind::analysis_mirror ? 17 : k.PT );
+	if( pt == 17 && !analysis_mirror_fits( N, W, hop ) ) pt = N >= 4096 ? 16 : 8;
+	if( pt != 17 && ( pt != 16 || N < 512 ) ) pt = 8;
+	const int tps = ctx->tps_analysis ? ctx->tps_analysis : ( pt == 8 ? 768 : 512 );
+	k.kind = pt == 17 ? KernelKind::analysis_mirror : KernelKind::analysis;
+	k.PT = pt == 8 ? 8 : 16;
+	k.TPS = pt == 8 ? ( tps >= 1024 ? 1024 : tps < 768 ? 512 : 768 ) : ( tps >= 768 ? 768 : tps >= 640 ? 640 : tps < 512 ? 384 : 512 );
+	k.ONE = pt != 8 && ctx->one_buffer != 0;
+	k.PAD = analysis_pad_fits( k, W, aligned2 );
+	k.EMIT = emit && !k.PAD && analysis_emit_fits( k, W );
+#endif
+	return k;
+	}
+
+// The resynthesis kernel: the launch policy's choice. Development builds apply FLAN_B200_SYNTH_VARIANT (17: mirrored
+// where it fits, anything else the 8-point kernel), FLAN_B200_TPS_SYNTHESIS and FLAN_B200_SYNTH_ONEBUF.
+static TransformKernel synthesis_kernel( const flan_b200_ctx * ctx, int N, int W, int hop )
+	{
+	TransformKernel k = choose_synthesis( N, W, hop );
+#ifdef FLAN_B200_DEBUG
+	if( k.kind == KernelKind::generic_synthesis ) return k;
+	const bool mirror = ( ctx->synth_variant < 0 || ctx->synth_variant == 17 ) && synthesis_mirror_fits( N, W, hop );
+	const bool one = ctx->synth_one_buffer >= 0 ? ctx->synth_one_buffer != 0 : N == 8192;
+	const int tps = ctx->tps_synthesis ? ctx->tps_synthesis : ( mirror ? 384 : ( N == 8192 ? 1024 : 768 ) );
+	k.kind = mirror ? KernelKind::synthesis_mirror : KernelKind::synthesis;
+	k.PT = mirror ? 16 : 8;
+	k.GEN = mirror && !standard_shape( N, W, hop );
+	if( mirror && N == 8192 ) { k.TPS = one ? 512 : 256; k.ONE = one; }
+	else if( mirror && ( tps >= 512 || one ) ) { k.TPS = tps >= 512 ? 512 : 384; k.ONE = one; }
+	else if( mirror ) k = choose_synthesis( N, W, hop );
+	else if( N == 8192 && tps >= 1024 ) { k.TPS = 1024; k.ONE = true; }
+	else { k.TPS = tps >= 1024 ? 1024 : ( tps < 768 ? 512 : 768 ); k.ONE = false; }
+#endif
+	return k;
+	}
+
+// A failed launch or occupancy query of a transform kernel names the kernel. cudaErrorInvalidValue is also what a
+// descriptor outside this build's kernel list gives: an internal error of the launch policy.
+static int transform_fail( flan_b200_ctx * ctx, cudaError_t e, const TransformKernel & k, const char * what )
+	{
+	return cuda_fail( ctx, e, ( std::string( e == cudaErrorInvalidValue ? "internal: " : "" ) + what + " of " + k.name() ).c_str() );
+	}
+#define CK_KERNEL( call, k, what ) do { cudaError_t e_ = ( call ); if( e_ != cudaSuccess ) return transform_fail( ctx, e_, k, what ); } while( 0 )
+
 int analysis_range( flan_b200_ctx * ctx, const AnalysisCall & c )
 	{
 	const int C = c.C, W = c.W, hop = c.hop, N = c.N;
@@ -393,8 +451,7 @@ int analysis_range( flan_b200_ctx * ctx, const AnalysisCall & c )
 	a.frame_begin = c.frame_begin; a.frame_end = c.frame_end;
 	a.seg_len = seg_len; a.segs_per_channel = segs;
 	a.W = W; a.hop = hop;
-	a.aligned2 = ( hop % 2 == 0 ) && ( ( W / 2 ) % 2 == 0 ) && ( c.audio_stride % 2 == 0 ) && ( c.audio_offset % 2 == 0 )
-	          && ( (uintptr_t) c.d_audio_local % 8 == 0 );
+	a.aligned2 = audio_aligned2( W, hop, c.d_audio_local, c.audio_stride, c.audio_offset );
 	a.win = plan->win_analysis; a.binc = plan->binc; a.binc4 = plan->binc4; a.post_rot = plan->post_rot;
 	a.k = plan->host.k;
 	if( plan->generic )
@@ -403,7 +460,6 @@ int analysis_range( flan_b200_ctx * ctx, const AnalysisCall & c )
 		ga.a = a; ga.g = plan->generic_fft;
 		ga.total_segments = (int64_t) C * segs;
 		const GenericGeometry geo = generic_geometry( ga.g, generic_analysis_state_bytes( ga.g ), ga.total_segments, ctx->sms );
-		if( c.wave_out ) { *c.wave_out = (int) geo.blocks; return FLAN_B200_OK; }
 		void * ws = nullptr;
 		rc = get_workspace( ctx, (size_t)( geo.blocks * geo.scratch_stride ), &ws );
 		if( rc ) return rc;
@@ -411,62 +467,38 @@ int analysis_range( flan_b200_ctx * ctx, const AnalysisCall & c )
 		{ LaunchTimer lt( ctx, 0 ); CK( launch_generic_analysis( ga, geo, ctx->compute ), "analysis launch" ); }
 		return FLAN_B200_OK;
 		}
-	// measured on B200 (tools/experiments/exp_r1*.sh): 16 points per thread with one exchange buffer from dft 4096 up; the mirrored
-	// last pass for dft 1024 with the standard window / hop; 8 points per thread otherwise
-	// (dft 2048: 16 points per thread once the grid covers the SMs a few times over -- 2.52 -> 2.31 ms on a cfg4 channel --
-	// 8 for short signals, where twice the threads per frame matter more)
-	// (decided on the WHOLE signal's frame count, so that every frame-range shard of a signal runs the same arithmetic)
-	const bool large = (int64_t) C * ( c.n_total / hop + 1 ) >= (int64_t) ctx->sms * 128;
-	int pt = ( N >= 4096 ? 16 : ( N == 2048 ? ( large ? 16 : 8 ) : ( N == 1024 ? PV_PT_MIRROR : 8 ) ) );
-#ifdef FLAN_B200_DEBUG
-	if( ctx->pt_analysis ) pt = ctx->pt_analysis;
-#endif
-	if( pt == PV_PT_MIRROR && !( mirror_supported( N ) && W == N && hop == N / 16 ) ) pt = ( N >= 4096 ) ? 16 : 8;
-	if( pt != PV_PT_MIRROR && ( pt != 16 || N < 512 ) ) pt = 8;
-	int tps_a = ( pt >= 16 ? 512 : 768 );
-	a.one_buffer = ( pt == 16 || pt == PV_PT_MIRROR ) ? 1 : 0;
-#ifdef FLAN_B200_DEBUG
-	if( ctx->tps_analysis ) tps_a = ctx->tps_analysis;
-	if( ctx->one_buffer >= 0 ) a.one_buffer = ctx->one_buffer;
-#endif
-	a.pass_tw = ( pt >= 16 ) ? plan->pass_tw16 : plan->pass_tw;
-	if( c.wave_out )
+	// Summaries for a resynthesis of these rows as they are (flan_b200_hint_resynthesis): the kernel that can leave them
+	// writes them to the workspace, in the segments resynthesis will use, when the scan that repairs marked entries (three
+	// launches) will read them; anything else ignores the hint. (A frame range without emit_seg_len is a shard of a
+	// per-GPU process: its resynthesis chooses the segments from the local frame count, and so does this.)
+	const int B = N / 2 + 1;
+	PhaseLayout lay{};
+	if( c.emit_summary && c.pv_channel_stride == frames * (int64_t) B ) lay = phase_layout( ctx, C, frames, B, W, hop, c.emit_seg_len );
+	const TransformKernel k = analysis_kernel( ctx, N, W, hop, C, c.n_total, a.aligned2, lay.segs > 256 && lay.seg_len <= 128 );
+	a.one_buffer = k.ONE;
+	a.pass_tw = k.PT == 16 ? plan->pass_tw16 : plan->pass_tw;
+	if( k.EMIT )
 		{
-		CK( launch_analysis( N, a, -1, ctx->compute, tps_a, pt ), "occupancy query" );
-		*c.wave_out = ctx->sms * std::max( 1, last_occupancy() );
+		void * ws = nullptr;
+		rc = get_workspace( ctx, lay.bytes(), &ws );
+		if( rc ) return rc;
+		seg_len = lay.seg_len; segs = lay.segs;
+		a.seg_len = seg_len; a.segs_per_channel = segs;
+		a.seg_out = (PhaseSeg *) ws; a.P = plan->host.P; a.rcpP = plan->host.rcpP;
+		CK( cudaMemsetAsync( ctx->summaries.nan_flag, 0, sizeof( int ), ctx->compute ), "flag clear" );
+		{ LaunchTimer lt( ctx, 0 ); CK_KERNEL( launch( k, a, (int64_t) C * segs, ctx->compute ), k, "analysis launch" ); }
+		ctx->summaries.publish( { c.d_pv_rows, c.pv_channel_stride, c.frame_begin, c.frame_end, C, B, W, seg_len, c.sr, flan_b200_analysis_rate( c.sr, hop ) },
+		                        { /* needs_fix */ true, /* nan_known */ true } );
 		return FLAN_B200_OK;
-		}
-	// Summaries for a resynthesis of these rows as they are (flan_b200_hint_resynthesis): the 16-point full-window kernel
-	// leaves them in the workspace, in the segments resynthesis will use; anything else ignores the hint.
-	// (a frame range without emit_seg_len is a shard of a per-GPU process: its resynthesis chooses the segments from the
-	// local frame count, and so does this)
-	if( c.emit_summary && pt == 16 && a.one_buffer && tps_a == 512 && N >= 2048 && W == N
-	    && c.pv_channel_stride == frames * (int64_t)( N / 2 + 1 ) )
-		{
-		const int B = N / 2 + 1;
-		const PhaseLayout lay = phase_layout( ctx, C, frames, B, W, hop, c.emit_seg_len );
-		if( lay.segs > 256 && lay.seg_len <= 128 )           // the three-launch scan is the one that repairs marked entries
-			{
-			void * ws = nullptr;
-			rc = get_workspace( ctx, lay.bytes(), &ws );
-			if( rc ) return rc;
-			seg_len = lay.seg_len; segs = lay.segs;
-			a.seg_len = seg_len; a.segs_per_channel = segs;
-			a.seg_out = (PhaseSeg *) ws; a.P = plan->host.P; a.rcpP = plan->host.rcpP;
-			CK( cudaMemsetAsync( ctx->summaries.nan_flag, 0, sizeof( int ), ctx->compute ), "flag clear" );
-			{ LaunchTimer lt( ctx, 0 ); CK( launch_analysis( N, a, (int64_t) C * segs, ctx->compute, tps_a, pt ), "analysis launch" ); }
-			ctx->summaries.publish( { c.d_pv_rows, c.pv_channel_stride, c.frame_begin, c.frame_end, C, B, W, seg_len, c.sr, flan_b200_analysis_rate( c.sr, hop ) },
-			                        { /* needs_fix */ true, /* nan_known */ true } );
-			return FLAN_B200_OK;
-			}
 		}
 	// Whole waves: with a few waves of CTAs the last, partly filled one is a large share of the launch (a 1/8 shard of cfg3:
 	// 660 CTAs = 2.23 waves of 296). Segments are shortened until the CTAs just fill the waves they need anyway. Analysis
 	// results do not depend on where segments are cut (the warm-up frame recomputes the previous phase exactly).
 	if( (int64_t) C * segs > 2 * (int64_t) ctx->sms )
 		{
-		CK( launch_analysis( N, a, -1, ctx->compute, tps_a, pt ), "occupancy query" );
-		const int64_t wave = (int64_t) ctx->sms * std::max( 1, last_occupancy() );
+		int per_sm = 0;
+		CK_KERNEL( resident_ctas( k, a, &per_sm ), k, "occupancy query" );
+		const int64_t wave = (int64_t) ctx->sms * std::max( 1, per_sm );
 		const int64_t ctas = (int64_t) C * segs;
 		const int64_t per_channel = ( ( ctas + wave - 1 ) / wave * wave ) / C;
 		const int64_t shorter = per_channel > 0 ? ( frames + per_channel - 1 ) / per_channel : seg_len;
@@ -477,7 +509,7 @@ int analysis_range( flan_b200_ctx * ctx, const AnalysisCall & c )
 			}
 		}
 	ctx->summaries.drop();          // new rows, no summaries of them
-	{ LaunchTimer lt( ctx, 0 ); CK( launch_analysis( N, a, (int64_t) C * segs, ctx->compute, tps_a, pt ), "analysis launch" ); }
+	{ LaunchTimer lt( ctx, 0 ); CK_KERNEL( launch( k, a, (int64_t) C * segs, ctx->compute ), k, "analysis launch" ); }
 	return FLAN_B200_OK;
 	}
 
@@ -642,16 +674,9 @@ int synth_range( flan_b200_ctx * ctx, const SynthCall & s )
 	a.win = plan->win_synthesis; a.post_tw = plan->post_tw; a.pass_tw = plan->pass_tw; a.pass_tw_rev = plan->pass_tw_rev;
 	a.out_aligned2 = ( s.out_stride % 2 == 0 ) && ( s.out_offset % 2 == 0 ) && ( (uintptr_t) s.d_out % 8 == 0 );
 	a.pv_aligned16 = ( (uintptr_t) s.d_pv_rows % 16 == 0 ); a.channels = C;
-	a.one_buffer = ( N == 8192 ? 1 : 0 );                                // dft 8192: two 256-thread CTAs per SM
 	a.k = plan->host.k; a.P = plan->host.P; a.rcpP = plan->host.rcpP;
-	int variant = PV_PT_MIRROR;
-	int tps_mirror = 384, tps_plain = ( N == 8192 ) ? 1024 : 768;
-#ifdef FLAN_B200_DEBUG
-	if( ctx->synth_one_buffer >= 0 ) a.one_buffer = ctx->synth_one_buffer;
-	if( ctx->synth_variant >= 0 ) variant = ctx->synth_variant;
-	if( ctx->tps_synthesis ) tps_mirror = tps_plain = ctx->tps_synthesis;
-#endif
-	const bool mirror = variant == PV_PT_MIRROR && synthesis_mirror_applies( N, a );
+	const TransformKernel kernel = synthesis_kernel( ctx, N, W, hop );
+	a.one_buffer = kernel.ONE;
 	// One launch, or -- for the pipelined host forms -- slices of whole waves of CTAs so that a download can follow each.
 	int segs_per_slice = segs;
 	if( s.on_chunk && s.head_segments <= 0 )
@@ -660,8 +685,9 @@ int synth_range( flan_b200_ctx * ctx, const SynthCall & s )
 		if( plan->generic ) wave = geo.blocks;
 		else
 			{
-			CK( launch_synthesis( N, a, -1, ctx->compute, mirror ? tps_mirror : tps_plain, variant ), "occupancy query" );
-			wave = (int64_t) ctx->sms * std::max( 1, last_occupancy() );
+			int per_sm = 0;
+			CK_KERNEL( resident_ctas( kernel, a, &per_sm ), kernel, "occupancy query" );
+			wave = (int64_t) ctx->sms * std::max( 1, per_sm );
 			}
 		segs_per_slice = (int) std::max<int64_t>( 1, ctas_per_slice( (int64_t) C * segs, wave, s.copy_bytes ) / C );
 		}
@@ -671,7 +697,7 @@ int synth_range( flan_b200_ctx * ctx, const SynthCall & s )
 		std::unique_ptr<LaunchTimer> lt;
 		if( timed ) lt.reset( new LaunchTimer( ctx, 3 ) ); else ctx->launches++;
 		if( plan->generic ) { ga.a = a; CK( launch_generic_synthesis( ga, geo, st ), "synthesis launch" ); }
-		else CK( launch_synthesis( N, a, (int64_t) C * ( s1 - s0 ), st, mirror ? tps_mirror : tps_plain, variant ), "synthesis launch" );
+		else CK_KERNEL( launch( kernel, a, (int64_t) C * ( s1 - s0 ), st ), kernel, "synthesis launch" );
 		return FLAN_B200_OK;
 		};
 	if( s.head_segments > 0 && !plan->generic )
@@ -1226,14 +1252,22 @@ int flan_b200_convert_to_pv_h2d( flan_b200_ctx * ctx, const float * h_audio, flo
 	int rc = get_plan( ctx, N, W, hop, sr, flan_b200_analysis_rate( sr, hop ), &plan );     // argument errors before any copy
 	if( rc ) return rc;
 	// slices of whole waves of the analysis kernel's CTAs (a partial wave at the end of every slice would be paid each time)
-	int wave = ctx->sms;
-		{
-		AnalysisCall q{ d_audio, n, 0, n, C, n, sr, W, hop, N, 0, F, d_pv, F * (int64_t) B };
-		q.wave_out = &wave;
-		rc = analysis_range( ctx, q );
-		if( rc ) return rc;
-		}
 	const int cap = seg_len_cap( ctx, N );
+	int64_t wave = ctx->sms;
+	if( plan->generic )
+		{
+		const int seg_len = choose_seg_len( F, C, ctx->sms, W, hop, cap, true );
+		wave = generic_geometry( plan->generic_fft, generic_analysis_state_bytes( plan->generic_fft ), ( F + seg_len - 1 ) / seg_len * C, ctx->sms ).blocks;
+		}
+	else
+		{
+		const TransformKernel k = analysis_kernel( ctx, N, W, hop, C, n, audio_aligned2( W, hop, d_audio, n, 0 ), false );
+		AnalysisArgs q{};
+		q.one_buffer = k.ONE;
+		int per_sm = 0;
+		CK_KERNEL( resident_ctas( k, q, &per_sm ), k, "occupancy query" );
+		wave = (int64_t) ctx->sms * std::max( 1, per_sm );
+		}
 	const int64_t ctas = ( F + cap - 1 ) / cap * C;
 	const int64_t frames_per_slice = std::max<int64_t>( 1, ctas_per_slice( ctas, wave, sizeof( float ) * (size_t) C * n ) / C ) * cap;
 	const int slices = (int)( ( F + frames_per_slice - 1 ) / frames_per_slice );

@@ -166,7 +166,8 @@ struct flan_b200_ctx
 	pvrt::PhaseSummaries summaries;         // the phase summaries held in the workspace, and which rows they describe
 	int max_seg_len = 0;                   // frames per CTA at most; 0 = by size (FLAN_B200_DEBUG builds: FLAN_B200_SEG_LEN)
 #ifdef FLAN_B200_DEBUG
-	// experiment knobs of development builds only (tools/experiments); release builds carry the measured policy
+	// experiment knobs of development builds only (tools/experiments; pv_capi.cu: analysis_kernel / synthesis_kernel);
+	// release builds carry the measured policy
 	int tps_analysis = 0, pt_analysis = 0, one_buffer = -1, synth_variant = -1, tps_synthesis = 0, synth_one_buffer = -1;
 #endif
 	struct Timed { int kind; cudaEvent_t start, stop; };
@@ -310,7 +311,6 @@ struct AnalysisCall
 	float sr; int W, hop, N;
 	int64_t frame_begin, frame_end;
 	float * d_pv_rows; int64_t pv_channel_stride;
-	int * wave_out = nullptr;       // query only: CTAs of one full wave of the kernel this call would launch; nothing is launched
 	bool emit_summary = false;      // the rows will be resynthesised unchanged: also leave their phase summaries
 	int emit_seg_len = 0;           // frame-range shards: the segment length of the WHOLE signal (0: this call is the whole signal)
 	};

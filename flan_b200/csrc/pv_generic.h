@@ -7,11 +7,10 @@
 #include <vector>
 
 #include "pv_generic_body.cuh"
+#include "pv_policy.h"
 
 namespace pvk {
 
-// Sizes served by the templated kernels of pv_body.cuh; everything else takes the generic path.
-inline bool dft_size_is_templated( int N ) { return N == 256 || N == 512 || N == 1024 || N == 2048 || N == 4096 || N == 8192; }
 // Largest dft size accepted (scratch per CTA grows with it: 16 bytes x 2 x the FFT length).
 constexpr int GENERIC_MAX_DFT = 1 << 20;
 

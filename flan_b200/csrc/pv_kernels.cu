@@ -10,10 +10,13 @@
 // device Env (barrier, cp.async staging, cache-hinted loads/stores, red.add) and the launch geometry.
 #include "pv_body.cuh"
 #include "pv_launch.h"
+#include "pv_kernel_list.h"
 
 #include <cuda_runtime.h>
 
 #include <cstdlib>
+#include <type_traits>
+#include <vector>
 
 namespace pvk {
 
@@ -459,14 +462,15 @@ __global__ void __launch_bounds__( 256 ) pv_add_kernel( float * out, const float
 // launchers
 // ------------------------------------------------------------------------------------------------
 // Development aids (FLAN_B200_DEBUG builds only): FLAN_B200_SMEM_PAD=<bytes> inflates the dynamic shared memory request
-// so that fewer CTAs fit per SM; FLAN_B200_CARVEOUT=<percent> sets the preferred shared-memory carveout of the transforms.
+// so that fewer CTAs fit per SM; FLAN_B200_CARVEOUT=<percent> sets the preferred shared-memory carveout of the transforms
+// (the 8-point resynthesis excepted).
 #ifdef FLAN_B200_DEBUG
 static int carveout()
 	{
 	static const int v = [] { const char * e = std::getenv( "FLAN_B200_CARVEOUT" ); return e ? std::atoi( e ) : -1; }();
 	return v;
 	}
-template<class K> static void apply_carveout( K kernel )
+static void apply_carveout( const void * kernel )
 	{
 	if( carveout() >= 0 ) cudaFuncSetAttribute( kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carveout() );
 	}
@@ -476,19 +480,9 @@ static size_t smem_pad()
 	return pad;
 	}
 #else
-template<class K> static void apply_carveout( K ) {}
+static void apply_carveout( const void * ) {}
 static constexpr size_t smem_pad() { return 0; }
 #endif
-
-// blocks < 0 asks the launchers for the kernel's resident CTAs per SM instead of a launch (the pipelined host forms cut a
-// signal into slices of whole waves); the answer is left here.
-static thread_local int g_occupancy = 0;
-template<class K> static cudaError_t report_occupancy( K kernel, int threads, size_t smem )
-	{
-	g_occupancy = 0;
-	return cudaOccupancyMaxActiveBlocksPerMultiprocessor( &g_occupancy, kernel, threads, smem );
-	}
-int last_occupancy() { return g_occupancy; }
 
 // CTAs per SM of a kernel that allocates COLS columns of tensor memory. The driver's occupancy query answers 1 for such
 // kernels (measured on a B200, tools/micro/tmem.cu: query 1, 4 resident), so the bound is taken from the register file
@@ -509,211 +503,154 @@ template<auto KERNEL, int THREADS, int COLS> static cudaError_t tmem_kernel_ctas
 	*ctas = n;
 	return r;
 	}
-template<int N, int PT, int TPS, bool ONE, bool PAD, bool EMIT> static cudaError_t launch_analysis_kernel( const AnalysisArgs & a, int64_t blocks, size_t smem, cudaStream_t st )
+
+// One instantiation of a transform kernel: its descriptor, entry point, threads per CTA, the bytes of one exchange
+// buffer, and for the kernels that allocate tensor memory the CTAs per SM that allocation admits.
+struct KernelEntry
 	{
-	auto kernel = pv_analysis_kernel<N, PT, TPS, ONE, PAD, EMIT>;
-	cudaError_t e = cudaFuncSetAttribute( kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem );
-	if( e != cudaSuccess ) return e;
-	apply_carveout( kernel );
-	if constexpr( analysis_uses_tmem<N, PT, TPS>() )
-		{
-		int ctas = 0;
-		e = tmem_kernel_ctas<pv_analysis_kernel<N, PT, TPS, ONE, PAD, EMIT>, N / ( 2 * PT ), AN_TM_COLS>( &ctas );
-		if( e != cudaSuccess ) return e;
-		if( blocks < 0 ) { g_occupancy = ctas; return cudaSuccess; }
-		}
-	if( blocks < 0 ) return report_occupancy( kernel, N / ( 2 * PT ), smem );
-	kernel<<<(unsigned) blocks, N / ( 2 * PT ), smem, st>>>( a );
-	return cudaGetLastError();
+	TransformKernel k;
+	const void * fn;
+	int threads;
+	size_t xbuf;
+	cudaError_t ( *tmem_ctas )( int * );
+	};
+
+template<int N, int PT, int TPS, bool ONE, bool PAD, bool EMIT> static KernelEntry analysis_entry()
+	{
+	constexpr auto fn = pv_analysis_kernel<N, PT, TPS, ONE, PAD, EMIT>;
+	return { { KernelKind::analysis, N, PT, TPS, ONE, PAD, EMIT, false }, (const void *) fn, N / ( 2 * PT ), sizeof( float2 ) * XBuf<N / 2>::size,
+	         analysis_uses_tmem<N, PT, TPS>() ? &tmem_kernel_ctas<fn, N / ( 2 * PT ), AN_TM_COLS> : nullptr };
 	}
-template<int N, int PT, int TPS, bool ONE> static cudaError_t launch_analysis_nto( const AnalysisArgs & a, int64_t blocks, cudaStream_t st )
+template<int N, int TPS> static KernelEntry analysis_mirror_entry()
 	{
-	const size_t smem = ( ONE ? 1 : 2 ) * sizeof( float2 ) * XBuf<N / 2>::size + smem_pad();
-	// zero-padded windows that fill whole slots (the API default shape): vector loads, 16 points per thread form only
-	if constexpr( PT == 16 && ONE )
-		{
-		if( a.W < N && a.W % ( N / PT ) == 0 && a.aligned2 ) return launch_analysis_kernel<N, PT, TPS, ONE, true, false>( a, blocks, smem, st );
-		}
-	// the full-window launch that also leaves the phase summaries of its rows (16 points per thread, one buffer, TPS 512: the
-	// policy's variant from dft 2048 up)
-	if constexpr( PT == 16 && ONE && TPS == 512 && N >= 2048 )
-		{
-		if( a.seg_out ) return launch_analysis_kernel<N, PT, TPS, ONE, false, true>( a, blocks, smem + sizeof( int ) * ( N / 2 + 4 ), st );
-		}
-	if( a.seg_out ) return cudaErrorInvalidValue;          // the caller asks for summaries only where this form exists
-	return launch_analysis_kernel<N, PT, TPS, ONE, false, false>( a, blocks, smem, st );
+	return { { KernelKind::analysis_mirror, N, 16, TPS, true, false, false, false }, (const void *) pv_analysis_mirror_kernel<N, TPS>, N / 32,
+	         sizeof( float2 ) * XBuf<N / 2>::size, nullptr };
 	}
-// the one-buffer form is built for 16 points per thread only (the variant the large transforms use)
-template<int N, int PT, int TPS> static cudaError_t launch_analysis_nt( const AnalysisArgs & a, int64_t blocks, cudaStream_t st )
+template<int N, int TPS, bool ONE> static KernelEntry synthesis_entry()
 	{
+	return { { KernelKind::synthesis, N, 8, TPS, ONE, false, false, false }, (const void *) pv_synthesis_kernel<N, TPS, ONE>, N / 16,
+	         sizeof( float2 ) * XBuf<N / 2>::size, nullptr };
+	}
+template<int N, int TPS, bool ONE, bool GEN> static KernelEntry synthesis_mirror_entry()
+	{
+	constexpr auto fn = pv_synthesis_mirror_kernel<N, TPS, ONE, GEN>;
+	return { { KernelKind::synthesis_mirror, N, 16, TPS, ONE, false, false, GEN }, (const void *) fn, N / 32, sizeof( float2 ) * XBuf<N / 2>::size,
+	         synthesis_uses_tmem<N, TPS, GEN>() ? &tmem_kernel_ctas<fn, N / 32, SY_TM_COLS> : nullptr };
+	}
+
 #ifdef FLAN_B200_DEBUG
-	if constexpr( PT == 16 ) { if( a.one_buffer ) return launch_analysis_nto<N, PT, TPS, true>( a, blocks, st ); }
-	return launch_analysis_nto<N, PT, TPS, false>( a, blocks, st );
-#else
-	return launch_analysis_nto<N, PT, TPS, PT == 16>( a, blocks, st );      // the policy: one buffer exactly when 16 points per thread
-#endif
-	}
-bool analysis_mirror_applies( int N, const AnalysisArgs & a )
+// Development builds also carry the register and buffer variants the FLAN_B200_* knobs reach (pv_capi.cu: the knobs of
+// analysis_kernel / synthesis_kernel), for the experiments under tools/experiments.
+template<int... V, class F> static void each( F && f ) { ( f( std::integral_constant<int, V>() ), ... ); }
+template<int N> static void add_variants( std::vector<KernelEntry> & v )
 	{
-	return mirror_supported( N ) && a.W == N && a.hop == N / 16;
-	}
-template<int N, int TPS> static cudaError_t launch_analysis_mirror_nt( const AnalysisArgs & a, int64_t blocks, cudaStream_t st )
-	{
-	const size_t smem = ( a.one_buffer ? 1 : 2 ) * sizeof( float2 ) * XBuf<N / 2>::size + sizeof( float2 ) * ( N / 2 + 16 ) + smem_pad();
-	cudaError_t e = cudaFuncSetAttribute( pv_analysis_mirror_kernel<N, TPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem );
-	if( e != cudaSuccess ) return e;
-	apply_carveout( pv_analysis_mirror_kernel<N, TPS> );
-	if( blocks < 0 ) return report_occupancy( pv_analysis_mirror_kernel<N, TPS>, N / 32, smem );
-	pv_analysis_mirror_kernel<N, TPS><<<(unsigned) blocks, N / 32, smem, st>>>( a );
-	return cudaGetLastError();
-	}
-// Release builds instantiate only what the launch policy (pv_capi.cu: analysis_range) selects -- 8 points per thread at
-// 85 registers, 16 points per thread / mirrored at 128 registers; FLAN_B200_DEBUG builds carry every register variant
-// for the experiments under tools/experiments.
-template<int N> static cudaError_t launch_analysis_n( const AnalysisArgs & a, int64_t blocks, cudaStream_t st, int tps, int pt )
-	{
-	if constexpr( N == 1024 || N == 2048 || N == 4096 )
+	each<512, 768, 1024>( [&]( auto tps )
 		{
-		if( pt == PV_PT_MIRROR && analysis_mirror_applies( N, a ) )
-			{
-#ifdef FLAN_B200_DEBUG
-			if( tps >= 768 ) return launch_analysis_mirror_nt<N, 768>( a, blocks, st );
-			if( tps >= 640 ) return launch_analysis_mirror_nt<N, 640>( a, blocks, st );
-			if( tps < 512 ) return launch_analysis_mirror_nt<N, 384>( a, blocks, st );
-#endif
-			return launch_analysis_mirror_nt<N, 512>( a, blocks, st );
-			}
-		}
-#ifdef FLAN_B200_DEBUG
+		v.push_back( analysis_entry<N, 8, decltype( tps )::value, false, false, false>() );
+		v.push_back( synthesis_entry<N, decltype( tps )::value, false>() );
+		} );
 	if constexpr( N >= 512 )
-#else
-	if constexpr( N >= 2048 )       // the policy asks for 16 points per thread from dft 2048 up only
-#endif
-		{
-		if( pt == 16 )
+		each<384, 512, 640, 768>( [&]( auto tps )
 			{
-#ifdef FLAN_B200_DEBUG
-			if( tps >= 768 ) return launch_analysis_nt<N, 16, 768>( a, blocks, st );
-			if( tps >= 640 ) return launch_analysis_nt<N, 16, 640>( a, blocks, st );
-			if( tps < 512 ) return launch_analysis_nt<N, 16, 384>( a, blocks, st );
-#endif
-			return launch_analysis_nt<N, 16, 512>( a, blocks, st );
-			}
-		}
-#ifdef FLAN_B200_DEBUG
-	if( tps >= 1024 ) return launch_analysis_nt<N, 8, 1024>( a, blocks, st );
-	if( tps < 768 ) return launch_analysis_nt<N, 8, 512>( a, blocks, st );
-#endif
-	return launch_analysis_nt<N, 8, 768>( a, blocks, st );
+			constexpr int TPS = decltype( tps )::value;
+			v.push_back( analysis_entry<N, 16, TPS, false, false, false>() );
+			v.push_back( analysis_entry<N, 16, TPS, true, false, false>() );
+			v.push_back( analysis_entry<N, 16, TPS, true, true, false>() );
+			if constexpr( N >= 1024 && N <= 4096 ) v.push_back( analysis_mirror_entry<N, TPS>() );
+			} );
+	if constexpr( N >= 1024 && N <= 4096 )
+		each<384, 512>( [&]( auto tps )
+			{
+			constexpr int TPS = decltype( tps )::value;
+			v.push_back( synthesis_mirror_entry<N, TPS, false, false>() ); v.push_back( synthesis_mirror_entry<N, TPS, false, true>() );
+			v.push_back( synthesis_mirror_entry<N, TPS, true, false>() ); v.push_back( synthesis_mirror_entry<N, TPS, true, true>() );
+			} );
+	if constexpr( N == 8192 ) { v.push_back( synthesis_mirror_entry<N, 256, false, false>() ); v.push_back( synthesis_mirror_entry<N, 256, false, true>() ); }
 	}
-template<int N, int TPS, bool ONE> static cudaError_t launch_synthesis_nt( const SynthArgs & a, int64_t blocks, cudaStream_t st )
+#endif
+
+// The instantiations of this build: pv_kernel_list.h (development builds: and their variants).
+static const std::vector<KernelEntry> & kernels()
 	{
-	const size_t smem = sizeof( float ) * N + ( ONE ? 1 : 2 ) * sizeof( float2 ) * XBuf<N / 2>::size + sizeof( float2 ) * ( N / 2 + 2 ) + smem_pad();
-	cudaError_t e = cudaFuncSetAttribute( pv_synthesis_kernel<N, TPS, ONE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem );
-	if( e != cudaSuccess ) return e;
-	if( blocks < 0 ) return report_occupancy( pv_synthesis_kernel<N, TPS, ONE>, N / 16, smem );
-	pv_synthesis_kernel<N, TPS, ONE><<<(unsigned) blocks, N / 16, smem, st>>>( a );
+	static const std::vector<KernelEntry> list = []
+		{
+#define PV_A( N, PT, TPS, ONE, PAD, EMIT ) analysis_entry<N, PT, TPS, ONE, PAD, EMIT>(),
+#define PV_AM( N, TPS ) analysis_mirror_entry<N, TPS>(),
+#define PV_S( N, TPS, ONE ) synthesis_entry<N, TPS, ONE>(),
+#define PV_SM( N, TPS, ONE, GEN ) synthesis_mirror_entry<N, TPS, ONE, GEN>(),
+		std::vector<KernelEntry> v{ PV_RELEASE_KERNELS( PV_A, PV_AM, PV_S, PV_SM ) };
+#undef PV_A
+#undef PV_AM
+#undef PV_S
+#undef PV_SM
+#ifdef FLAN_B200_DEBUG
+		add_variants<256>( v ); add_variants<512>( v ); add_variants<1024>( v ); add_variants<2048>( v ); add_variants<4096>( v ); add_variants<8192>( v );
+#endif
+		return v;
+		}();
+	return list;
+	}
+
+// The entry of a descriptor whose kind takes these arguments, or null.
+template<class Args> static const KernelEntry * find_kernel( const TransformKernel & k )
+	{
+	if( k.is_analysis() != std::is_same_v<Args, AnalysisArgs> ) return nullptr;
+	for( const KernelEntry & e : kernels() ) if( e.k == k ) return &e;
+	return nullptr;
+	}
+
+// Dynamic shared memory: the exchange buffers (one when they alias), then the analysis's per-bin sums (EMIT), the
+// mirrored analysis's window ring and scratch, or the resynthesis's overlap-add ring and row buffer.
+static size_t smem_bytes( const KernelEntry & e, int one_buffer )
+	{
+	const TransformKernel & k = e.k;
+	switch( k.kind )
+		{
+		case KernelKind::analysis: return ( k.ONE ? 1 : 2 ) * e.xbuf + ( k.EMIT ? sizeof( int ) * ( k.N / 2 + 4 ) : 0 ) + smem_pad();
+		case KernelKind::analysis_mirror: return ( one_buffer ? 1 : 2 ) * e.xbuf + sizeof( float2 ) * ( k.N / 2 + 16 ) + smem_pad();
+		default: return sizeof( float ) * k.N + ( k.ONE ? 1 : 2 ) * e.xbuf + sizeof( float2 ) * ( k.N / 2 + 2 ) + smem_pad();
+		}
+	}
+
+// Sets the kernel's shared-memory size (and in development builds the carveout); a tensor-memory kernel's CTAs per SM
+// go to *tmem_ctas (0 for the others).
+static cudaError_t prepare( const KernelEntry & e, size_t smem, int * tmem_ctas )
+	{
+	*tmem_ctas = 0;
+	const cudaError_t r = cudaFuncSetAttribute( e.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem );
+	if( r != cudaSuccess ) return r;
+	if( e.k.kind != KernelKind::synthesis ) apply_carveout( e.fn );
+	return e.tmem_ctas ? e.tmem_ctas( tmem_ctas ) : cudaSuccess;
+	}
+
+template<class Args> static cudaError_t launch_kernel( const TransformKernel & k, const Args & a, int64_t blocks, cudaStream_t st )
+	{
+	const KernelEntry * e = find_kernel<Args>( k );
+	if( !e ) return cudaErrorInvalidValue;
+	const size_t smem = smem_bytes( *e, a.one_buffer );
+	int ctas = 0;
+	const cudaError_t r = prepare( *e, smem, &ctas );
+	if( r != cudaSuccess ) return r;
+	void * args[] = { const_cast<Args *>( &a ) };
+	cudaLaunchKernel( e->fn, dim3( (unsigned) blocks ), dim3( (unsigned) e->threads ), args, smem, st );
 	return cudaGetLastError();
 	}
-template<int N, int TPS, bool ONE, bool GEN> static cudaError_t launch_synthesis_mirror_ntg( const SynthArgs & a, int64_t blocks, cudaStream_t st )
+
+template<class Args> static cudaError_t kernel_ctas( const TransformKernel & k, const Args & a, int * ctas )
 	{
-	const size_t smem = sizeof( float ) * N + ( ONE ? 1 : 2 ) * sizeof( float2 ) * XBuf<N / 2>::size + sizeof( float2 ) * ( N / 2 + 2 ) + smem_pad();
-	cudaError_t e = cudaFuncSetAttribute( pv_synthesis_mirror_kernel<N, TPS, ONE, GEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem );
-	if( e != cudaSuccess ) return e;
-	apply_carveout( pv_synthesis_mirror_kernel<N, TPS, ONE, GEN> );
-	if constexpr( synthesis_uses_tmem<N, TPS, GEN>() )
-		{
-		int ctas = 0;
-		e = tmem_kernel_ctas<pv_synthesis_mirror_kernel<N, TPS, ONE, GEN>, N / 32, SY_TM_COLS>( &ctas );
-		if( e != cudaSuccess ) return e;
-		if( blocks < 0 ) { g_occupancy = ctas; return cudaSuccess; }
-		}
-	if( blocks < 0 ) return report_occupancy( pv_synthesis_mirror_kernel<N, TPS, ONE, GEN>, N / 32, smem );
-	pv_synthesis_mirror_kernel<N, TPS, ONE, GEN><<<(unsigned) blocks, N / 32, smem, st>>>( a );
-	return cudaGetLastError();
-	}
-// the standard shape (window == dft, hop == dft/16: every BASELINE config) runs the compile-time form, any other aligned
-// window / hop (the API default 2048 / 128 / 4096 among them) the general one
-template<int N, int TPS, bool ONE> static cudaError_t launch_synthesis_mirror_nt( const SynthArgs & a, int64_t blocks, cudaStream_t st )
-	{
-	if( a.W == N && a.hop == N / 16 ) return launch_synthesis_mirror_ntg<N, TPS, ONE, false>( a, blocks, st );
-	return launch_synthesis_mirror_ntg<N, TPS, ONE, true>( a, blocks, st );
-	}
-bool synthesis_mirror_applies( int N, const SynthArgs & a )
-	{
-	if( !synth_mirror_supported( N ) ) return false;
-	if( a.W == N && a.hop == N / 16 ) return true;
-	// general form: the window fills whole slots of the thread layout (a multiple of dft/16 samples), the hop is even and
-	// at most one slot (dft/16 samples) and leaves no gaps
-	return a.W >= N / 16 && a.W % ( N / 16 ) == 0 && a.W <= N && a.hop >= 2 && a.hop % 2 == 0 && a.hop <= a.W && a.hop <= N / 16;
-	}
-template<int N> static cudaError_t launch_synthesis_n( const SynthArgs & a, int64_t blocks, cudaStream_t st, int tps, int variant )
-	{
-	if constexpr( N == 8192 )
-		{
-		// 256 threads: two CTAs per SM need 128 registers and one exchange buffer (102 KB of shared memory each)
-		if( variant == PV_PT_MIRROR && synthesis_mirror_applies( N, a ) )
-			{
-#ifdef FLAN_B200_DEBUG
-			if( !a.one_buffer ) return launch_synthesis_mirror_nt<N, 256, false>( a, blocks, st );
-#endif
-			return launch_synthesis_mirror_nt<N, 512, true>( a, blocks, st );
-			}
-		}
-	if constexpr( N == 1024 || N == 2048 || N == 4096 )
-		{
-		if( variant == PV_PT_MIRROR && synthesis_mirror_applies( N, a ) )
-			{
-#ifdef FLAN_B200_DEBUG
-			if( tps >= 512 ) return a.one_buffer ? launch_synthesis_mirror_nt<N, 512, true>( a, blocks, st ) : launch_synthesis_mirror_nt<N, 512, false>( a, blocks, st );
-			if( a.one_buffer ) return launch_synthesis_mirror_nt<N, 384, true>( a, blocks, st );
-#endif
-			// dft 4096, standard shape: window and tables in tensor memory, 128 registers, one exchange buffer, 4 CTAs per SM
-			if constexpr( N == 4096 ) { if( a.W == N && a.hop == N / 16 ) return launch_synthesis_mirror_ntg<N, 512, true, false>( a, blocks, st ); }
-			return launch_synthesis_mirror_nt<N, 384, false>( a, blocks, st );
-			}
-		}
-	// dft 8192: one exchange buffer and 64 registers per thread let two 512-thread CTAs share an SM
-	if constexpr( N == 8192 ) { if( tps >= 1024 ) return launch_synthesis_nt<N, 1024, true>( a, blocks, st ); }
-#ifdef FLAN_B200_DEBUG
-	if( tps >= 1024 ) return launch_synthesis_nt<N, 1024, false>( a, blocks, st );
-	if( tps < 768 ) return launch_synthesis_nt<N, 512, false>( a, blocks, st );
-#endif
-	return launch_synthesis_nt<N, 768, false>( a, blocks, st );
+	*ctas = 0;
+	const KernelEntry * e = find_kernel<Args>( k );
+	if( !e ) return cudaErrorInvalidValue;
+	const size_t smem = smem_bytes( *e, a.one_buffer );
+	const cudaError_t r = prepare( *e, smem, ctas );
+	if( r != cudaSuccess || e->tmem_ctas ) return r;
+	return cudaOccupancyMaxActiveBlocksPerMultiprocessor( ctas, e->fn, e->threads, smem );
 	}
 
-bool dft_size_supported( int N )
-	{
-	return N == 256 || N == 512 || N == 1024 || N == 2048 || N == 4096 || N == 8192;
-	}
-
-cudaError_t launch_analysis( int N, const AnalysisArgs & a, int64_t blocks, cudaStream_t st, int tps, int pt )
-	{
-	switch( N )
-		{
-		case 256:  return launch_analysis_n<256>( a, blocks, st, tps, pt );
-		case 512:  return launch_analysis_n<512>( a, blocks, st, tps, pt );
-		case 1024: return launch_analysis_n<1024>( a, blocks, st, tps, pt );
-		case 2048: return launch_analysis_n<2048>( a, blocks, st, tps, pt );
-		case 4096: return launch_analysis_n<4096>( a, blocks, st, tps, pt );
-		case 8192: return launch_analysis_n<8192>( a, blocks, st, tps, pt );
-		default:   return cudaErrorInvalidValue;
-		}
-	}
-
-cudaError_t launch_synthesis( int N, const SynthArgs & a, int64_t blocks, cudaStream_t st, int tps, int variant )
-	{
-	switch( N )
-		{
-		case 256:  return launch_synthesis_n<256>( a, blocks, st, tps, variant );
-		case 512:  return launch_synthesis_n<512>( a, blocks, st, tps, variant );
-		case 1024: return launch_synthesis_n<1024>( a, blocks, st, tps, variant );
-		case 2048: return launch_synthesis_n<2048>( a, blocks, st, tps, variant );
-		case 4096: return launch_synthesis_n<4096>( a, blocks, st, tps, variant );
-		case 8192: return launch_synthesis_n<8192>( a, blocks, st, tps, variant );
-		default:   return cudaErrorInvalidValue;
-		}
-	}
+cudaError_t launch( const TransformKernel & k, const AnalysisArgs & a, int64_t blocks, cudaStream_t st ) { return launch_kernel( k, a, blocks, st ); }
+cudaError_t launch( const TransformKernel & k, const SynthArgs & a, int64_t blocks, cudaStream_t st ) { return launch_kernel( k, a, blocks, st ); }
+cudaError_t resident_ctas( const TransformKernel & k, const AnalysisArgs & a, int * ctas ) { return kernel_ctas( k, a, ctas ); }
+cudaError_t resident_ctas( const TransformKernel & k, const SynthArgs & a, int * ctas ) { return kernel_ctas( k, a, ctas ); }
 
 cudaError_t launch_phase_seg( const PhaseSegArgs & a, int C, cudaStream_t st )
 	{

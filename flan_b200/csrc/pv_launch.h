@@ -3,6 +3,7 @@
 
 #include <cuda_runtime.h>
 #include "pv_body.cuh"
+#include "pv_policy.h"
 
 namespace pvk {
 
@@ -39,21 +40,14 @@ struct PhaseScanArgs
 	PvConsts fix_k; int * fix_nan_flag;
 	};
 
-// points_per_thread values of launch_analysis: 8, 16, or PV_PT_MIRROR (16 points per thread with the mirrored last
-// pass; dft 1024 / 2048 / 4096 only)
-#define PV_PT_MIRROR 17
-inline bool mirror_supported( int N ) { return N == 1024 || N == 2048 || N == 4096; }                 // analysis
-inline bool synth_mirror_supported( int N ) { return mirror_supported( N ) || N == 8192; }            // resynthesis
-
-bool dft_size_supported( int N );
-// launch_analysis / launch_synthesis with blocks < 0 launch nothing and leave the kernel's resident CTAs per SM here
-int last_occupancy();
-cudaError_t launch_analysis( int N, const AnalysisArgs & a, int64_t blocks, cudaStream_t st, int threads_per_sm, int points_per_thread );
-// variant: 8 = 8 points per thread (every size and shape); PV_PT_MIRROR = synthesis_cta_mirror where it applies
-// (synthesis_mirror_applies), the 8-point kernel otherwise
-cudaError_t launch_synthesis( int N, const SynthArgs & a, int64_t blocks, cudaStream_t st, int threads_per_sm, int variant );
-bool synthesis_mirror_applies( int N, const SynthArgs & a );
-bool analysis_mirror_applies( int N, const AnalysisArgs & a );
+// The transform kernels this build carries (pv_kernel_list.h), by the descriptor the launch policy (pv_policy.h)
+// returns. A descriptor the build does not carry, or one of the other stage, gives cudaErrorInvalidValue.
+cudaError_t launch( const TransformKernel & k, const AnalysisArgs & a, int64_t blocks, cudaStream_t st );
+cudaError_t launch( const TransformKernel & k, const SynthArgs & a, int64_t blocks, cudaStream_t st );
+// The kernel's resident CTAs per SM with these arguments' shared memory (the pipelined host forms cut a signal into
+// slices of whole waves). Kernels that allocate tensor memory: what their registers and columns admit.
+cudaError_t resident_ctas( const TransformKernel & k, const AnalysisArgs & a, int * ctas );
+cudaError_t resident_ctas( const TransformKernel & k, const SynthArgs & a, int * ctas );
 cudaError_t launch_phase_seg( const PhaseSegArgs & a, int C, cudaStream_t st );
 cudaError_t launch_phase_scan( const PhaseScanArgs & a, int C, cudaStream_t st );
 cudaError_t launch_phase_carry( const PhaseSeg * all, int rank, int64_t per_rank, PhaseSeg * carry, double P, double rcpP, cudaStream_t st );

@@ -1,7 +1,7 @@
 """Every release instantiation of the analysis and resynthesis kernels, reached on the GPU at the shapes and edges that
 select it, and checked against the oracle.
 
-The launch policy (pv_capi.cu: analysis_range / synth_range, pv_kernels.cu: launch_analysis_n / launch_synthesis_n)
+The launch policy (pv_policy.h: choose_analysis / choose_synthesis; tests/test_launch_policy.py checks it without a GPU)
 picks the instantiation from the dft size, W == N, hop == N/16, whether the window fills whole slots, even hops, pointer
 alignment, the resynthesis hint and the whole signal's frame count. Each test here names the instantiation its shape must
 reach and reads the kernels the call launched from the CUDA profiler, so a change of policy cannot move a shape off the
@@ -382,6 +382,8 @@ def test_synthesis_4096_standard_shape_variants(eng, oracle):
     (3000, 100, 4096, synthesis_plain(4096, 768, False)),
     (256, 16, 256, synthesis_plain(256, 768, False)),
     (300, 7, 512, synthesis_plain(512, 768, False)),
+    (1000, 50, 1024, synthesis_plain(1024, 768, False)),
+    (2048, 127, 2048, synthesis_plain(2048, 768, False)),
 ])
 def test_synthesis(eng, oracle, W, hop, N, expect):
     C = 3 if hop % 4 else 2
