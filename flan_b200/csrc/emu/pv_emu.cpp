@@ -61,28 +61,36 @@ struct HostEnv
 		while( std::atomic_ref<BulkBarrier>( *bar ).load( std::memory_order_acquire ) <= bulk_waits ) std::this_thread::yield();
 		++bulk_waits;
 		}
-	// tensor memory: the CTA's 128 lanes x TMEM_COLS words, lane = thread; a column read before this thread wrote it aborts
+	// tensor memory: the CTA's 128 lanes x TMEM_COLS words, lane = thread. A stored word stays pending until the thread's
+	// next tmem_wait_st; a column read before this thread wrote it, or while its store is pending, aborts.
 	static constexpr int TMEM_COLS = 128;
+	enum : unsigned char { TM_UNWRITTEN = 0, TM_DONE = 1, TM_PENDING = 2 };
 	float * tmem_words;
-	unsigned char * tmem_written;
+	unsigned char * tmem_state;
 	template<int K> void tmem_st( int col, const float * r )
 		{
 		for( int i = 0; i < K; ++i )
 			{
 			tmem_check( col + i );
 			tmem_words[tid * TMEM_COLS + col + i] = r[i];
-			tmem_written[tid * TMEM_COLS + col + i] = 1;
+			tmem_state[tid * TMEM_COLS + col + i] = TM_PENDING;
 			}
 		}
-	void tmem_wait_st() {}
+	void tmem_wait_st()
+		{
+		for( int j = 0; j < TMEM_COLS; ++j )
+			if( tmem_state[tid * TMEM_COLS + j] == TM_PENDING ) tmem_state[tid * TMEM_COLS + j] = TM_DONE;
+		}
 	template<int K> void tmem_ld( int col, float * r )
 		{
 		for( int i = 0; i < K; ++i )
 			{
 			tmem_check( col + i );
-			if( !tmem_written[tid * TMEM_COLS + col + i] )
+			const unsigned char s = tmem_state[tid * TMEM_COLS + col + i];
+			if( s != TM_DONE )
 				{
-				std::fprintf( stderr, "pv_emu: thread %d reads tensor-memory column %d before writing it\n", tid, col + i );
+				std::fprintf( stderr, s == TM_PENDING ? "pv_emu: thread %d reads tensor-memory column %d while its store is pending (no tmem_wait_st since)\n"
+				                                      : "pv_emu: thread %d reads tensor-memory column %d before writing it\n", tid, col + i );
 				std::abort();
 				}
 			r[i] = tmem_words[tid * TMEM_COLS + col + i];
@@ -105,7 +113,7 @@ template<int N, int PT, class Body> void run_cta( Body && body )
 	std::vector<float> ring( N );
 	std::vector<float2> x0( XBuf<N / 2>::size ), x1( XBuf<N / 2>::size ), rowbuf( N / 2 + 16 );
 	std::vector<float> tmem( 128 * HostEnv::TMEM_COLS );
-	std::vector<unsigned char> tmem_written( 128 * HostEnv::TMEM_COLS, 0 );
+	std::vector<unsigned char> tmem_state( 128 * HostEnv::TMEM_COLS, HostEnv::TM_UNWRITTEN );
 	std::barrier<> bar( T );
 	std::vector<std::unique_ptr<std::barrier<>>> warpbars;
 	for( int w = 0; w < ( T + 31 ) / 32; ++w ) warpbars.emplace_back( new std::barrier<>( T - 32 * w < 32 ? T - 32 * w : 32 ) );
@@ -113,7 +121,7 @@ template<int N, int PT, class Body> void run_cta( Body && body )
 	for( int t = 0; t < T; ++t )
 		th.emplace_back( [&, t]
 			{
-			HostEnv env{ t, &bar, 0, warpbars[t / 32].get(), tmem.data(), tmem_written.data() };
+			HostEnv env{ t, &bar, 0, warpbars[t / 32].get(), tmem.data(), tmem_state.data() };
 			body( env, ring.data(), x0.data(), x1.data(), rowbuf.data() );
 			} );
 	for( auto & x : th ) x.join();

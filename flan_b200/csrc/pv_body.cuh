@@ -119,10 +119,12 @@ struct AnalysisArgs
 // the walk is stored there once, instead of living in registers (the window) or being re-read through L1 (the tables):
 //   columns  0..31  window coefficients w[0..31]
 //           32..59  the 14 twiddles of the last pass (radix 8, two butterflies)
-//           64..127 per slot u, 8 columns: binc4[k] (4), post_rot[k] (2), two unused, k = t + u*T
-// The first pass's twiddles stay in L1: their index is t mod 16, 240 entries in all.
+//           60      EMIT: the sum of bin M/2 (thread T/2; the other threads' column 60 stays zero)
+//           64..127 per slot u, 8 columns: binc4[k] (4), post_rot[k] (2), EMIT: the sums of bins k and M-k (2), k = t + u*T
+// The first pass's twiddles stay in L1: their index is t mod 16, 240 entries in all. The sums (EMIT, below) are int32
+// bit patterns; they start as the zeros the table stores write.
 template<int N, int PT> constexpr bool analysis_tmem() { return PT == 16 && N == 4096; }
-constexpr int AN_TM_COLS = 128, AN_TM_WIN = 0, AN_TM_TW = 32, AN_TM_BIN = 64;
+constexpr int AN_TM_COLS = 128, AN_TM_WIN = 0, AN_TM_TW = 32, AN_TM_MID = 60, AN_TM_BIN = 64, AN_TM_SUM = 6;
 
 // PAD: a zero-padded window that fills whole slots of the thread layout (window a multiple of 2T samples, < dft: the
 // API default window 2048 / dft 4096, Audio.h:158-163) loads its samples as vectors like the full window does; a
@@ -131,7 +133,8 @@ constexpr int AN_TM_COLS = 128, AN_TM_WIN = 0, AN_TM_TW = 32, AN_TM_BIN = 64;
 // from a second read of the rows. A bin's increment inc = float( f / ar * pi2 ) lies within pi of its expected phase
 // advance c (the table value the phase vocoder subtracts); from c >= 2 and inc >= 2 on both are multiples of 2^-22, so
 // d = inc - c is exact, |d| < 4, and the segment's sum of up to 128 such d fits an int32 in units of 2^-22: ONE shared-
-// memory word per bin, private to the thread that owns the bin (`ssum`, M + 1 ints), no registers. The total
+// memory word per bin, private to the thread that owns the bin (`ssum`, M + 1 ints; TM: two spare columns of the slot's
+// group of the tensor-memory layout and column AN_TM_MID, read with the slot's constants), no registers. The total
 // frames * c + 2^-22 * sum is exact in double and equals the plain double running sum of pv_phase_seg_kernel bit for
 // bit (that sum is exact too: multiples of 2^-22 below 2^18); increments are positive, so the running maximum is the
 // total. A bin that ever leaves those conditions (the lowest bins, NaN / Inf) is marked and gets the NaN entry.
@@ -202,12 +205,14 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 #pragma unroll
 		for( int u = 0; u < H; ++u )
 			{
-			ssum[t + u * T] = 0; ssum[M - t - u * T] = 0;
+			if( !TM ) { ssum[t + u * T] = 0; ssum[M - t - u * T] = 0; }
 			const float4 cc = env.ldg4( a.binc4 + ( t + u * T ) );
 			dirty |= ( cc.z >= 6.0f ? 0u : 1u << ( 2 * u ) ) | ( -cc.w >= 6.0f ? 0u : 2u << ( 2 * u ) );
 			}
-		if( t == T / 2 ) { ssum[M / 2] = 0; dirty |= env.ldg2( a.binc + M / 2 ).y >= 6.0f ? 0u : 1u << ( 2 * H ); }
+		if( t == T / 2 ) { if( !TM ) ssum[M / 2] = 0; dirty |= env.ldg2( a.binc + M / 2 ).y >= 6.0f ? 0u : 1u << ( 2 * H ); }
 		}
+	// EMIT, TM: the warp of thread T/2 reads and writes column AN_TM_MID together (tcgen05 is warp-wide)
+	const bool mid_warp = ( t >> 5 ) == ( ( T / 2 ) >> 5 );
 
 	// The serial reference loop carries frame f-1's phase into frame f (phase_vocoder.cpp:44-45); a segment
 	// that does not start at frame 0 recomputes it with one warm-up FFT.
@@ -297,6 +302,7 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 			if constexpr( ONE ) env.sync();
 			env.template tmem_wait<28>( reinterpret_cast<float *>( tw2 ) );
 			fft_butterflies_w<M, PT, P::radix( 2 ), P::ns( 2 )>( v, tw2 );
+			if constexpr( EMIT ) env.tmem_wait_st();       // the sums the previous frame stored (long done) are read next
 			env.template tmem_ld<8>( AN_TM_BIN, tab[0] );
 #pragma unroll
 			for( int s = PT / 2; s < PT; ++s ) x0[t + s * T] = v[s];
@@ -313,9 +319,11 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 		// real-FFT unpack + phase vocoder (AudioPV.cpp:69-73). The warm-up frame runs the same code with its stores
 		// predicated off: only the phases it leaves in prev[] matter.
 		const bool emit = ( f >= fa );
+		float mid[2];               // EMIT, TM: columns AN_TM_MID, +1 of the warp of thread T/2, requested with slot H-1's constants
 #pragma unroll
 		for( int u = 0; u < H; ++u )
 			{
+			const float * tu = tab[u & 1];
 			const int k = t + u * T;
 			// X[k] = (Zk + conj Zm) + (-i w_k)(Zk - conj Zm),  conj X[M-k] = (Zk + conj Zm) - (-i w_k)(Zk - conj Zm), Zm = Z[M-k].
 			// k = 0 pairs Z[0] with itself and yields DC in X[k] and Nyquist (bin M) in X[M-k], both real.
@@ -329,11 +337,12 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 			float4 cc;
 			if constexpr( TM )
 				{
-				// slot u's constants were requested one slot ahead (slot 0's before the barrier)
-				float * tu = tab[u & 1];
-				env.template tmem_wait<6>( tu );
+				// slot u's constants (and sums) were requested one slot ahead (slot 0's before the barrier)
+				env.template tmem_wait<EMIT ? 8 : 6>( tab[u & 1] );
+				if( EMIT && u == H - 1 && emit && mid_warp ) env.template tmem_wait<2>( mid );
 				cc.x = tu[0]; cc.y = tu[1]; cc.z = tu[2]; cc.w = tu[3]; rot.x = tu[4]; rot.y = tu[5];
 				if( u + 1 < H ) env.template tmem_ld<8>( AN_TM_BIN + 8 * ( u + 1 ), tab[( u + 1 ) & 1] );
+				if( EMIT && u + 1 == H - 1 && emit && mid_warp ) env.template tmem_ld<2>( AN_TM_MID, mid );
 				}
 			else
 				{
@@ -373,13 +382,24 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 					const float2 sc = mul2( dd, splat2( 4194304.0f ) );                     // (inc - c) * 2^22: exact, an integer
 					const bool ok_k = fabsf( sc.x ) < 16777216.0f && fabsf( mk.x ) <= 3.402823466e38f;
 					const bool ok_m = fabsf( sc.y ) < 16777216.0f && fabsf( mm.x ) <= 3.402823466e38f;
-					env.shared_add( ssum + k, (int) sc.x );
-					env.shared_add( ssum + ( M - k ), (int) sc.y );
+					if constexpr( TM )
+						{
+						float s2[2];
+						s2[0] = int_bits_add( tu[AN_TM_SUM], (int) sc.x );
+						s2[1] = int_bits_add( tu[AN_TM_SUM + 1], (int) sc.y );
+						env.template tmem_st<2>( AN_TM_BIN + 8 * u + AN_TM_SUM, s2 );
+						}
+					else
+						{
+						env.shared_add( ssum + k, (int) sc.x );
+						env.shared_add( ssum + ( M - k ), (int) sc.y );
+						}
 					dirty |= ( ok_k ? 0u : 1u << ( 2 * u ) ) | ( ok_m ? 0u : 2u << ( 2 * u ) );
 					}
 				}
 			}
 		if constexpr( TM ) { if( f + 1 < fb ) env.template tmem_ld<2 * PT>( AN_TM_WIN, w ); }     // the next frame's window
+		int mid_add = 0;            // EMIT, TM: what thread T/2 adds to its column AN_TM_MID (the rest of its warp adds 0)
 		if( t == T / 2 )
 			{
 			const float2 zh = z[M / 2];                           // X[M/2] = conj(Z[M/2])
@@ -390,8 +410,17 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 				{
 				const float sc = mul_rn( sub_rn( phase_increment( mh.y, a.k ), ch.y ), 4194304.0f );
 				const bool ok = fabsf( sc ) < 16777216.0f && fabsf( mh.x ) <= 3.402823466e38f;
-				env.shared_add( ssum + M / 2, (int) sc );
+				if( TM ) mid_add = (int) sc;
+				else env.shared_add( ssum + M / 2, (int) sc );
 				dirty |= ok ? 0u : 1u << ( 2 * H );
+				}
+			}
+		if constexpr( EMIT && TM )
+			{
+			if( emit && mid_warp )
+				{
+				mid[0] = int_bits_add( mid[0], mid_add );
+				env.template tmem_st<2>( AN_TM_MID, mid );
 				}
 			}
 		// the next frame's pass 0 writes x0, last read two barriers ago; its pass 1 writes x1 after one more barrier
@@ -401,24 +430,46 @@ PV_HD void analysis_cta( const AnalysisArgs & a, int64_t block, Env & env, float
 		{
 		PhaseSeg * out = a.seg_out + ( (int64_t) c * a.segs_per_channel + seg ) * (int64_t)( M + 1 );
 		const double frames = (double)( fb - fa );
-		auto put = [&]( int bin, float center, bool bad )
+		auto put = [&]( int bin, float center, bool bad, int sum )
 			{
 			PhaseSeg s;
-			const double total = frames * (double) center + (double) ssum[bin] * 2.384185791015625e-07;    // 2^-22; exact
+			const double total = frames * (double) center + (double) sum * 2.384185791015625e-07;    // 2^-22; exact
 			phase_sum_from_double( total, a.P, a.rcpP, s.sum.q, s.sum.r );
 			s.mx = s.sum;                                                 // every increment was positive
 			if( bad ) s.sum.q = nan_marker();
 			out[bin] = s;
 			};
+		if constexpr( TM ) env.tmem_wait_st();
 #pragma unroll
 		for( int u = 0; u < H; ++u )
 			{
 			const int k = t + u * T;
+			int sk, sm;
+			if constexpr( TM )
+				{
+				float s2[2];
+				env.template tmem_ld<2>( AN_TM_BIN + 8 * u + AN_TM_SUM, s2 );
+				env.template tmem_wait<2>( s2 );
+				sk = int_bits( s2[0] ); sm = int_bits( s2[1] );
+				}
+			else { sk = ssum[k]; sm = ssum[M - k]; }
 			const float4 cc = env.ldg4( a.binc4 + k );
-			put( k, cc.z, ( dirty >> ( 2 * u ) ) & 1u );
-			put( M - k, -cc.w, ( dirty >> ( 2 * u + 1 ) ) & 1u );           // slot (0, 0): DC in lane x, Nyquist (bin M) in lane y
+			put( k, cc.z, ( dirty >> ( 2 * u ) ) & 1u, sk );
+			put( M - k, -cc.w, ( dirty >> ( 2 * u + 1 ) ) & 1u, sm );           // slot (0, 0): DC in lane x, Nyquist (bin M) in lane y
 			}
-		if( t == T / 2 ) put( M / 2, env.ldg2( a.binc + M / 2 ).y, ( dirty >> ( 2 * H ) ) & 1u );
+		int smid = 0;
+		if constexpr( TM )
+			{
+			if( mid_warp )
+				{
+				float s2[2];
+				env.template tmem_ld<2>( AN_TM_MID, s2 );
+				env.template tmem_wait<2>( s2 );
+				smid = int_bits( s2[0] );
+				}
+			}
+		else if( t == T / 2 ) smid = ssum[M / 2];
+		if( t == T / 2 ) put( M / 2, env.ldg2( a.binc + M / 2 ).y, ( dirty >> ( 2 * H ) ) & 1u, smid );
 		}
 	}
 
@@ -978,10 +1029,14 @@ template<int R> PV_HD int mpad( int i )
 // CTA: four CTAs per SM at 128 registers use all 512):
 //   columns  0..31  window coefficients w[0..31]
 //           32..47  post_tw[k] of the thread's 8 bins (slot r at 32 + 2r)
-//           48..77  the 15 twiddles of the second radix-16 pass (78..79 unused)
-// The window is read once per frame, for the overlap-add; the first pass's twiddles stay in L1 (index t mod 8).
+//           48..77  the 15 twiddles of the second radix-16 pass (78..95 zero)
+//           96..125 the overlap-add partials: R[j] at 96 + 2j, j = 0..14, the partial sum of slot j of the next frame
+//                   (126..127 zero)
+// The window is read once per frame, for the overlap-add; the first pass's twiddles stay in L1 (index t mod 8). The
+// partials replace the shared-memory ring of the other sizes: slot s of frame f is slot s-1 of frame f+1, so instead of
+// a rotating address the sums move down one column pair per frame, a renaming fixed at compile time.
 template<int N, bool GEN> constexpr bool synthesis_tmem() { return N == 4096 && !GEN; }
-constexpr int SY_TM_COLS = 128, SY_TM_WIN = 0, SY_TM_POST = 32, SY_TM_TW = 48;
+constexpr int SY_TM_COLS = 128, SY_TM_WIN = 0, SY_TM_POST = 32, SY_TM_TW = 48, SY_TM_OLA = 96;
 
 // TM: the tensor-memory form (synthesis_tmem); the Env then addresses the CTA's SY_TM_COLS columns.
 template<int N, bool ONE, bool GEN, bool TM = synthesis_tmem<N, GEN>(), class Env>
@@ -1027,6 +1082,31 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 			}
 		else { w[2 * s] = 0.0f; w[2 * s + 1] = 0.0f; }
 		}
+	// TM: the tables go to tensor memory before the accumulators are loaded; with all three live at once ptxas keeps four
+	// accumulators in local memory for the whole frame loop
+	if constexpr( TM )
+		{
+		env.template tmem_st<32>( SY_TM_WIN, w );
+		float2 tb[32];              // columns 32..95: post_tw, the pass twiddles, zeros
+#pragma unroll
+		for( int r = 0; r < R; ++r ) tb[r] = env.ldg2( a.post_tw + ( t + ( ( r >= R / 2 ) ? khi : 0 ) + r * NS ) );
+		fft_load_twiddles<M, PT, PT, RP::NS2>( t, tb + 8, a.pass_tw_rev + RP::tw2, [&]( const float2 * q ) { return env.ldg2( q ); } );
+#pragma unroll
+		for( int i = 23; i < 32; ++i ) { tb[i].x = 0.0f; tb[i].y = 0.0f; }
+		env.template tmem_st<32>( SY_TM_POST, reinterpret_cast<const float *>( tb ) );
+		env.template tmem_st<32>( SY_TM_POST + 32, reinterpret_cast<const float *>( tb + 16 ) );
+#pragma unroll
+		for( int i = 0; i < 16; ++i ) { tb[i].x = 0.0f; tb[i].y = 0.0f; }
+		env.template tmem_st<32>( SY_TM_OLA, reinterpret_cast<const float *>( tb ) );
+		env.tmem_wait_st();
+		}
+	else
+		{
+		// thread-private overlap-add ring: 16 pairs at ring[t + T*j]; absolute pair index t + T*A lives in slot A & 15
+#pragma unroll
+		for( int j = 0; j < PT; ++j ) { float2 z; z.x = 0.0f; z.y = 0.0f; ring[t + T * j] = z; }
+		}
+
 	// bin of slot (q, r): k = kbase + r*NS with kbase = p (+ khi for the irregular upper slots); its mirror is M - k
 	double acc[Q][R][2], acc_mid = 0.0;
 	const double * acc0 = a.acc_start + ( (int64_t) c * a.segs_per_channel + seg ) * B;
@@ -1040,24 +1120,6 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 			acc[q][r][1] = acc0[M - k];
 			}
 	if( irregular ) acc_mid = acc0[M / 2];
-	if constexpr( TM )
-		{
-		env.template tmem_st<32>( SY_TM_WIN, w );
-		float2 tb[32];              // columns 32..95: post_tw, the pass twiddles, zeros
-#pragma unroll
-		for( int r = 0; r < R; ++r ) tb[r] = env.ldg2( a.post_tw + ( t + ( ( r >= R / 2 ) ? khi : 0 ) + r * NS ) );
-		fft_load_twiddles<M, PT, PT, RP::NS2>( t, tb + 8, a.pass_tw_rev + RP::tw2, [&]( const float2 * q ) { return env.ldg2( q ); } );
-#pragma unroll
-		for( int i = 23; i < 32; ++i ) { tb[i].x = 0.0f; tb[i].y = 0.0f; }
-		env.template tmem_st<32>( SY_TM_POST, reinterpret_cast<const float *>( tb ) );
-		env.template tmem_st<32>( SY_TM_POST + 32, reinterpret_cast<const float *>( tb + 16 ) );
-		env.tmem_wait_st();
-		}
-
-	// thread-private overlap-add ring: 16 pairs at ring[t + T*j]; absolute pair index t + T*A lives in slot A & 15
-#pragma unroll
-	for( int j = 0; j < PT; ++j ) { float2 z; z.x = 0.0f; z.y = 0.0f; ring[t + T * j] = z; }
-
 	// Row staging. A row is 8 B * (M+1) long and only 8-byte aligned, so the bulk (TMA) copy fetches the enclosing
 	// 16-byte aligned span -- at most one (m,f) pair of a neighbouring row on either side -- and the row starts `shift`
 	// elements into the buffer. One thread issues it, completion arrives on an mbarrier. Where the span would leave
@@ -1244,47 +1306,67 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 			fft_butterflies_w<M, PT, RP::R3, RP::NS3>( v, tw );
 			}
 
-		// windowed overlap-add (AudioPV.cpp:133-134). !GEN: on the thread's own ring; slot s of this frame is absolute pair
-		// t + T*(f + s - 8) (half/2 == 8T), i.e. ring entry (f + s + 8) & 15
-		// (byte offsets: (t + T*((f + 8 + s) & 15)) * 8 == ((t + T*(f + 8)) * 8 + s*T*8) & (16*T*8 - 1), one add and one mask per slot).
-		// GEN: absolute pair hp*f - wp/2 + t + s*T, ring entry that modulo 16T (the ring holds dft/2 >= wp pairs).
-		const unsigned xb = GEN ? (unsigned)( ( (int64_t) hp * f - wp / 2 + t + (int64_t) PT * T * 4096 ) & (int64_t)( PT * T - 1 ) ) * 8u
-		                        : ( (unsigned) t + (unsigned) T * (unsigned)( ( f + 8 ) & 15 ) ) * 8u;
-		auto slot = [&]( int s ) { return reinterpret_cast<float2 *>( reinterpret_cast<char *>( ring ) + ( ( xb + (unsigned)( s * T * 8 ) ) & (unsigned)( 16 * T * 8 - 1 ) ) ); };
-		if constexpr( TM ) env.template tmem_wait<2 * PT>( w );
+		// windowed overlap-add (AudioPV.cpp:133-134)
 		float2 sum[PT];
-#pragma unroll
-		for( int s = 0; s < PT; ++s )
+		if constexpr( TM )
 			{
-			float2 ww; ww.x = w[2 * s]; ww.y = w[2 * s + 1];
-			const float2 prod = mul2( swap2( v[s] ), ww );
-			// a fresh slot receives its first contribution (its ring entry is simply overwritten)
-			if( GEN )
-				{
-				float2 cur; cur.x = 0.0f; cur.y = 0.0f;
-				if( s < slots_in ) cur = *slot( s );                       // uniform over the CTA
-				sum[s] = ( s == slots_in - 1 && is_fresh ) ? prod : add2( cur, prod );
-				}
-			else sum[s] = ( s == PT - 1 ) ? prod : add2( *slot( s ), prod );
-			}
-		if( GEN )
-			{
+			// TM: sum[s] = R[s] + prod[s], sum[15] = prod[15], then R[s-1] = sum[s]. R is read in x8 chunks of four slots (the
+			// last one ends in the zero columns 126..127), each requested one chunk ahead, and written back in x8 chunks as soon
+			// as the four sums of one are complete: 30 more live registers at once would not fit. The stores of this frame are
+			// waited for (wait::st) before the next frame reads the columns, long after they were issued.
+			float rb[2][8];
+			env.tmem_wait_st();
+			env.template tmem_ld<8>( SY_TM_OLA, rb[0] );
+			env.template tmem_wait<2 * PT>( w );
+			env.template tmem_wait<8>( rb[0] );
 #pragma unroll
-			for( int s = 1; s < PT; ++s ) if( s < slots_in ) *slot( s ) = sum[s];
-			if( !is_final ) *slot( 0 ) = sum[0];
-			else
+			for( int c = 0; c < PT / 4; ++c )
 				{
-				// final pairs: no later frame reaches them
-				const bool fast = start >= interior_lo && start + hop <= interior_hi && start >= a.out_lo && start + hop <= a.out_hi && a.out_aligned2;
-				const int64_t pos = start + 2 * t;
-				if( fast ) env.st_stream2( reinterpret_cast<float2 *>( och + ( pos - a.out_offset ) ), sum[0] );
-				else { emit( pos, sum[0].x ); emit( pos + 1, sum[0].y ); }
+				if( c > 0 ) env.template tmem_wait<8>( rb[c & 1] );
+				if( c + 1 < PT / 4 ) env.template tmem_ld<8>( SY_TM_OLA + 8 * ( c + 1 ), rb[( c + 1 ) & 1] );
+#pragma unroll
+				for( int j = 0; j < 4; ++j )
+					{
+					const int s = 4 * c + j;
+					float2 ww; ww.x = w[2 * s]; ww.y = w[2 * s + 1];
+					const float2 prod = mul2( swap2( v[s] ), ww );
+					float2 cur; cur.x = rb[c & 1][2 * j]; cur.y = rb[c & 1][2 * j + 1];
+					sum[s] = ( s == PT - 1 ) ? prod : add2( cur, prod );
+					}
+				if( c > 0 ) env.template tmem_st<8>( SY_TM_OLA + 8 * ( c - 1 ), reinterpret_cast<const float *>( sum + 4 * c - 3 ) );
 				}
+			env.template tmem_st<4>( SY_TM_OLA + 24, reinterpret_cast<const float *>( sum + 13 ) );
+			env.template tmem_st<2>( SY_TM_OLA + 28, reinterpret_cast<const float *>( sum + 15 ) );
 			}
 		else
 			{
+			// !GEN: on the thread's own ring; slot s of this frame is absolute pair t + T*(f + s - 8) (half/2 == 8T), i.e. ring
+			// entry (f + s + 8) & 15 (byte offsets: (t + T*((f + 8 + s) & 15)) * 8 == ((t + T*(f + 8)) * 8 + s*T*8) & (16*T*8 - 1),
+			// one add and one mask per slot).
+			// GEN: absolute pair hp*f - wp/2 + t + s*T, ring entry that modulo 16T (the ring holds dft/2 >= wp pairs).
+			const unsigned xb = GEN ? (unsigned)( ( (int64_t) hp * f - wp / 2 + t + (int64_t) PT * T * 4096 ) & (int64_t)( PT * T - 1 ) ) * 8u
+			                        : ( (unsigned) t + (unsigned) T * (unsigned)( ( f + 8 ) & 15 ) ) * 8u;
+			auto slot = [&]( int s ) { return reinterpret_cast<float2 *>( reinterpret_cast<char *>( ring ) + ( ( xb + (unsigned)( s * T * 8 ) ) & (unsigned)( 16 * T * 8 - 1 ) ) ); };
 #pragma unroll
-			for( int s = 1; s < PT; ++s ) *slot( s ) = sum[s];
+			for( int s = 0; s < PT; ++s )
+				{
+				float2 ww; ww.x = w[2 * s]; ww.y = w[2 * s + 1];
+				const float2 prod = mul2( swap2( v[s] ), ww );
+				// a fresh slot receives its first contribution (its ring entry is simply overwritten)
+				if( GEN )
+					{
+					float2 cur; cur.x = 0.0f; cur.y = 0.0f;
+					if( s < slots_in ) cur = *slot( s );                       // uniform over the CTA
+					sum[s] = ( s == slots_in - 1 && is_fresh ) ? prod : add2( cur, prod );
+					}
+				else sum[s] = ( s == PT - 1 ) ? prod : add2( *slot( s ), prod );
+				}
+#pragma unroll
+			for( int s = 1; s < PT; ++s ) if( !GEN || s < slots_in ) *slot( s ) = sum[s];
+			if( !is_final ) *slot( 0 ) = sum[0];
+			}
+		if( is_final )
+			{
 			// slot 0: no later frame reaches these two samples
 			const bool fast = start >= interior_lo && start + hop <= interior_hi && start >= a.out_lo && start + hop <= a.out_hi && a.out_aligned2;
 			const int64_t pos = start + 2 * t;
@@ -1310,10 +1392,19 @@ PV_HD void synthesis_cta_mirror( const SynthArgs & a, int64_t block, Env & env, 
 		return;
 		}
 	const int j0 = (int)( ( ( fb - 1 ) + 8 ) & 15 );
+	if constexpr( TM ) env.tmem_wait_st();
 #pragma unroll 1
 	for( int s = 1; s < PT; ++s )
 		{
-		const float2 val = ring[t + T * ( ( j0 + s ) & 15 )];
+		float2 val;
+		if constexpr( TM )
+			{
+			float r[2];
+			env.template tmem_ld<2>( SY_TM_OLA + 2 * ( s - 1 ), r );
+			env.template tmem_wait<2>( r );
+			val.x = r[0]; val.y = r[1];
+			}
+		else val = ring[t + T * ( ( j0 + s ) & 15 )];
 		const int64_t pos = last_start + 2 * ( t + s * T );
 		emit( pos, val.x ); emit( pos + 1, val.y );
 		}

@@ -13,6 +13,7 @@
 
 #include <stdint.h>
 #include <math.h>
+#include <string.h>
 #include <vector_types.h>
 
 #if defined(__CUDACC__)
@@ -58,6 +59,28 @@ PV_HD float fma_rn( float a, float b, float c )
 	return __fmaf_rn( a, b, c );
 #else
 	return fmaf( a, b, c );
+#endif
+	}
+
+// An int32 kept as the bit pattern of a float (a tensor-memory column) plus v, as such a bit pattern again.
+PV_HD float int_bits_add( float bits, int v )
+	{
+#if defined(__CUDA_ARCH__)
+	return __int_as_float( __float_as_int( bits ) + v );
+#else
+	int i; memcpy( &i, &bits, sizeof i );
+	i = (int)( (unsigned) i + (unsigned) v );
+	float r; memcpy( &r, &i, sizeof r );
+	return r;
+#endif
+	}
+PV_HD int int_bits( float bits )
+	{
+#if defined(__CUDA_ARCH__)
+	return __float_as_int( bits );
+#else
+	int i; memcpy( &i, &bits, sizeof i );
+	return i;
 #endif
 	}
 

@@ -89,20 +89,35 @@ struct DeviceEnv
 	// Tensor memory as per-thread storage (no MMA): `tmem` is the CTA's allocation plus this warp's lane quarter, so
 	// column j of the calling thread is word j of its private row. tcgen05.ld / .st are .sync.aligned: every lane of the
 	// warp issues them together. A load's registers are defined only after tmem_wait, which also ties them to it so
-	// that no use can be scheduled above the wait.
+	// that no use can be scheduled above the wait. A column this thread stored is read back only after a tmem_wait_st
+	// that follows the store (tcgen05.st and tcgen05.ld of one thread are not ordered with each other otherwise); the
+	// emulator (emu/pv_emu.cpp) aborts on a load that breaks this. Stores and waits carry no memory clobber either.
 	uint32_t tmem;
 	template<int K> __device__ __forceinline__ void tmem_st( int col, const float * r )
 		{
-		static_assert( K == 32, "stores go in 32-column chunks" );
-		asm volatile( "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,"
-		              "%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,%32};"
-		              :: "r"( tmem + (uint32_t) col ),
-		                 "f"( r[0] ), "f"( r[1] ), "f"( r[2] ), "f"( r[3] ), "f"( r[4] ), "f"( r[5] ), "f"( r[6] ), "f"( r[7] ),
-		                 "f"( r[8] ), "f"( r[9] ), "f"( r[10] ), "f"( r[11] ), "f"( r[12] ), "f"( r[13] ), "f"( r[14] ), "f"( r[15] ),
-		                 "f"( r[16] ), "f"( r[17] ), "f"( r[18] ), "f"( r[19] ), "f"( r[20] ), "f"( r[21] ), "f"( r[22] ), "f"( r[23] ),
-		                 "f"( r[24] ), "f"( r[25] ), "f"( r[26] ), "f"( r[27] ), "f"( r[28] ), "f"( r[29] ), "f"( r[30] ), "f"( r[31] ) : "memory" );
+		const uint32_t a = tmem + (uint32_t) col;
+		if constexpr( K == 2 )
+			asm volatile( "tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1,%2};" :: "r"( a ), "f"( r[0] ), "f"( r[1] ) );
+		else if constexpr( K == 4 )
+			asm volatile( "tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" :: "r"( a ), "f"( r[0] ), "f"( r[1] ), "f"( r[2] ), "f"( r[3] ) );
+		else if constexpr( K == 8 )
+			asm volatile( "tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
+			              :: "r"( a ), "f"( r[0] ), "f"( r[1] ), "f"( r[2] ), "f"( r[3] ), "f"( r[4] ), "f"( r[5] ), "f"( r[6] ), "f"( r[7] ) );
+		else if constexpr( K == 16 )
+			asm volatile( "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
+			              :: "r"( a ), "f"( r[0] ), "f"( r[1] ), "f"( r[2] ), "f"( r[3] ), "f"( r[4] ), "f"( r[5] ), "f"( r[6] ), "f"( r[7] ),
+			                 "f"( r[8] ), "f"( r[9] ), "f"( r[10] ), "f"( r[11] ), "f"( r[12] ), "f"( r[13] ), "f"( r[14] ), "f"( r[15] ) );
+		else if constexpr( K == 32 )
+			asm volatile( "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,"
+			              "%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,%32};"
+			              :: "r"( a ),
+			                 "f"( r[0] ), "f"( r[1] ), "f"( r[2] ), "f"( r[3] ), "f"( r[4] ), "f"( r[5] ), "f"( r[6] ), "f"( r[7] ),
+			                 "f"( r[8] ), "f"( r[9] ), "f"( r[10] ), "f"( r[11] ), "f"( r[12] ), "f"( r[13] ), "f"( r[14] ), "f"( r[15] ),
+			                 "f"( r[16] ), "f"( r[17] ), "f"( r[18] ), "f"( r[19] ), "f"( r[20] ), "f"( r[21] ), "f"( r[22] ), "f"( r[23] ),
+			                 "f"( r[24] ), "f"( r[25] ), "f"( r[26] ), "f"( r[27] ), "f"( r[28] ), "f"( r[29] ), "f"( r[30] ), "f"( r[31] ) );
+		else static_assert( K == 2, "tcgen05.st widths 2, 4, 8, 16, 32" );
 		}
-	__device__ __forceinline__ void tmem_wait_st() { asm volatile( "tcgen05.wait::st.sync.aligned;" ::: "memory" ); }
+	__device__ __forceinline__ void tmem_wait_st() { asm volatile( "tcgen05.wait::st.sync.aligned;" ); }
 	template<int K> __device__ __forceinline__ void tmem_ld( int col, float * r )
 		{
 		const uint32_t a = tmem + (uint32_t) col;
@@ -188,9 +203,11 @@ __global__ void __launch_bounds__( N / ( 2 * PT ), min_blocks( N / ( 2 * PT ), T
 	extern __shared__ __align__( 16 ) unsigned char smem_raw[];
 	float2 * x0 = reinterpret_cast<float2 *>( smem_raw );
 	float2 * x1 = ONE ? x0 : x0 + XBuf<N / 2>::size;
-	int * ssum = EMIT ? reinterpret_cast<int *>( x1 + XBuf<N / 2>::size ) : nullptr;      // N/2 + 1 per-bin sums (EMIT only)
+	constexpr bool TM = analysis_uses_tmem<N, PT, TPS>();
+	// N/2 + 1 per-bin sums (EMIT only; TM: in tensor memory)
+	int * ssum = EMIT && !TM ? reinterpret_cast<int *>( x1 + XBuf<N / 2>::size ) : nullptr;
 	DeviceEnv env; env.tid = threadIdx.x;
-	if constexpr( analysis_uses_tmem<N, PT, TPS>() )
+	if constexpr( TM )
 		{
 		__shared__ uint32_t tmem_slot;
 		TmemScope<AN_TM_COLS> scope( &tmem_slot );
@@ -229,14 +246,15 @@ __global__ void __launch_bounds__( N / 16, min_blocks( N / 16, TPS ) ) pv_synthe
 template<int N, int TPS, bool ONE, bool GEN>
 __global__ void __launch_bounds__( N / 32, min_blocks( N / 32, TPS ) ) pv_synthesis_mirror_kernel( const SynthArgs a )
 	{
+	constexpr bool TM = synthesis_uses_tmem<N, TPS, GEN>();
 	extern __shared__ __align__( 16 ) unsigned char smem_raw[];
-	float2 * ring = reinterpret_cast<float2 *>( smem_raw );                 // N/2 pairs
-	float2 * x0 = ring + N / 2;
+	float2 * ring = TM ? nullptr : reinterpret_cast<float2 *>( smem_raw );  // N/2 pairs (TM: the partials are in tensor memory)
+	float2 * x0 = reinterpret_cast<float2 *>( smem_raw ) + ( TM ? 0 : N / 2 );
 	float2 * x1 = ONE ? x0 : x0 + XBuf<N / 2>::size;
 	float2 * rowbuf = x1 + XBuf<N / 2>::size;                               // N/2 + 2 pairs
 	__shared__ __align__( 8 ) DeviceEnv::BulkBarrier bar;
 	DeviceEnv env; env.tid = threadIdx.x;
-	if constexpr( synthesis_uses_tmem<N, TPS, GEN>() )
+	if constexpr( TM )
 		{
 		__shared__ uint32_t tmem_slot;
 		TmemScope<SY_TM_COLS> scope( &tmem_slot );
@@ -600,14 +618,17 @@ template<class Args> static const KernelEntry * find_kernel( const TransformKern
 	}
 
 // Dynamic shared memory: the exchange buffers (one when they alias), then the analysis's per-bin sums (EMIT), the
-// mirrored analysis's window ring and scratch, or the resynthesis's overlap-add ring and row buffer.
+// mirrored analysis's window ring and scratch, or the resynthesis's overlap-add ring and row buffer. The tensor-memory
+// kernels keep the per-bin sums and the overlap-add partials in tensor memory instead.
 static size_t smem_bytes( const KernelEntry & e, int one_buffer )
 	{
 	const TransformKernel & k = e.k;
+	const bool tm = e.tmem_ctas != nullptr;
 	switch( k.kind )
 		{
-		case KernelKind::analysis: return ( k.ONE ? 1 : 2 ) * e.xbuf + ( k.EMIT ? sizeof( int ) * ( k.N / 2 + 4 ) : 0 ) + smem_pad();
+		case KernelKind::analysis: return ( k.ONE ? 1 : 2 ) * e.xbuf + ( k.EMIT && !tm ? sizeof( int ) * ( k.N / 2 + 4 ) : 0 ) + smem_pad();
 		case KernelKind::analysis_mirror: return ( one_buffer ? 1 : 2 ) * e.xbuf + sizeof( float2 ) * ( k.N / 2 + 16 ) + smem_pad();
+		case KernelKind::synthesis_mirror: return ( tm ? 0 : sizeof( float ) * k.N ) + ( k.ONE ? 1 : 2 ) * e.xbuf + sizeof( float2 ) * ( k.N / 2 + 2 ) + smem_pad();
 		default: return sizeof( float ) * k.N + ( k.ONE ? 1 : 2 ) * e.xbuf + sizeof( float2 ) * ( k.N / 2 + 2 ) + smem_pad();
 		}
 	}

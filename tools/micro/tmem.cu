@@ -1,6 +1,7 @@
 // Tensor memory (TMEM) used as per-thread storage, no MMA: dependent-chain latency of tcgen05.ld.32x32b.x{4,16,32} +
 // tcgen05.wait::ld against an L1-hit LDG.64 and an LDS.64, and per-SM load throughput with 16 resident warps
-// (4 CTAs x 128 threads, 128 columns each: the whole 512-column TMEM of the SM).
+// (4 CTAs x 128 threads, 128 columns each: the whole 512-column TMEM of the SM); tcgen05.st.32x32b.x8 throughput alone
+// and interleaved with loads, and the latency of a store -> wait::st -> load round trip on one column.
 //
 //     nvcc -std=c++17 -O3 -gencode arch=compute_100a,code=sm_100a -o tools/micro/tmem.bin tools/micro/tmem.cu
 #include <cstdio>
@@ -127,6 +128,63 @@ __global__ void __launch_bounds__( 128, 4 ) thr_tmem( uint32_t * sink, int iters
 	sink[blockIdx.x * 128 + threadIdx.x] = s;
 	tm_free( slot );
 	}
+// Store throughput: every thread writes 16 words per iteration (two x8 stores), and with LD also reads 16 other words
+// (two x8 loads) of the same iteration, one wait::st per iteration either way, 4 CTAs per SM.
+template<bool LD> __global__ void __launch_bounds__( 128, 4 ) thr_tmem_st( uint32_t * sink, int iters )
+	{
+	__shared__ uint32_t slot;
+	const uint32_t base = tm_alloc( &slot );
+	for( int c = 0; c < COLS; c += 4 ) tm_st4( base + c, c, c + 1, c + 2, c + 3 );
+	asm volatile( "tcgen05.wait::st.sync.aligned;" ::: "memory" );
+	uint32_t s = threadIdx.x;
+#pragma unroll 1
+	for( int i = 0; i < iters; ++i )
+		{
+		const uint32_t a = base + ( ( i * 32 ) & ( COLS - 1 ) );
+		const uint32_t v = s + i;
+		asm volatile( "tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1};" :: "r"( a ), "r"( v ) : "memory" );
+		asm volatile( "tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1};" :: "r"( a + 8 ), "r"( v ) : "memory" );
+		if( LD )
+			{
+			uint32_t r[16];
+			asm volatile( "tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+			              : "=r"( r[0] ), "=r"( r[1] ), "=r"( r[2] ), "=r"( r[3] ), "=r"( r[4] ), "=r"( r[5] ), "=r"( r[6] ), "=r"( r[7] ) : "r"( a + 16 ) : "memory" );
+			asm volatile( "tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+			              : "=r"( r[8] ), "=r"( r[9] ), "=r"( r[10] ), "=r"( r[11] ), "=r"( r[12] ), "=r"( r[13] ), "=r"( r[14] ), "=r"( r[15] ) : "r"( a + 24 ) : "memory" );
+			tm_wait();
+#pragma unroll
+			for( int j = 0; j < 16; ++j ) s ^= r[j];
+			}
+		asm volatile( "tcgen05.wait::st.sync.aligned;" ::: "memory" );
+		}
+	sink[blockIdx.x * 128 + threadIdx.x] = s;
+	tm_free( slot );
+	}
+
+// Round trip on one column: x2 store, wait::st, x2 load of the same column, wait::ld; the loaded value feeds the next
+// store (dependent chain).
+__global__ void __launch_bounds__( 128 ) lat_tmem_rt( long long * cyc, uint32_t * sink )
+	{
+	__shared__ uint32_t slot;
+	const uint32_t base = tm_alloc( &slot );
+	uint32_t x = threadIdx.x, y = 0;
+	long long t0 = 0;
+#pragma unroll 1
+	for( int i = -1; i < ITERS; ++i )
+		{
+		if( i == 0 ) t0 = clock64();
+		asm volatile( "tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1,%2};" :: "r"( base + 96 ), "r"( x ), "r"( y ) : "memory" );
+		asm volatile( "tcgen05.wait::st.sync.aligned;" ::: "memory" );
+		asm volatile( "tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0,%1}, [%2];" : "=r"( x ), "=r"( y ) : "r"( base + 96 ) : "memory" );
+		tm_wait();
+		x += 1u;
+		}
+	const long long t1 = clock64();
+	if( threadIdx.x == 0 ) cyc[0] = t1 - t0;
+	sink[threadIdx.x] = x + y;
+	tm_free( slot );
+	}
+
 // The same 16 words per thread per iteration as eight LDG.64 from a 2 KB table (L1 hits), 4 CTAs per SM.
 __global__ void __launch_bounds__( 128, 4 ) thr_ldg( const float2 * tab, uint32_t * sink, int iters )
 	{
@@ -190,6 +248,7 @@ int main()
 		lat_tmem<4><<<1, 128>>>( cyc, sink ); CK( cudaDeviceSynchronize() ); lat( "tcgen05.ld.32x32b.x4 + wait::ld" );
 		lat_tmem<16><<<1, 128>>>( cyc, sink ); CK( cudaDeviceSynchronize() ); lat( "tcgen05.ld.32x32b.x16 + wait::ld" );
 		lat_tmem<32><<<1, 128>>>( cyc, sink ); CK( cudaDeviceSynchronize() ); lat( "tcgen05.ld.32x32b.x32 + wait::ld" );
+		lat_tmem_rt<<<1, 128>>>( cyc, sink ); CK( cudaDeviceSynchronize() ); lat( "st.x2 + wait::st + ld.x2 + wait::ld" );
 		}
 	const int ctas = prop.multiProcessorCount * 4, iters = 1 << 16;
 	int occ = 0;
@@ -212,6 +271,8 @@ int main()
 		};
 	thr( "TMEM 4 x ld.x4 + wait, 16 warps/SM", [&] { thr_tmem<<<ctas, 128>>>( sink, iters ); } );
 	thr( "LDG.64 L1 hits, 16 warps/SM", [&] { thr_ldg<<<ctas, 128>>>( tab, sink, iters ); } );
+	thr( "TMEM 2 x st.x8 + wait::st", [&] { thr_tmem_st<false><<<ctas, 128>>>( sink, iters ); } );
+	thr( "TMEM 2 x st.x8 + 2 x ld.x8, both waits", [&] { thr_tmem_st<true><<<ctas, 128>>>( sink, iters ); } );
 	CK( cudaDeviceSynchronize() );
 	unsigned * cnt;
 	CK( cudaMalloc( &cnt, 2 * 1024 * sizeof( unsigned ) ) );
